@@ -17,6 +17,9 @@ tokens over the paged KV cache.  One "step" = one pass over one such batch.
             Linux) timed on this box's host cores on a bounded sample
 
 `--impl reference` times only that CPU restatement (rank 0), for the driver's reference arm.
+`--dump-outputs DIR` writes the token ids of the last device-timed step to DIR/ids.npy (float32 [clips, max_tokens]; one
+DIR/ids_rank<r>.npy per rank on several GPUs).  The inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import json
@@ -28,6 +31,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the benchmark may run from a read-only tree and writes nothing into it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "qwen3-asr-swift_b200"))
@@ -39,6 +43,7 @@ MAX_TOKENS = 128
 SEED = 20260418
 METRIC = "RTFx (audio-sec/sec) Qwen3-ASR-0.6B batched"
 UNIT = "audio-seconds/second"
+DUMP_LIMIT = 64 << 20  # bytes that --dump-outputs may write in all
 
 
 def peaks():
@@ -315,6 +320,7 @@ def main():
     ap.add_argument("--no-profile", action="store_true")
     ap.add_argument("--no-pipelined", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the pool / strong-scaling / 1.7B sub-records")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the token ids of the last timed step to DIR/ids.npy (float32)")
     args = ap.parse_args()
     MODEL, CLIP_SECONDS, CLIPS_PER_GPU, MAX_TOKENS = args.model, args.clip_seconds, args.clips_per_gpu, args.max_tokens
     METRIC = f"RTFx (audio-sec/sec) Qwen3-ASR-{MODEL} batched"
@@ -322,6 +328,12 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computes; the reference arm has none")
+    if args.dump_outputs and world * CLIPS_PER_GPU * MAX_TOKENS * 4 > DUMP_LIMIT:
+        ap.error(f"--dump-outputs: the ids of {world} x {CLIPS_PER_GPU} clips x {MAX_TOKENS} tokens exceed {DUMP_LIMIT >> 20} MB")
 
     if args.impl == "reference":
         run_reference(args, rank)
@@ -374,13 +386,18 @@ def main():
         model.batch_run(q3asr.STAGE_ALL, MAX_TOKENS, False)
         model.timer_record(1)
         dev_ms += model.timer_ms(0, 1)
-        model.batch_download(CLIPS_PER_GPU, MAX_TOKENS)
+        ids_last = model.batch_download(CLIPS_PER_GPU, MAX_TOKENS)
         stage += model.stage_ms()
     barrier()
     clocks = sampler.stop()
     launches = model.launch_count - l0
     dev_ms = max_over_ranks(dev_ms)
     value = world * audio_s * args.steps / (dev_ms / 1000.0)
+    if args.dump_outputs:
+        # fixed length (stop_on_eos off), so the ids stack to [clips, max_tokens]; float32 holds every id of the vocabulary exactly
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        name = "ids" if world == 1 else f"ids_rank{rank}"
+        np.save(os.path.join(args.dump_outputs, name + ".npy"), np.stack(ids_last).astype(np.float32))
 
     # ---- end to end: host buffers in, ids out ----
     model.transcribe_ids(clips, MAX_TOKENS, stop_on_eos=False)

@@ -6,6 +6,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from conftest import ROOT
@@ -51,3 +52,30 @@ def test_reference_arm_is_rank0_only():
 def test_product_arm_has_no_cpu_fallback():
     r = _run(["--steps", "1", "--warmup", "1"])
     assert r.returncode != 0 and r.stdout.strip() == "" and "no CPU fallback" in r.stderr
+
+
+def test_steps_and_dump_arguments_are_checked():
+    r = _run(["--steps", "0"])
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+    r = _run(["--impl", "reference", "--dump-outputs", "unused"])
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr
+    r = _run(["--clips-per-gpu", "1025", "--max-tokens", "16384", "--dump-outputs", "unused"])
+    assert r.returncode == 2 and "exceed 64 MB" in r.stderr
+    assert not os.path.exists(os.path.join(ROOT, "unused"))
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_ids(tmp_path):
+    """--dump-outputs writes the ids of the last timed step, [clips, max_tokens] in float32, the same in every run."""
+    args = ["--gpus", "1", "--steps", "2", "--warmup", "1", "--clips-per-gpu", "3", "--clip-seconds", "2", "--max-tokens", "6",
+            "--no-cpu-baseline", "--no-profile", "--no-pipelined", "--no-extras"]
+    dumps = []
+    for run in ("a", "b"):
+        r = _run(args + ["--dump-outputs", str(tmp_path / run)])
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout)["steps"] == 2
+        assert os.listdir(tmp_path / run) == ["ids.npy"]
+        dumps.append(np.load(tmp_path / run / "ids.npy"))
+    assert dumps[0].dtype == np.float32 and dumps[0].shape == (3, 6)
+    assert (dumps[0] == np.round(dumps[0])).all() and dumps[0].min() >= 0
+    assert np.array_equal(dumps[0], dumps[1])

@@ -6,8 +6,8 @@ length", at the sizes the configs name:
   q06b_ragged    0.6B, a 17.3 s clip: ragged last chunk, attention windows [104, 104, 17]
   q17b_clip15s   Qwen3-ASR-1.7B, one 15 s clip (config 4's shape)
 The fixtures are screened so that the ids are a real target (>= 32 distinct tokens in 128 steps, >= 90 % of the margins above
-two bf16 ulps); every step carries the oracle's eight best tokens and logits, and the prefill position its full-vocabulary logits
-from both the bf16-emulating and the plain fp32 oracle.
+two bf16 ulps); every step carries the oracle's eight best tokens and logits, and the prefill position its logits from both the
+bf16-emulating and the plain fp32 oracle (every `sample_step`-th vocabulary entry, which keeps a fixture under 1 MB).
 
 Why not plain equality everywhere: two correct bf16 implementations of an 18-layer encoder + 28-layer decoder do not agree bit for
 bit.  Every op rounds to bf16; a different fp32 summation order moves a few values across a rounding boundary and the flips spread.
@@ -23,9 +23,10 @@ An id is only determined by the arithmetic contract where its top-1 / top-2 marg
 NOISE_DEC = 16 ulps with the decoder isolated, NOISE_E2E = 40 ulps end to end.
 
 What is asserted:
-  * encoder, over the FULL output: relative L2 <= 2e-2 against the bf16-emulating oracle, and against the plain fp32 oracle at
-    most 1.5 x what the bf16 oracle itself shows (noise-calibrated) and <= 3e-2;
-  * prefill logits, full vocabulary: the same noise-calibrated bound against the fp32 oracle;
+  * encoder, over the FULL output: relative L2 <= 2e-2 against the bf16-emulating oracle, and against the plain fp32 oracle (on
+    every `sample_step`-th row) at most 1.5 x what the bf16 oracle itself shows (noise-calibrated) and <= 3e-2;
+  * prefill logits: the same noise-calibrated bound against the fp32 oracle on every `sample_step`-th vocabulary entry, and the
+    argmax over the full vocabulary among the oracle's in-noise candidates;
   * teacher-forced steps (the oracle's own ids, and a pseudo-random token stream), decoder isolated and end to end, EVERY step
     constrained: the chosen id equals the oracle's wherever the oracle's margin exceeds the bound; elsewhere it is one of the
     oracle's eight best tokens whose logit is within the bound of the best; the chosen token's logit is within 2 x the bound of the
@@ -146,8 +147,9 @@ def test_encoder_full_output(models, name):
     assert mx <= 16 * np.abs(ref).max() * 2.0 ** -8, (name, mx)
     msg = f"{name}: encoder {enc.shape} relL2 vs bf16 oracle {e1:.2e}, max |diff| {mx:.3g}"
     if "encoder_fp32_as_bf16" in g:
-        r32 = _bf16_bits_to_f32(g["encoder_fp32_as_bf16"])
-        e2, e_ref = _rel_l2(enc, r32), _rel_l2(ref, r32)
+        r32 = _bf16_bits_to_f32(g["encoder_fp32_as_bf16"])  # every sample_step-th row
+        step = int(g["sample_step"])
+        e2, e_ref = _rel_l2(enc[::step], r32), _rel_l2(ref[::step], r32)
         assert e2 <= 3e-2 and e2 <= 1.5 * e_ref, (name, e2, e_ref)
         msg += f"; vs fp32 oracle {e2:.2e} (the bf16 oracle itself: {e_ref:.2e})"
     print(msg)
@@ -158,13 +160,15 @@ def test_prefill_logits_full_vocabulary(models, name):
     g = _load(name)
     m = models(FIXTURES[name], int(g["seed"]))
     x = synth.clip(int(g["clip_index"]), int(g["n_samples"]))
-    got = m.prefill_logits(x)
+    logits = m.prefill_logits(x)
+    got = logits[::int(g["sample_step"])]  # the vocabulary entries the fixture keeps
     l32 = g["prefill_logits_fp32"].astype(np.float32)
     lbf = g["prefill_logits_bf16emu"].astype(np.float32)
+    assert got.shape == l32.shape == lbf.shape, (name, got.shape, l32.shape, lbf.shape)
     e_gpu, e_ref = _rel_l2(got, l32), _rel_l2(lbf, l32)
     assert e_gpu <= 1.5 * e_ref + 1e-3, (name, e_gpu, e_ref)
     assert _rel_l2(got, lbf) <= 2.0 * e_ref + 1e-3, (name, _rel_l2(got, lbf), e_ref)
-    assert int(np.argmax(got)) in _allowed(g["topk_ids"][0], g["topk_vals"][0], NOISE_E2E)
+    assert int(np.argmax(logits)) in _allowed(g["topk_ids"][0], g["topk_vals"][0], NOISE_E2E)
     print(f"{name}: prefill logits relL2 vs fp32 oracle {e_gpu:.2e} (the bf16 oracle itself: {e_ref:.2e}), vs bf16 oracle {_rel_l2(got, lbf):.2e}")
 
 

@@ -33,8 +33,10 @@ for name in (sys.argv[1:] or list(SIZES)):
     rel = np.linalg.norm(enc - ref) / np.linalg.norm(ref)
     msg = f"{name}: encoder relL2 vs bf16 oracle {rel:.3e}, max |diff| {np.abs(enc - ref).max():.3g} (max |ref| {np.abs(ref).max():.3g})"
     if "encoder_fp32_as_bf16" in g:
-        r32 = (np.asarray(g["encoder_fp32_as_bf16"], dtype=np.uint32) << 16).view(np.float32)
-        msg += f", vs fp32 oracle {np.linalg.norm(enc - r32) / np.linalg.norm(r32):.3e}; bf16 oracle vs fp32 oracle {np.linalg.norm(ref - r32) / np.linalg.norm(r32):.3e}"
+        r32 = (np.asarray(g["encoder_fp32_as_bf16"], dtype=np.uint32) << 16).view(np.float32)  # every sample_step-th row
+        step = int(g["sample_step"])
+        msg += (f", vs fp32 oracle {np.linalg.norm(enc[::step] - r32) / np.linalg.norm(r32):.3e}; bf16 oracle vs fp32 oracle "
+                f"{np.linalg.norm(ref[::step] - r32) / np.linalg.norm(r32):.3e} (every {step}th row)")
     print(msg)
     streams = (("own ids", g["ids"][:-1], g["ids"], g["tops"], g["margins"]),) + (
         (("random stream", g["forced"], g["forced_ids"], g["forced_tops"], g["forced_margins"]),) if "forced" in g else ())
