@@ -177,6 +177,26 @@ int q3asr_transcribe_ids_opts(q3asr_handle* h, const float* const* pcm, const si
                               int32_t* ids_out, int* lens_out);
 /* resident-batch form: call between q3asr_batch_upload and the prefill stage */
 int q3asr_batch_set_sampling(q3asr_handle* h, const q3asr_sampling* sampling);
+
+/* Per-token log-probabilities (the score behind sc_transcription_result_t.confidence, VoicePipeline.swift:374-411).  For the token t
+ * emitted at step s of utterance i:
+ *     logprob[i][s] = z[t] - logsumexp(z)
+ * z = the model's bf16-rounded logits over the whole vocabulary (the values the argmax ranks), the sum evaluated in fp32 with max
+ * subtraction on the device, in the LM head's epilogue.  Step 0 is the token chosen at the prefill position (like top_out of
+ * q3asr_decode_forced).  With decoder knobs z is the UNMODIFIED model logits — before repetition penalty, n-gram mask, temperature
+ * and noise (Whisper's convention), so the number means the same on both paths.  Entries at and beyond lens_out[i] are 0.
+ * An utterance's log-probabilities do not depend on the size of the request or the sub-batch it lands in.
+ * Utterance score (host side): avg_logprob = mean(logprob[i][0 .. lens_out[i])) (an emitted EOS counts, as in Whisper),
+ * confidence = exp(avg_logprob).
+ * q3asr_transcribe_ids_lp: q3asr_transcribe_ids_opts plus logprobs_out [batch, max_tokens] (may be NULL: no extra work). */
+int q3asr_transcribe_ids_lp(q3asr_handle* h, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
+                            const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
+                            int32_t* ids_out, int* lens_out, float* logprobs_out);
+/* resident-batch form: enable != 0 between q3asr_batch_upload and the prefill stage (every upload starts with them off), then
+ * q3asr_batch_download_logprobs after the run: out [batch, max_tokens], the layout of q3asr_batch_download's ids.
+ * Q3ASR_ERR_STATE when they were not enabled for the batch. */
+int q3asr_batch_set_logprobs(q3asr_handle* h, int enable);
+int q3asr_batch_download_logprobs(q3asr_handle* h, float* out, int max_tokens);
 /* pickNextToken on caller-provided logits ([vocab] fp32; the reference's own unit tests drive it this way,
  * Tests/Qwen3ASRTests/Qwen3DecodingOptionsTests.swift:47-235).  draw selects the noise draw (the decode step). */
 int q3asr_pick_next_token(q3asr_handle* h, const float* logits, int vocab, const int32_t* generated, int n_generated,
@@ -268,6 +288,10 @@ int q3asr_pool_transcribe_ids(q3asr_pool* p, const float* const* pcm, const size
 int q3asr_pool_transcribe_ids_opts(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
                                    const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
                                    int max_batch_per_gpu, int32_t* ids_out, int* lens_out);
+/* the same plus per-token log-probabilities (see q3asr_transcribe_ids_lp), logprobs_out [batch, max_tokens] (may be NULL) */
+int q3asr_pool_transcribe_ids_lp(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
+                                 const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
+                                 int max_batch_per_gpu, int32_t* ids_out, int* lens_out, float* logprobs_out);
 /* Submit / wait form of the call above (the "optional submit/poll pair" of the scheduler): the batch runs on a thread of the
  * library while the caller prepares the next one.  The sample, prompt-id and sample-rate arrays are borrowed until q3asr_job_wait
  * returns (the pointer tables themselves are copied); jobs of one pool run one after the other.  q3asr_job_wait blocks, copies
@@ -278,6 +302,12 @@ int q3asr_pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_sa
                       q3asr_job** job);
 int q3asr_job_done(const q3asr_job* job);
 int q3asr_job_wait(q3asr_job* job, int32_t* ids_out, int* lens_out);
+/* q3asr_pool_submit that also records per-token log-probabilities; after a successful q3asr_job_wait, q3asr_job_logprobs copies them
+ * out ([batch, max_tokens]).  Q3ASR_ERR_INVALID for a job submitted without them or not yet waited for. */
+int q3asr_pool_submit_lp(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
+                         const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu,
+                         q3asr_job** job);
+int q3asr_job_logprobs(const q3asr_job* job, float* logprobs_out);
 const char* q3asr_job_last_error(const q3asr_job* job);
 void q3asr_job_free(q3asr_job* job);
 /* the scheduler's assignment alone (host logic; no GPU needed): gpu_out[i] = GPU of utterance i */
@@ -346,7 +376,8 @@ int q3asr_longform_plan(size_t n_samples, size_t window, size_t min_tail, size_t
  * use_simt != 0 runs the CUDA-core checker kernel instead of tcgen05.  out: bf16 as uint16 (epi 0,1: [M,N] / [M,N/2]),
  * fp32 (epi 2) or int32 argmax ids [M] (epi 3). bn = 0 picks the tile width.
  * epi 4,5 run the decode-step weight-streaming kernel (M <= 128): 4 split-K fp32 partials summed -> fp32 [M,N]; 5 bf16 [M,N];
- * epi 7 runs the decode-step LM-head kernel (M <= 128): int32 argmax ids [M]. */
+ * epi 7 runs the decode-step LM-head kernel (M <= 256): int32 argmax ids [M].  epi 8 (the LM-head kernel) and 9 (epi 3) also reduce
+ * the log-sum-exp: int32 ids [M] followed by fp32 log-probabilities of those ids [M] (q3asr_transcribe_ids_lp's definition). */
 int q3asr_debug_gemm(q3asr_handle* h, const uint16_t* A, const uint16_t* W, const uint16_t* bias, const uint16_t* resid, int M,
                      int N, int K, int epi, int gelu, int bn, int use_simt, void* out);
 /* 3x3 stride-2 pad-1 NHWC convolution as implicit GEMM: in [B,H,W,C] bf16, w [O,3,3,C] bf16, out [B,OH,OW,O] bf16 (+bias, GELU) */

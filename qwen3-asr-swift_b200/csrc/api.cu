@@ -318,7 +318,8 @@ namespace {
 // utterance's ids would depend on the size of the request it arrived in.  Utterances are independent; outputs land at their own
 // offsets; stage times are summed over the sub-batches.
 void transcribe_chunked(Handle& x, const float* const* pcm, const size_t* n, const int* rates, int batch, const q3asr_prompt* prompts,
-                        const q3asr_sampling* sampling, bool set_sampling, int max_tokens, int stop_on_eos, int32_t* ids_out, int* lens_out) {
+                        const q3asr_sampling* sampling, bool set_sampling, int max_tokens, int stop_on_eos, int32_t* ids_out, int* lens_out,
+                        float* lp_out = nullptr) {
     Q3_CHECK(ids_out != nullptr && lens_out != nullptr, Q3ASR_ERR_INVALID, "transcribe: null output");
     const int chunks = batch <= SKINNY_MAX_ROWS ? 1 : (batch + SKINNY_MAX_ROWS - 1) / SKINNY_MAX_ROWS;
     const int per = chunks == 1 ? batch : (batch + chunks - 1) / chunks;  // batch <= 0 is refused by batch_upload below
@@ -329,8 +330,10 @@ void transcribe_chunked(Handle& x, const float* const* pcm, const size_t* n, con
         UploadGuard ug{&x};  // the staging threads never outlive this call (they read the caller's buffers)
         batch_upload(&x, pcm + b0, n + b0, nb, prompts ? prompts + b0 : nullptr, rates ? rates + b0 : nullptr, true);
         if (set_sampling) batch_set_sampling(&x, sampling);
+        if (lp_out) batch_set_logprobs(&x, 1);
         batch_run(&x, Q3ASR_STAGE_ALL, max_tokens, stop_on_eos);
         batch_download(&x, ids_out + (size_t)b0 * max_tokens, max_tokens, lens_out + b0);
+        if (lp_out) batch_download_logprobs(&x, lp_out + (size_t)b0 * max_tokens, max_tokens);
         for (int i = 0; i < 4; i++) stage_sum[i] += x.stage_ms[i];
         b0 += nb;
     } while (b0 < batch);
@@ -361,7 +364,20 @@ int q3asr_batch_set_sampling(q3asr_handle* h, const q3asr_sampling* opts) {
 int q3asr_transcribe_ids_opts(q3asr_handle* h, const float* const* pcm, const size_t* n, const int* sample_rates, int batch,
                               const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
                               int32_t* ids_out, int* lens_out) {
-    return guarded(h, [&](Handle& x) { transcribe_chunked(x, pcm, n, sample_rates, batch, prompts, sampling, true, max_tokens, stop_on_eos, ids_out, lens_out); });
+    return q3asr_transcribe_ids_lp(h, pcm, n, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, ids_out, lens_out, nullptr);
+}
+int q3asr_transcribe_ids_lp(q3asr_handle* h, const float* const* pcm, const size_t* n, const int* sample_rates, int batch,
+                            const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
+                            int32_t* ids_out, int* lens_out, float* logprobs_out) {
+    return guarded(h, [&](Handle& x) {
+        transcribe_chunked(x, pcm, n, sample_rates, batch, prompts, sampling, true, max_tokens, stop_on_eos, ids_out, lens_out, logprobs_out);
+    });
+}
+int q3asr_batch_set_logprobs(q3asr_handle* h, int enable) {
+    return guarded(h, [&](Handle& x) { batch_set_logprobs(&x, enable); });
+}
+int q3asr_batch_download_logprobs(q3asr_handle* h, float* out, int max_tokens) {
+    return guarded(h, [&](Handle& x) { batch_download_logprobs(&x, out, max_tokens); });
 }
 int q3asr_pick_next_token(q3asr_handle* h, const float* logits, int vocab, const int32_t* generated, int n_generated,
                           const q3asr_sampling* opts, int draw, int32_t* token) {
@@ -474,9 +490,12 @@ int q3asr_debug_gemm(q3asr_handle* hh, const uint16_t* A, const uint16_t* W, con
                      int K, int epi, int gelu, int bn, int use_simt, void* out) {
     return guarded(hh, [&](Handle& h) {
         Q3_CHECK(A && W && out && M > 0 && N > 0 && K > 0, Q3ASR_ERR_INVALID, "debug_gemm: bad argument");
-        if (epi == 7) {  // decode-step LM head (lmhead.cuh): int32 argmax ids [M]
+        // 8 / 9: the LM-head kernel / EPI_ARGMAX with the per-tile sums of exp(z - tile max) -> int32 ids [M], then fp32 logprobs [M]
+        const bool lp = epi == 8 || epi == 9;
+        if (epi == 9) epi = EPI_ARGMAX;
+        if (epi == 7 || epi == 8) {  // decode-step LM head (lmhead.cuh): int32 argmax ids [M]
             bf16 *dA, *dW;
-            float* dv;
+            float *dv, *ds = nullptr, *dlp = nullptr;
             int* di;
             int32_t* dtok;
             const int tiles = lmhead_tiles(N);
@@ -485,19 +504,26 @@ int q3asr_debug_gemm(q3asr_handle* hh, const uint16_t* A, const uint16_t* W, con
             Q3_CUDA(cudaMalloc(&dv, sizeof(float) * (size_t)M * tiles));
             Q3_CUDA(cudaMalloc(&di, sizeof(int) * (size_t)M * tiles));
             Q3_CUDA(cudaMalloc(&dtok, sizeof(int32_t) * (size_t)M));
+            if (lp) {
+                Q3_CUDA(cudaMalloc(&ds, sizeof(float) * (size_t)M * tiles));
+                Q3_CUDA(cudaMalloc(&dlp, sizeof(float) * (size_t)M));
+            }
             cudaError_t se = cudaSuccess;
+            auto release = [&]() { cudaFree(dA); cudaFree(dW); cudaFree(dv); cudaFree(di); cudaFree(dtok); cudaFree(ds); cudaFree(dlp); };
             try {
                 Q3_H2D_SYNC(dA, A, 2 * (size_t)M * K);
                 Q3_H2D_SYNC(dW, W, 2 * (size_t)N * K);
-                lmhead_argmax(dA, K, M, K, dW, N, dv, di, h.stream);
-                argmax_reduce(dv, di, M, tiles, dtok, nullptr, h.stream);
+                lmhead_argmax(dA, K, M, K, dW, N, dv, di, h.stream, ds);
+                if (lp) argmax_lse_reduce(dv, di, ds, nullptr, nullptr, 0, M, tiles, dtok, nullptr, dlp, h.stream);
+                else argmax_reduce(dv, di, M, tiles, dtok, nullptr, h.stream);
                 se = cudaStreamSynchronize(h.stream);
                 if (se == cudaSuccess) se = cudaMemcpy(out, dtok, sizeof(int32_t) * (size_t)M, cudaMemcpyDeviceToHost);
+                if (se == cudaSuccess && lp) se = cudaMemcpy(reinterpret_cast<int32_t*>(out) + M, dlp, sizeof(float) * (size_t)M, cudaMemcpyDeviceToHost);
             } catch (...) {
-                cudaFree(dA); cudaFree(dW); cudaFree(dv); cudaFree(di); cudaFree(dtok);
+                release();
                 throw;
             }
-            cudaFree(dA); cudaFree(dW); cudaFree(dv); cudaFree(di); cudaFree(dtok);
+            release();
             Q3_CUDA(se);
             return;
         }
@@ -543,7 +569,7 @@ int q3asr_debug_gemm(q3asr_handle* hh, const uint16_t* A, const uint16_t* W, con
         }
         bf16 *dA, *dW, *dB = nullptr, *dR = nullptr;
         void* dO;
-        float* dv = nullptr;
+        float *dv = nullptr, *ds = nullptr, *dlp = nullptr;
         int* di = nullptr;
         int32_t* dtok = nullptr;
         const int bnn = bn ? bn : gemm_pick_bn(N, epi, cdiv(M, GEMM_BM));
@@ -579,16 +605,25 @@ int q3asr_debug_gemm(q3asr_handle* hh, const uint16_t* A, const uint16_t* W, con
             Q3_CUDA(cudaMalloc(&dtok, sizeof(int32_t) * (size_t)M));
             e.amax_val = dv;
             e.amax_idx = di;
+            if (lp) {
+                Q3_CUDA(cudaMalloc(&ds, sizeof(float) * (size_t)M * tiles_n));
+                Q3_CUDA(cudaMalloc(&dlp, sizeof(float) * (size_t)M));
+                e.amax_sum = ds;
+            }
         }
         gemm(dA, K, M, K, dW, N, e, h.stream, use_simt != 0, bnn);
-        if (epi == EPI_ARGMAX) {
+        if (epi == EPI_ARGMAX && lp) {
+            argmax_lse_reduce(dv, di, ds, nullptr, nullptr, 0, M, tiles_n, dtok, nullptr, dlp, h.stream);
+            Q3_CUDA(cudaMemcpyAsync(out, dtok, out_bytes, cudaMemcpyDeviceToHost, h.stream));
+            Q3_CUDA(cudaMemcpyAsync(reinterpret_cast<int32_t*>(out) + M, dlp, sizeof(float) * (size_t)M, cudaMemcpyDeviceToHost, h.stream));
+        } else if (epi == EPI_ARGMAX) {
             argmax_reduce(dv, di, M, tiles_n, dtok, nullptr, h.stream);
             Q3_CUDA(cudaMemcpyAsync(out, dtok, out_bytes, cudaMemcpyDeviceToHost, h.stream));
         } else {
             Q3_CUDA(cudaMemcpyAsync(out, dO, out_bytes, cudaMemcpyDeviceToHost, h.stream));
         }
         cudaError_t se = cudaStreamSynchronize(h.stream);
-        cudaFree(dA); cudaFree(dW); cudaFree(dO); cudaFree(dB); cudaFree(dR); cudaFree(dv); cudaFree(di); cudaFree(dtok);
+        cudaFree(dA); cudaFree(dW); cudaFree(dO); cudaFree(dB); cudaFree(dR); cudaFree(dv); cudaFree(di); cudaFree(dtok); cudaFree(ds); cudaFree(dlp);
         Q3_CUDA(se);
     });
 }

@@ -252,6 +252,11 @@ void reserve_decoder(Handle* h, BatchState* bs) {
     bs->st_finished.reserve(B * 4);
     bs->st_slot_seq.reserve(B * 4);
     bs->st_scalars.reserve(64);
+    if (bs->logprobs_on) {
+        bs->amax_sum.reserve((size_t)bs->B * tiles * 4);
+        bs->st_next_lp.reserve(B * 4);
+        bs->st_out_lp.reserve(B * mt * 4);
+    }
     bs->h_out.reserve(B * mt * 8 + B * 8 + 64);
 }
 
@@ -605,8 +610,8 @@ void decoder_layers_decode(Handle* h, BatchState* bs) {
     }
 }
 
-// final norm of the given rows + tied LM head + argmax -> st_next_tok / st_next_val.  normed: bs->dlast already holds
-// the final-norm hidden states (fused decode path).
+// final norm of the given rows + tied LM head + argmax -> st_next_tok / st_next_val (+ st_next_lp with logprobs_on: every branch
+// also reduces the log-sum-exp of the bf16 logits).  normed: bs->dlast already holds the final-norm hidden states (fused decode path).
 void lm_head_argmax(Handle* h, BatchState* bs, const int* row_index, bool normed = false) {
     const q3asr_config& c = h->cfg;
     const Model& m = *h->model;
@@ -626,29 +631,46 @@ void lm_head_argmax(Handle* h, BatchState* bs, const int* row_index, bool normed
         e.out = bs->logits_bf.p;
         e.ldo = c.dec_vocab;
         gemm(bs->dlast.as<bf16>(), H, B, H, m.embed, c.dec_vocab, e, st);
-        sample_launch(bs->logits_bf.as<bf16>(), nullptr, c.dec_vocab, c.dec_vocab, bs->st_out_ids.as<int32_t>(), bs->max_tokens,
-                      bs->st_out_len.as<int>(), bs->sampling, bs->st_scalars.as<int>() + 1, B, bs->amax_val.as<float>(), bs->amax_idx.as<int>(),
-                      st);
-        argmax_reduce(bs->amax_val.as<float>(), bs->amax_idx.as<int>(), B, sample_parts(c.dec_vocab), bs->st_next_tok.as<int32_t>(),
-                      bs->st_next_val.as<float>(), st);
+        const int parts = sample_parts(c.dec_vocab);
+        if (bs->logprobs_on) {  // raw (max, sum) per slice: amax_sum = [sums | maxima], [B, parts] each
+            float* rsum = bs->amax_sum.as<float>();
+            float* rmax = rsum + (size_t)B * parts;
+            sample_launch(bs->logits_bf.as<bf16>(), nullptr, c.dec_vocab, c.dec_vocab, bs->st_out_ids.as<int32_t>(), bs->max_tokens,
+                          bs->st_out_len.as<int>(), bs->sampling, bs->st_scalars.as<int>() + 1, B, bs->amax_val.as<float>(),
+                          bs->amax_idx.as<int>(), st, rmax, rsum);
+            argmax_lse_reduce(bs->amax_val.as<float>(), bs->amax_idx.as<int>(), rsum, rmax, bs->logits_bf.as<bf16>(), c.dec_vocab, B, parts,
+                              bs->st_next_tok.as<int32_t>(), bs->st_next_val.as<float>(), bs->st_next_lp.as<float>(), st);
+        } else {
+            sample_launch(bs->logits_bf.as<bf16>(), nullptr, c.dec_vocab, c.dec_vocab, bs->st_out_ids.as<int32_t>(), bs->max_tokens,
+                          bs->st_out_len.as<int>(), bs->sampling, bs->st_scalars.as<int>() + 1, B, bs->amax_val.as<float>(),
+                          bs->amax_idx.as<int>(), st);
+            argmax_reduce(bs->amax_val.as<float>(), bs->amax_idx.as<int>(), B, parts, bs->st_next_tok.as<int32_t>(), bs->st_next_val.as<float>(),
+                          st);
+        }
         h->launches += 2;
         return;
     }
+    float* sums = bs->logprobs_on ? bs->amax_sum.as<float>() : nullptr;
+    int tiles = 0;
     if (B <= SKINNY_MAX_ROWS && env_int("Q3ASR_LM_GENERAL", 0) == 0) {
         // decode-step shape (few token rows): the persistent weight-streaming kernel of lmhead.cuh
-        lmhead_argmax(bs->dlast.as<bf16>(), H, B, H, m.embed, c.dec_vocab, bs->amax_val.as<float>(), bs->amax_idx.as<int>(), st);
-        argmax_reduce(bs->amax_val.as<float>(), bs->amax_idx.as<int>(), B, lmhead_tiles(c.dec_vocab), bs->st_next_tok.as<int32_t>(),
-                      bs->st_next_val.as<float>(), st);
-        h->launches++;
-        return;
+        lmhead_argmax(bs->dlast.as<bf16>(), H, B, H, m.embed, c.dec_vocab, bs->amax_val.as<float>(), bs->amax_idx.as<int>(), st, sums);
+        tiles = lmhead_tiles(c.dec_vocab);
+    } else {
+        const int bn = gemm_pick_bn(c.dec_vocab, EPI_ARGMAX, 1);
+        GemmEpiArgs e;
+        e.epi = EPI_ARGMAX;
+        e.amax_val = bs->amax_val.as<float>();
+        e.amax_idx = bs->amax_idx.as<int>();
+        e.amax_sum = sums;
+        gemm(bs->dlast.as<bf16>(), H, B, H, m.embed, c.dec_vocab, e, st, false, bn);
+        tiles = c.dec_vocab / bn;
     }
-    const int bn = gemm_pick_bn(c.dec_vocab, EPI_ARGMAX, 1);
-    GemmEpiArgs e;
-    e.epi = EPI_ARGMAX;
-    e.amax_val = bs->amax_val.as<float>();
-    e.amax_idx = bs->amax_idx.as<int>();
-    gemm(bs->dlast.as<bf16>(), H, B, H, m.embed, c.dec_vocab, e, st, false, bn);
-    argmax_reduce(e.amax_val, e.amax_idx, B, c.dec_vocab / bn, bs->st_next_tok.as<int32_t>(), bs->st_next_val.as<float>(), st);
+    if (sums)
+        argmax_lse_reduce(bs->amax_val.as<float>(), bs->amax_idx.as<int>(), sums, nullptr, nullptr, 0, B, tiles, bs->st_next_tok.as<int32_t>(),
+                          bs->st_next_val.as<float>(), bs->st_next_lp.as<float>(), st);
+    else
+        argmax_reduce(bs->amax_val.as<float>(), bs->amax_idx.as<int>(), B, tiles, bs->st_next_tok.as<int32_t>(), bs->st_next_val.as<float>(), st);
     h->launches++;
 }
 
@@ -661,6 +683,10 @@ DecodeState decode_state(Handle* h, BatchState* bs, int stop_on_eos, bool forced
     s.kv_len = bs->st_kv_len.as<int>();
     s.out_ids = bs->st_out_ids.as<int32_t>();
     s.out_val = bs->st_out_val.as<float>();
+    if (bs->logprobs_on) {
+        s.next_lp = bs->st_next_lp.as<float>();
+        s.out_lp = bs->st_out_lp.as<float>();
+    }
     s.out_len = bs->st_out_len.as<int>();
     s.finished = bs->st_finished.as<int>();
     s.n_active = bs->st_scalars.as<int>();
@@ -695,6 +721,7 @@ void run_prefill(Handle* h, BatchState* bs, int stop_on_eos, bool forced) {
     bs->slot_map_on = false;
     bs->stat_row_steps = bs->stat_steps = bs->stat_compactions = 0;
     Q3_CUDA(cudaMemsetAsync(bs->st_out_ids.p, 0, sizeof(int32_t) * B * std::max(bs->max_tokens, 1), st));
+    if (bs->logprobs_on) Q3_CUDA(cudaMemsetAsync(bs->st_out_lp.p, 0, sizeof(float) * B * std::max(bs->max_tokens, 1), st));
     const int scal[2] = {B, 0};
     memcpy(bs->h_out.p, scal, sizeof(scal));
     Q3_CUDA(cudaMemcpyAsync(bs->st_scalars.p, bs->h_out.p, sizeof(scal), cudaMemcpyHostToDevice, st));
@@ -908,6 +935,7 @@ void batch_upload(Handle* h, const float* const* pcm, const size_t* n_in, int ba
     bs->steps_done = 0;
     bs->has_audio = true;
     bs->sampler_on = false;  // every batch starts greedy; batch_set_sampling turns the decoder knobs on
+    bs->logprobs_on = false;  // batch_set_logprobs turns them on
     // samples: pinned staging -> device
     bs->pcm.reserve(sizeof(float) * (bs->mel.pcm_floats + 64));
     bs->mel_out.reserve(sizeof(float) * std::max<long long>(bs->mel.out_floats, 1));
@@ -1096,6 +1124,13 @@ void batch_set_sampling(Handle* h, const q3asr_sampling* opts) {
     bs->sampling.seed = opts->seed;
 }
 
+void batch_set_logprobs(Handle* h, int enable) {
+    BatchState* bs = h->batch.get();
+    Q3_CHECK(bs != nullptr && bs->B > 0 && bs->has_audio, Q3ASR_ERR_STATE, "batch_set_logprobs: no batch uploaded");
+    Q3_CHECK(!bs->prefill_done, Q3ASR_ERR_STATE, "batch_set_logprobs: the first token of this batch has already been chosen");
+    bs->logprobs_on = enable != 0;
+}
+
 void pick_next_token(Handle* h, const float* logits, int vocab, const int32_t* generated, int n_generated, const q3asr_sampling* opts,
                      int draw, int32_t* token) {
     Q3_CHECK(logits != nullptr && vocab > 0 && n_generated >= 0 && (generated != nullptr || n_generated == 0) && opts != nullptr &&
@@ -1199,6 +1234,25 @@ void batch_download(Handle* h, int32_t* ids, int max_tokens, int* lens) {
         float ms = 0.f;
         if (cudaEventElapsedTime(&ms, bs->ev[i], bs->ev[i + 1]) == cudaSuccess) h->stage_ms[i] = ms;
     }
+}
+
+void batch_download_logprobs(Handle* h, float* out, int max_tokens) {
+    BatchState* bs = h->batch.get();
+    Q3_CHECK(bs != nullptr && bs->B > 0, Q3ASR_ERR_STATE, "batch_download_logprobs: no batch");
+    Q3_CHECK(out != nullptr && max_tokens >= 0, Q3ASR_ERR_INVALID, "batch_download_logprobs: bad argument");
+    Q3_CHECK(bs->logprobs_on, Q3ASR_ERR_STATE, "batch_download_logprobs: log-probabilities were not requested for this batch");
+    const int B = bs->B, mt = bs->max_tokens;
+    cudaStream_t st = h->stream;
+    std::fill(out, out + (size_t)B * max_tokens, 0.f);
+    if (!bs->prefill_done) {
+        Q3_CUDA(cudaStreamSynchronize(st));
+        return;
+    }
+    float* h_lp = reinterpret_cast<float*>(bs->h_out.p) + 16;  // (the staging area of batch_download: ids [B, mt] + lens fit)
+    Q3_CUDA(cudaMemcpyAsync(h_lp, bs->st_out_lp.p, sizeof(float) * B * mt, cudaMemcpyDeviceToHost, st));
+    Q3_CUDA(cudaStreamSynchronize(st));
+    const int L = std::min(max_tokens, mt);
+    for (int b = 0; b < B; b++) memcpy(out + (size_t)b * max_tokens, h_lp + (size_t)b * mt, sizeof(float) * L);
 }
 
 void encode_one(Handle* h, const float* mel, int frames, float* out, int* tokens) {

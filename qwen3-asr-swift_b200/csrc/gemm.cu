@@ -129,6 +129,11 @@ __global__ void simt_epi_kernel(const float* acc, long rows, GemmDev p, int epi,
         }
         p.amax_val[idx] = best;
         p.amax_idx[idx] = bi;
+        if (p.amax_sum) {
+            float sum = 0.f;
+            for (int j = 0; j < BN; j++) sum += __expf(bf16_round(acc[row * p.N + tn * BN + j]) - best);
+            p.amax_sum[idx] = sum;
+        }
         return;
     }
     if (epi == EPI_SWIGLU) {
@@ -203,6 +208,81 @@ __global__ void argmax_reduce_kernel(const float* val, const int* idx, int rows,
     }
 }
 
+// argmax_reduce_kernel plus the log-probability of the chosen token: lse = M + log sum_t s_t exp(m_t - M) over the per-tile maxima
+// m_t (tile_max, or val when null) and sums s_t = sum exp(z - m_t) of the tile's logits; out_lp = z[chosen] - lse, with z[chosen]
+// read from the raw bf16 logits when given (decoder knobs: the chosen index need not be the raw maximum), else the maximum itself.
+// Every thread walks its tiles in ascending order and the 256 threads are merged by a fixed tree, so the result depends only on
+// `tiles`, never on the row count.
+__global__ void __launch_bounds__(256) argmax_lse_reduce_kernel(const float* val, const int* idx, const float* tile_sum, const float* tile_max,
+                                                                const bf16* raw, int ld, int rows, int tiles, int32_t* out, float* out_val,
+                                                                float* out_lp) {
+    ptx::grid_dep_launch();
+    ptx::grid_dep_wait();
+    const int row = blockIdx.x;
+    if (row >= rows) return;
+    const float* mx = (tile_max ? tile_max : val) + (size_t)row * tiles;
+    const float* sm = tile_sum + (size_t)row * tiles;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    __shared__ float sv[8];
+    __shared__ int si[8];
+    __shared__ float s_m;
+    float best = -INFINITY, m = -INFINITY;
+    int bi = 0x7fffffff;
+    for (int t = threadIdx.x; t < tiles; t += blockDim.x) {
+        const float v = val[(size_t)row * tiles + t];
+        const int i = idx[(size_t)row * tiles + t];
+        if (v > best || (v == best && i < bi)) { best = v; bi = i; }
+        m = fmaxf(m, mx[t]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }
+        m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+    }
+    if (lane == 0) { sv[warp] = best; si[warp] = bi; }
+    __syncthreads();
+    if (warp == 0) {
+        best = lane < 8 ? sv[lane] : -INFINITY;
+        bi = lane < 8 ? si[lane] : 0x7fffffff;
+#pragma unroll
+        for (int o = 4; o > 0; o >>= 1) {
+            const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+            const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+            if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }
+        }
+    }
+    __syncthreads();
+    if (lane == 0) sv[warp] = m;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float mm = sv[0];
+        for (int w = 1; w < 8; w++) mm = fmaxf(mm, sv[w]);
+        s_m = mm;
+    }
+    __syncthreads();
+    const float M = s_m;
+    float s = 0.f;
+    for (int t = threadIdx.x; t < tiles; t += blockDim.x) {
+        const float mt = mx[t];
+        if (mt != -INFINITY) s += sm[t] * __expf(mt - M);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    __syncthreads();  // sv is reused
+    if (lane == 0) sv[warp] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float tot = 0.f;
+        for (int w = 0; w < 8; w++) tot += sv[w];
+        const float z = raw ? __bfloat162float(raw[(size_t)row * ld + bi]) : best;
+        out[row] = bi;
+        if (out_val) out_val[row] = best;
+        out_lp[row] = (z - M) - logf(tot);  // z - M first: both are logits of similar size, the difference is exact
+    }
+}
+
 }  // namespace
 
 void make_tmap_2d_bf16(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint64_t row_stride_elems, uint32_t box_cols,
@@ -266,7 +346,7 @@ void gemm_conv(const GemmA& a, const GemmShape& s, const bf16* W, int N, const G
     for (int t = 0; t < GEMM_MAX_TAPS; t++) { p.tap_dw[t] = s.tap_dw[t]; p.tap_dh[t] = s.tap_dh[t]; }
     p.out = e.out; p.ldo = e.ldo; p.bias = e.bias; p.resid = e.resid; p.ldr = e.ldr;
     p.row_add = e.row_add; p.row_map = e.row_map; p.valid_w = e.valid_w; p.gelu = e.gelu;
-    p.amax_val = e.amax_val; p.amax_idx = e.amax_idx;
+    p.amax_val = e.amax_val; p.amax_idx = e.amax_idx; p.amax_sum = e.amax_sum;
     p.rp = e.rp;
     const long m_tiles = (long)p.tiles_w * p.tiles_h * p.tiles_b;
     if (bn == 0 && e.epi == EPI_QKV) bn = (N % 256 == 0 && m_tiles * (N / 256) >= g_num_sms) ? 256 : 128;  // tiles of whole heads
@@ -461,19 +541,25 @@ void gemm_skinny(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N, 
 }
 
 namespace {
-template <int NB>
-void launch_lmhead(const CUtensorMap& tw, const CUtensorMap& tx, const LmHeadDev& p, int grid, cudaStream_t st) {
+template <int NB, bool LSE>
+void launch_lmhead_k(const CUtensorMap& tw, const CUtensorMap& tx, const LmHeadDev& p, int grid, cudaStream_t st) {
     static PerDeviceOnce attr_once;
     attr_once([] {
-        Q3_CUDA(cudaFuncSetAttribute(lmhead_argmax_kernel<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, lmh_smem_bytes(NB)));
+        Q3_CUDA(cudaFuncSetAttribute(lmhead_argmax_kernel<NB, LSE>, cudaFuncAttributeMaxDynamicSharedMemorySize, lmh_smem_bytes(NB, LSE)));
     });
-    launch_kernel(lmhead_argmax_kernel<NB>, grid, 256, lmh_smem_bytes(NB), st, tw, tx, p);
+    launch_kernel(lmhead_argmax_kernel<NB, LSE>, grid, 256, lmh_smem_bytes(NB, LSE), st, tw, tx, p);
+}
+template <int NB>
+void launch_lmhead(const CUtensorMap& tw, const CUtensorMap& tx, const LmHeadDev& p, int grid, cudaStream_t st) {
+    if (p.amax_sum) launch_lmhead_k<NB, true>(tw, tx, p, grid, st);
+    else launch_lmhead_k<NB, false>(tw, tx, p, grid, st);
 }
 }  // namespace
 
 int lmhead_tiles(int N) { return cdiv(N, SK_BM); }
 
-void lmhead_argmax(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N, float* amax_val, int* amax_idx, cudaStream_t st) {
+void lmhead_argmax(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N, float* amax_val, int* amax_idx, cudaStream_t st,
+                   float* amax_sum) {
     Q3_CHECK(Mtok > 0 && Mtok <= SKINNY_MAX_ROWS, 1, "lmhead_argmax: 1..256 token rows per launch");
     Q3_CHECK(K % 8 == 0 && ldx % 8 == 0 && N > 0 && amax_val && amax_idx, 1, "lmhead_argmax: bad argument");
     const int nb = Mtok <= 16 ? 16 : Mtok <= 32 ? 32 : Mtok <= 64 ? 64 : Mtok <= 128 ? 128 : 256;
@@ -485,6 +571,7 @@ void lmhead_argmax(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N
     p.tiles = lmhead_tiles(N);
     p.amax_val = amax_val;
     p.amax_idx = amax_idx;
+    p.amax_sum = amax_sum;
     CUtensorMap tw, tx;
     {
         cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)N};
@@ -515,6 +602,13 @@ void lmhead_argmax(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N
 void argmax_reduce(const float* val, const int* idx, int rows, int tiles, int32_t* out, float* out_val, cudaStream_t st) {
     if (rows <= 0) return;
     launch_kernel(argmax_reduce_kernel, rows, 256, 0, st, val, idx, rows, tiles, out, out_val);
+}
+
+void argmax_lse_reduce(const float* val, const int* idx, const float* tile_sum, const float* tile_max, const bf16* raw, int ld, int rows,
+                       int tiles, int32_t* out, float* out_val, float* out_lp, cudaStream_t st) {
+    if (rows <= 0) return;
+    Q3_CHECK(tile_sum != nullptr && out_lp != nullptr, 1, "argmax_lse_reduce: null sums / output");
+    launch_kernel(argmax_lse_reduce_kernel, rows, 256, 0, st, val, idx, tile_sum, tile_max, raw, ld, rows, tiles, out, out_val, out_lp);
 }
 
 }  // namespace q3

@@ -78,6 +78,7 @@ struct GemmDev {  // by-value kernel parameter
     int tma_out;           // EPI_NORMAL: output tiles are staged in shared memory and written with TMA stores (tmC is valid)
     float* amax_val;       // [rows, tiles_n]
     int* amax_idx;
+    float* amax_sum;       // [rows, tiles_n] sum of exp(bf16(acc) - tile max) over the tile, or null (EPI_ARGMAX)
     QkvRope rp;            // EPI_QKV only
 };
 
@@ -300,9 +301,19 @@ __device__ __forceinline__ void gemm_epilogue_tile(const GemmDev& p, const TileC
                 if (x > best) { best = x; best_i = n0 + c * 32 + j; }
             }
         }
+        float sum = 0.f;
+#pragma unroll 1
+        for (int c = 0; c < (chalf == 0 && p.amax_sum != nullptr ? BN / 32 : 0); c++) {  // second pass, columns in order
+            uint32_t v[32];
+            ptx::tmem_ld_32x32(t_row + c * 32, v);
+            ptx::tmem_ld_wait();
+#pragma unroll
+            for (int j = 0; j < 32; j++) sum += __expf(bf16_round(__uint_as_float(v[j])) - best);
+        }
         if (row_ok && chalf == 0) {
             p.amax_val[(size_t)row * p.tiles_n + tc.tn] = best;
             p.amax_idx[(size_t)row * p.tiles_n + tc.tn] = best_i;
+            if (p.amax_sum != nullptr) p.amax_sum[(size_t)row * p.tiles_n + tc.tn] = sum;
         }
     } else {
         // Bias and residual do not depend on the accumulator: the loads of chunk c + 2 are issued before chunk c is processed (and
@@ -620,6 +631,7 @@ struct GemmEpiArgs {
     int max_stages = 0;  // 0: as deep as shared memory allows
     float* amax_val = nullptr;
     int* amax_idx = nullptr;
+    float* amax_sum = nullptr;  // EPI_ARGMAX: also the per-(row, n-tile) sum of exp(bf16(acc) - tile max), for log-probabilities
     QkvRope rp = {};  // EPI_QKV
 };
 
@@ -649,8 +661,15 @@ void gemm_skinny(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N, 
 // Decode-step LM head (lmhead.cuh): per 128-row vocabulary tile the (value, index) of the first maximum of bf16(X E^T) for every token
 // row, amax_val / amax_idx [Mtok, lmhead_tiles(N)], to be merged by argmax_reduce.  Mtok <= SKINNY_MAX_ROWS.
 int lmhead_tiles(int N);
-void lmhead_argmax(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N, float* amax_val, int* amax_idx, cudaStream_t st);
+// amax_sum (may be null): also sum over the tile's rows of exp(z - tile max) per token, for log-probabilities (a second instantiation).
+void lmhead_argmax(const bf16* X, int ldx, int Mtok, int K, const bf16* W, int N, float* amax_val, int* amax_idx, cudaStream_t st,
+                   float* amax_sum = nullptr);
 // final reduce of EPI_ARGMAX partials: out[row] = index of the maximum (lowest index on ties)
 void argmax_reduce(const float* val, const int* idx, int rows, int tiles, int32_t* out, float* out_val, cudaStream_t st);
+// the same plus out_lp[row] = z[out[row]] - logsumexp(z) from the per-tile sums of exp(z - tile max) (tile_sum) and per-tile maxima
+// (tile_max, or val itself when null).  raw (may be null): bf16 logits [rows, ld] to read z[out[row]] from (decoder knobs, where the
+// chosen token need not be the maximum of the raw logits); else z[out[row]] is the maximum.
+void argmax_lse_reduce(const float* val, const int* idx, const float* tile_sum, const float* tile_max, const bf16* raw, int ld, int rows,
+                       int tiles, int32_t* out, float* out_val, float* out_lp, cudaStream_t st);
 
 }  // namespace q3

@@ -209,6 +209,8 @@ void pick_next_token(Handle* h, const float* logits, int vocab, const int32_t* g
                      int draw, int32_t* token);
 void batch_run(Handle* h, int stages, int max_tokens, int stop_on_eos);
 void batch_download(Handle* h, int32_t* ids, int max_tokens, int* lens);
+void batch_set_logprobs(Handle* h, int enable);
+void batch_download_logprobs(Handle* h, float* out, int max_tokens);
 void encode_one(Handle* h, const float* mel, int frames, float* out, int* tokens);
 void decode_forced(Handle* h, const float* pcm, size_t n, const q3asr_prompt* prompt, const int32_t* forced, int n_forced,
                    int32_t* argmax_out, float* top_out, const float* audio_embeds = nullptr, int n_audio_tokens = 0);

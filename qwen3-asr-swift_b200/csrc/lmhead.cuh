@@ -10,6 +10,15 @@
 // thread (TMEM lane): the per-token maximum over the 32 rows of a warp is a transpose-reduce (31 exchanges per 32 tokens instead
 // of 160), the four warps are merged through shared memory, and each tile writes (value, index) per token for argmax_reduce.
 //
+// LSE = true (log-probabilities, q3asr_batch_set_logprobs) also writes amax_sum[token, tile] = sum over the tile's valid rows of
+// exp(z_r - tile max), z = bf16(logits).  Formulation: the max transpose-reduce already leaves lane l with token l's maximum over the
+// warp's 32 rows; it is broadcast back with one shuffle per token, each lane takes one exponential per value against it (rows >= N
+// contribute 0, never exp(-inf - -inf)), a second transpose-reduce sums them, and the four warps' (max, sum) pairs are merged in
+// warp order with s = sum_w s_w exp(m_w - M).  Carrying (max, sum) pairs through the first reduce instead would take two exponentials
+// per exchange; broadcasting the TILE maximum is not possible, because it is known only after the four-warp merge, when the
+// accumulator has been handed back to the tensor core.  Every token's sum has one fixed tree (lane butterfly, then warps 0..3), so it
+// does not depend on NB, on the token count or on which CTA owns the tile.
+//
 // CTA = 256 threads: warp 0 TMA producer, warp 1 MMA issuer, warp 2 TMEM allocator, warps 4-7 epilogue.
 #pragma once
 #include "skinny.cuh"
@@ -20,11 +29,14 @@ struct LmHeadDev {
     int N, Mtok, num_kb, tiles;
     float* amax_val;  // [Mtok, tiles]
     int* amax_idx;
+    float* amax_sum;  // [Mtok, tiles], LSE instantiations only
 };
 
 constexpr int LMH_STAGES = 8;
 __host__ __device__ constexpr int lmh_stages(int NB) { return (200 * 1024) / sk_stage_bytes(NB) < LMH_STAGES ? (200 * 1024) / sk_stage_bytes(NB) : LMH_STAGES; }
-__host__ __device__ constexpr int lmh_smem_bytes(int NB) { return lmh_stages(NB) * sk_stage_bytes(NB) + 1024 + 512 + 4 * NB * 8; }
+__host__ __device__ constexpr int lmh_smem_bytes(int NB, bool LSE = false) {
+    return lmh_stages(NB) * sk_stage_bytes(NB) + 1024 + 512 + 4 * NB * (LSE ? 12 : 8);
+}
 
 // (value, index) maximum with the first index on ties
 __device__ __forceinline__ void amax_merge(float& v, int& i, float ov, int oi) {
@@ -49,7 +61,21 @@ __device__ __forceinline__ void transpose_reduce32(float (&v)[32], int (&ix)[32]
     }
 }
 
-template <int NB>
+// the same butterfly as transpose_reduce32, summing: afterwards lane l holds sum over the warp's 32 lanes of v[l]
+__device__ __forceinline__ void transpose_sum32(float (&v)[32], int lane) {
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const bool up = (lane & off) != 0;
+#pragma unroll
+        for (int i = 0; i < off; i++) {
+            const float sv = up ? v[i] : v[i + off];
+            const float kv = up ? v[i + off] : v[i];
+            v[i] = kv + __shfl_xor_sync(0xffffffffu, sv, off);
+        }
+    }
+}
+
+template <int NB, bool LSE = false>
 __global__ void __launch_bounds__(256, 1)
 lmhead_argmax_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_constant__ CUtensorMap tmX, const LmHeadDev p) {
     constexpr int STAGES = lmh_stages(NB);
@@ -69,6 +95,7 @@ lmhead_argmax_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_const
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
     float* s_val = reinterpret_cast<float*>(smem + STAGES * STAGE_BYTES + 512);  // [4 warps][NB]
     int* s_idx = reinterpret_cast<int*>(s_val + 4 * NB);
+    float* s_sum = reinterpret_cast<float*>(s_idx + 4 * NB);  // [4 warps][NB], LSE only
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int t0 = (int)(((long long)blockIdx.x * p.tiles) / gridDim.x), t1 = (int)(((long long)(blockIdx.x + 1) * p.tiles) / gridDim.x);
@@ -173,6 +200,16 @@ lmhead_argmax_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_const
                     s_val[q * NB + c * CH + lane] = v[0];
                     s_idx[q * NB + c * CH + lane] = ix[0];
                 }
+                if constexpr (LSE) {
+                    const float wmax = v[0];
+#pragma unroll
+                    for (int j = 0; j < 32; j++) {
+                        const float mj = __shfl_sync(0xffffffffu, wmax, j);
+                        v[j] = (j < CH && row_ok) ? __expf(bf16_round(__uint_as_float(u[j < CH ? j : 0])) - mj) : 0.f;
+                    }
+                    transpose_sum32(v, lane);
+                    if (lane < CH) s_sum[q * NB + c * CH + lane] = v[0];
+                }
             }
             asm volatile("bar.sync 1, 128;" ::: "memory");  // the four epilogue warps
             for (int m = threadIdx.x - 128; m < NB && m < p.Mtok; m += 128) {  // 128 epilogue threads, up to 256 tokens
@@ -182,6 +219,15 @@ lmhead_argmax_kernel(const __grid_constant__ CUtensorMap tmW, const __grid_const
                 for (int w = 1; w < 4; w++) amax_merge(bv, bi, s_val[w * NB + m], s_idx[w * NB + m]);
                 p.amax_val[(size_t)m * p.tiles + t] = bv;
                 p.amax_idx[(size_t)m * p.tiles + t] = bi;
+                if constexpr (LSE) {  // a warp without valid rows has max -inf and sum 0
+                    float sum = 0.f;
+#pragma unroll
+                    for (int w = 0; w < 4; w++) {
+                        const float mw = s_val[w * NB + m];
+                        sum += mw == -INFINITY ? 0.f : s_sum[w * NB + m] * __expf(mw - bv);
+                    }
+                    p.amax_sum[(size_t)m * p.tiles + t] = sum;
+                }
             }
             asm volatile("bar.sync 1, 128;" ::: "memory");  // s_val / s_idx are reused by the next tile
         }

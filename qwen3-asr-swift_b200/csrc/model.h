@@ -98,6 +98,7 @@ struct BatchState {
     bool has_audio = false, mel_done = false, enc_done = false, prefill_done = false;
     bool sampler_on = false;   // decoder knobs active: full logits + sample_kernel instead of the fused argmax epilogue
     SamplingParams sampling;
+    bool logprobs_on = false;  // per-token log-probabilities: the LM head also reduces the log-sum-exp (q3asr_batch_set_logprobs)
     int steps_done = 0;
     // decode rows: the sequences still being decoded (B until a compaction drops the finished ones; stop_on_eos only)
     int dec_rows = 0;
@@ -125,9 +126,10 @@ struct BatchState {
     DevBuf kv_pool, rope_tab, rope_tab_t, page_tab, page_tab2, st_slot_seq;  // rope_tab_t: the table dimension-major (EPI_QKV)
      // page_tab: [B][pages_per_seq] (plan_pages)
     int rope_n = 0;          // positions tabulated in rope_tab
-    DevBuf amax_val, amax_idx, logits, logits_bf;
-    // decode state (device)
+    DevBuf amax_val, amax_idx, amax_sum, logits, logits_bf;  // amax_sum: per-tile sums of exp(z - tile max) (logprobs_on only)
+    // decode state (device); st_next_lp / st_out_lp: logprobs_on only
     DevBuf st_next_tok, st_next_val, st_cur_tok, st_pos, st_kv_len, st_out_ids, st_out_val, st_out_len, st_finished, st_scalars, st_forced;
+    DevBuf st_next_lp, st_out_lp;
     HostBuf h_stage, h_ints, h_out, h_pages;
     cudaGraphExec_t step_graph = nullptr;
     int graph_B = 0;
@@ -138,9 +140,9 @@ struct BatchState {
     }
     std::vector<DevBuf*> all() {
         return {&pcm, &raw_pcm, &mel_out, &mel_clips, &mel_gmax, &mel_tmin, &ints, &a1, &a2, &a3, &ex, &exn, &eqkv, &eatt, &effn, &audio,
-                &dx, &dxn, &dqkv, &dq, &dkc, &datt, &dact, &dlast, &dws, &dattn_part, &dattn_cnt, &dws2, &mega_tab, &mega_trace, &kv_pool, &rope_tab, &rope_tab_t, &page_tab, &page_tab2, &st_slot_seq, &amax_val, &amax_idx, &logits, &logits_bf,
+                &dx, &dxn, &dqkv, &dq, &dkc, &datt, &dact, &dlast, &dws, &dattn_part, &dattn_cnt, &dws2, &mega_tab, &mega_trace, &kv_pool, &rope_tab, &rope_tab_t, &page_tab, &page_tab2, &st_slot_seq, &amax_val, &amax_idx, &amax_sum, &logits, &logits_bf,
                 &st_next_tok, &st_next_val, &st_cur_tok, &st_pos, &st_kv_len, &st_out_ids, &st_out_val, &st_out_len, &st_finished,
-                &st_scalars, &st_forced};
+                &st_scalars, &st_forced, &st_next_lp, &st_out_lp};
     }
     ~BatchState() {
         for (DevBuf* b : all()) b->release();

@@ -964,6 +964,7 @@ __global__ void decode_advance_kernel(DecodeState s, int n_seqs) {
         if (!s.finished[q] && step < s.max_tokens) {
             s.out_ids[(size_t)q * s.max_tokens + step] = tok;
             if (s.out_val && s.next_val) s.out_val[(size_t)q * s.max_tokens + step] = s.next_val[i];
+            if (s.out_lp && s.next_lp) s.out_lp[(size_t)q * s.max_tokens + step] = s.next_lp[i];
             s.out_len[q] = step + 1;
             if (s.stop_on_eos && tok == s.eos) {
                 s.finished[q] = 1;
@@ -1021,11 +1022,21 @@ __device__ __forceinline__ unsigned long long splitmix64_dev(unsigned long long 
     return x ^ (x >> 31);
 }
 
-template <typename T>
+// (max, sum of exp(x - max)) pairs: the merge of two partial log-sum-exps (an empty side has max -inf and sum 0)
+__device__ __forceinline__ void lse_merge(float& m, float& s, float om, float os) {
+    const float M = fmaxf(m, om);
+    s = (m == -INFINITY ? 0.f : s * __expf(m - M)) + (om == -INFINITY ? 0.f : os * __expf(om - M));
+    m = M;
+}
+
+// LP: also the (max, sum of exp(x - max)) of the slice's RAW logits (before penalty / mask / noise) to part_rmax / part_rsum, for the
+// log-probability of the chosen token (argmax_lse_reduce); every thread walks its indices in ascending order and the merge tree is
+// fixed, so the sums depend on the vocabulary and the slice count only.
+template <typename T, bool LP>
 __global__ void __launch_bounds__(1024) sample_kernel(const T* __restrict__ logits, int ld, int vocab, const int32_t* __restrict__ gen_ids,
                                                        int gen_stride, const int* __restrict__ gen_len, SamplingParams sp,
                                                        const int* __restrict__ step, float* __restrict__ part_val,
-                                                       int* __restrict__ part_idx) {
+                                                       int* __restrict__ part_idx, float* __restrict__ part_rmax, float* __restrict__ part_rsum) {
     // grid (sequence, slice): gridDim.y CTAs share a row's vocabulary scan (the bitmaps are rebuilt by each, they are tiny);
     // argmax_reduce_kernel merges the slices (first maximum)
     ptx::grid_dep_launch();
@@ -1067,8 +1078,17 @@ __global__ void __launch_bounds__(1024) sample_kernel(const T* __restrict__ logi
     int bidx = 0x7fffffff;
     const int per = (vocab + gridDim.y - 1) / gridDim.y;
     const int i_end = min(vocab, ((int)blockIdx.y + 1) * per);
+    float rm = -INFINITY, rs = 0.f;  // LP: running (max, sum) of the raw logits
     for (int i = blockIdx.y * per + tid; i < i_end; i += blockDim.x) {
         float v = (float)row[i];
+        if constexpr (LP) {
+            if (v > rm) {
+                rs = (rm == -INFINITY ? 0.f : rs * __expf(rm - v)) + 1.f;
+                rm = v;
+            } else {
+                rs += __expf(v - rm);
+            }
+        }
         const unsigned int bit = 1u << (i & 31);
         if (seen[i >> 5] & bit) v = v > 0.f ? v / sp.repetition_penalty : v * sp.repetition_penalty;
         if (forbidden[i >> 5] & bit) v = -INFINITY;
@@ -1084,6 +1104,11 @@ __global__ void __launch_bounds__(1024) sample_kernel(const T* __restrict__ logi
         const int oi = __shfl_xor_sync(0xffffffffu, bidx, o);
         if (ob > best || (ob == best && oi < bidx)) { best = ob; bidx = oi; }
     }
+    __shared__ float s_rm[32], s_rs[32];
+    if constexpr (LP) {
+        for (int o = 16; o > 0; o >>= 1) lse_merge(rm, rs, __shfl_xor_sync(0xffffffffu, rm, o), __shfl_xor_sync(0xffffffffu, rs, o));
+        if ((tid & 31) == 0) { s_rm[tid >> 5] = rm; s_rs[tid >> 5] = rs; }
+    }
     if ((tid & 31) == 0) { s_best[tid >> 5] = best; s_idx[tid >> 5] = bidx; }
     __syncthreads();
     if (tid < 32) {
@@ -1094,6 +1119,15 @@ __global__ void __launch_bounds__(1024) sample_kernel(const T* __restrict__ logi
             const float ob = __shfl_xor_sync(0xffffffffu, best, o);
             const int oi = __shfl_xor_sync(0xffffffffu, bidx, o);
             if (ob > best || (ob == best && oi < bidx)) { best = ob; bidx = oi; }
+        }
+        if constexpr (LP) {
+            rm = tid < nw ? s_rm[tid] : -INFINITY;
+            rs = tid < nw ? s_rs[tid] : 0.f;
+            for (int o = 16; o > 0; o >>= 1) lse_merge(rm, rs, __shfl_xor_sync(0xffffffffu, rm, o), __shfl_xor_sync(0xffffffffu, rs, o));
+            if (tid == 0) {
+                part_rmax[(size_t)seq * gridDim.y + blockIdx.y] = rm;
+                part_rsum[(size_t)seq * gridDim.y + blockIdx.y] = rs;
+            }
         }
         if (tid == 0) {  // an all -inf slice reports index 0 of ITS slice start only through the value: the reducer keeps the first maximum
             part_val[(size_t)seq * gridDim.y + blockIdx.y] = best;
@@ -1292,7 +1326,7 @@ int sample_parts(int vocab) { return vocab >= 32768 ? 4 : 1; }
 
 void sample_launch(const bf16* logits_bf16, const float* logits_f32, int ld, int vocab, const int32_t* gen_ids, int gen_stride,
                    const int* gen_len, const SamplingParams& sp, const int* step, int n_seqs, float* part_val, int* part_idx,
-                   cudaStream_t st) {
+                   cudaStream_t st, float* part_rmax, float* part_rsum) {
     if (n_seqs <= 0) return;
     Q3_CHECK(vocab > 0 && vocab <= 160 * 1024, 1, "sample: vocabulary too large for the shared-memory bitmaps");
     Q3_CHECK((logits_bf16 != nullptr) != (logits_f32 != nullptr), 1, "sample: exactly one logits pointer");
@@ -1300,10 +1334,17 @@ void sample_launch(const bf16* logits_bf16, const float* logits_f32, int ld, int
     const size_t smem = (size_t)2 * ((vocab + 31) / 32) * sizeof(unsigned int);
     const int parts = sample_parts(vocab);
     const dim3 grid(n_seqs, parts);
-    if (logits_bf16)
-        launch_kernel(sample_kernel<bf16>, grid, 1024, smem, st, logits_bf16, ld, vocab, gen_ids, gen_stride, gen_len, sp, step, part_val, part_idx);
+    Q3_CHECK((part_rmax != nullptr) == (part_rsum != nullptr) && (part_rmax == nullptr || logits_bf16 != nullptr), 1,
+             "sample: raw (max, sum) outputs come in pairs, bf16 logits only");
+    if (part_rmax)
+        launch_kernel(sample_kernel<bf16, true>, grid, 1024, smem, st, logits_bf16, ld, vocab, gen_ids, gen_stride, gen_len, sp, step, part_val,
+                      part_idx, part_rmax, part_rsum);
+    else if (logits_bf16)
+        launch_kernel(sample_kernel<bf16, false>, grid, 1024, smem, st, logits_bf16, ld, vocab, gen_ids, gen_stride, gen_len, sp, step, part_val,
+                      part_idx, nullptr, nullptr);
     else
-        launch_kernel(sample_kernel<float>, grid, 1024, smem, st, logits_f32, ld, vocab, gen_ids, gen_stride, gen_len, sp, step, part_val, part_idx);
+        launch_kernel(sample_kernel<float, false>, grid, 1024, smem, st, logits_f32, ld, vocab, gen_ids, gen_stride, gen_len, sp, step, part_val,
+                      part_idx, nullptr, nullptr);
 }
 
 void fill_i32_launch(int* p, int v, size_t n, cudaStream_t st) {

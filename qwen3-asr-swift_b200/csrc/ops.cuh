@@ -87,6 +87,8 @@ struct DecodeState {
     int* kv_len;          // [n_seqs]
     int32_t* out_ids;     // [n_seqs, max_tokens]
     float* out_val;       // [n_seqs, max_tokens] or null
+    float* next_lp = nullptr;  // [n_seqs] log-probability of this step's token (input, may be null)
+    float* out_lp = nullptr;   // [n_seqs, max_tokens] or null
     int* out_len;         // [n_seqs]
     int* finished;        // [n_seqs]
     int* n_active;        // [1]
@@ -118,11 +120,12 @@ struct SamplingParams {
 // logits: [n_seqs, ld] (bf16 or fp32); gen_ids: [n_seqs, gen_stride] with gen_len[seq] valid entries; step: device counter that
 // varies the noise per decode step (may be null).  A row's vocabulary is scanned by sample_parts(vocab) CTAs; each writes its best
 // adjusted score and index to part_val / part_idx [n_seqs, sample_parts(vocab)], to be merged by argmax_reduce (gemm.cuh), which
-// keeps the first maximum.
+// keeps the first maximum.  part_rmax / part_rsum (bf16 logits only, may be null): per slice also the maximum and the sum of
+// exp(x - maximum) of the raw logits, for argmax_lse_reduce.
 int sample_parts(int vocab);
 void sample_launch(const bf16* logits_bf16, const float* logits_f32, int ld, int vocab, const int32_t* gen_ids, int gen_stride,
                    const int* gen_len, const SamplingParams& sp, const int* step, int n_seqs, float* part_val, int* part_idx,
-                   cudaStream_t st);
+                   cudaStream_t st, float* part_rmax = nullptr, float* part_rsum = nullptr);
 
 void fill_i32_launch(int* p, int v, size_t n, cudaStream_t st);
 void bf16_to_f32_launch(const bf16* in, float* out, size_t n, cudaStream_t st);

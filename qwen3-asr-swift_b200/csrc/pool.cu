@@ -34,6 +34,9 @@ struct q3asr_job {
     std::vector<int> rates;
     bool has_sampling = false;
     q3asr_sampling sampling{};
+    bool has_lp = false;     // submitted through q3asr_pool_submit_lp
+    bool waited = false;     // q3asr_job_wait returned Q3ASR_OK
+    std::vector<float> lp;   // [batch, max_tokens] log-probabilities (has_lp only)
     std::string error;
 };
 
@@ -43,7 +46,8 @@ thread_local std::string g_create_error;  // q3asr_pool_last_error(NULL): why th
 // One batch over the pool's handles (arguments checked by the caller, p->run_mu held).  May throw from its own host allocations or
 // thread creation; workers already started are joined first.
 int pool_run(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const int* sample_rates, int batch, const q3asr_prompt* prompts,
-             const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu, int32_t* ids_out, int* lens_out) {
+             const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu, int32_t* ids_out, int* lens_out,
+             float* lp_out) {
     const int G = (int)p->handles.size();
     if (max_batch_per_gpu <= 0) max_batch_per_gpu = 256;  // the widest batch the weight-streaming decode kernels take (512 x 30 s on one GPU, two workers: 11 460 audio-s/s against 10 840 at 128 and 9 390 at 64)
     // the scheduler's cost model and the length sort work on 16 kHz-equivalent lengths
@@ -76,14 +80,18 @@ int pool_run(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const i
                 }
                 std::vector<int32_t> ids((size_t)nb * max_tokens);
                 std::vector<int> lens(nb);
-                rc[g] = q3asr_transcribe_ids_opts(p->handles[g], pp.data(), nn.data(), sample_rates ? rr.data() : nullptr, nb,
-                                                  prompts ? pr.data() : nullptr, sampling, max_tokens, stop_on_eos, ids.data(), lens.data());
+                std::vector<float> lp(lp_out ? (size_t)nb * max_tokens : 0);
+                rc[g] = q3asr_transcribe_ids_lp(p->handles[g], pp.data(), nn.data(), sample_rates ? rr.data() : nullptr, nb,
+                                                prompts ? pr.data() : nullptr, sampling, max_tokens, stop_on_eos, ids.data(), lens.data(),
+                                                lp_out ? lp.data() : nullptr);
                 if (rc[g] != Q3ASR_OK) break;
                 for (int j = 0; j < nb; j++) {  // host-side result gather, original order
                     const int i = mine[s + j];
                     lens_out[i] = lens[j];
                     std::copy(ids.begin() + (size_t)j * max_tokens, ids.begin() + (size_t)j * max_tokens + lens[j],
                               ids_out + (size_t)i * max_tokens);
+                    if (lp_out)  // the whole row: the entries past lens[j] are zeros
+                        std::copy(lp.begin() + (size_t)j * max_tokens, lp.begin() + (size_t)(j + 1) * max_tokens, lp_out + (size_t)i * max_tokens);
                 }
             }
         } catch (const std::bad_alloc&) {
@@ -114,7 +122,7 @@ int pool_run(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const i
 
 int pool_transcribe_locked(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const int* sample_rates, int batch,
                            const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
-                           int max_batch_per_gpu, int32_t* ids_out, int* lens_out) {
+                           int max_batch_per_gpu, int32_t* ids_out, int* lens_out, float* lp_out) {
     if (pcm == nullptr || n_in == nullptr || ids_out == nullptr || lens_out == nullptr || batch <= 0 || max_tokens <= 0) {
         p->last_error = "pool_transcribe: null argument, empty batch or max_tokens <= 0";
         return Q3ASR_ERR_INVALID;
@@ -126,7 +134,8 @@ int pool_transcribe_locked(q3asr_pool* p, const float* const* pcm, const size_t*
                 return Q3ASR_ERR_INVALID;
             }
     try {
-        return pool_run(p, pcm, n_in, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu, ids_out, lens_out);
+        return pool_run(p, pcm, n_in, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu, ids_out, lens_out,
+                        lp_out);
     } catch (const std::bad_alloc&) {
         p->last_error = "pool_transcribe: out of host memory";
         return Q3ASR_ERR_NOMEM;
@@ -140,11 +149,11 @@ int pool_transcribe_locked(q3asr_pool* p, const float* const* pcm, const size_t*
 // overwritten by the next job's.
 int pool_transcribe(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const int* sample_rates, int batch,
                     const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu,
-                    int32_t* ids_out, int* lens_out, std::string* err) {
+                    int32_t* ids_out, int* lens_out, float* lp_out, std::string* err) {
     if (p == nullptr) return Q3ASR_ERR_INVALID;
     std::lock_guard<std::mutex> run_lock(p->run_mu);
     const int rc = pool_transcribe_locked(p, pcm, n_in, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu,
-                                          ids_out, lens_out);
+                                          ids_out, lens_out, lp_out);
     if (rc != Q3ASR_OK && err) *err = p->last_error;
     return rc;
 }
@@ -212,13 +221,20 @@ int q3asr_pool_transcribe_ids_opts(q3asr_pool* p, const float* const* pcm, const
                                    const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
                                    int max_batch_per_gpu, int32_t* ids_out, int* lens_out) {
     return pool_transcribe(p, pcm, n_in, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu, ids_out, lens_out,
-                           nullptr);
+                           nullptr, nullptr);
+}
+
+int q3asr_pool_transcribe_ids_lp(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const int* sample_rates, int batch,
+                                 const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
+                                 int max_batch_per_gpu, int32_t* ids_out, int* lens_out, float* logprobs_out) {
+    return pool_transcribe(p, pcm, n_in, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu, ids_out, lens_out,
+                           logprobs_out, nullptr);
 }
 
 // ---- submit / wait: the blocking call on a thread of its own, so the caller can load the next files meanwhile (SURVEY.md 8b) ----
-int q3asr_pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
-                      const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu,
-                      q3asr_job** out) {
+namespace {
+int pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch, const q3asr_prompt* prompts,
+                const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu, bool want_lp, q3asr_job** out) {
     if (out) *out = nullptr;
     if (p == nullptr || pcm == nullptr || n_samples == nullptr || batch <= 0 || max_tokens <= 0 || out == nullptr) return Q3ASR_ERR_INVALID;
     q3asr_job* j = nullptr;
@@ -228,6 +244,8 @@ int q3asr_pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_sa
         j->max_tokens = max_tokens;
         j->ids.assign((size_t)batch * max_tokens, 0);
         j->lens.assign((size_t)batch, 0);
+        j->has_lp = want_lp;
+        if (want_lp) j->lp.assign((size_t)batch * max_tokens, 0.f);
         if (prompts) j->prompts.assign(prompts, prompts + batch);  // the id arrays they point to stay the caller's, like the samples
         if (sample_rates) j->rates.assign(sample_rates, sample_rates + batch);
         if (sampling) {
@@ -240,7 +258,8 @@ int q3asr_pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_sa
         j->worker = std::thread([p, j, pp = std::move(pp), nn = std::move(nn), stop_on_eos, max_batch_per_gpu]() {
             j->rc = pool_transcribe(p, pp.data(), nn.data(), j->rates.empty() ? nullptr : j->rates.data(), j->batch,
                                     j->prompts.empty() ? nullptr : j->prompts.data(), j->has_sampling ? &j->sampling : nullptr,
-                                    j->max_tokens, stop_on_eos, max_batch_per_gpu, j->ids.data(), j->lens.data(), &j->error);
+                                    j->max_tokens, stop_on_eos, max_batch_per_gpu, j->ids.data(), j->lens.data(),
+                                    j->has_lp ? j->lp.data() : nullptr, &j->error);
             j->done.store(1, std::memory_order_release);
         });
     } catch (const std::exception&) {  // bad_alloc for the result buffers, or no thread to be had
@@ -249,6 +268,18 @@ int q3asr_pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_sa
     }
     *out = j;
     return Q3ASR_OK;
+}
+}  // namespace
+
+int q3asr_pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
+                      const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu,
+                      q3asr_job** out) {
+    return pool_submit(p, pcm, n_samples, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu, false, out);
+}
+int q3asr_pool_submit_lp(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
+                         const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu,
+                         q3asr_job** out) {
+    return pool_submit(p, pcm, n_samples, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu, true, out);
 }
 
 int q3asr_job_done(const q3asr_job* j) { return j != nullptr && j->done.load(std::memory_order_acquire) != 0; }
@@ -259,6 +290,13 @@ int q3asr_job_wait(q3asr_job* j, int32_t* ids_out, int* lens_out) {
     if (j->rc != Q3ASR_OK) return j->rc;
     std::copy(j->ids.begin(), j->ids.end(), ids_out);
     std::copy(j->lens.begin(), j->lens.end(), lens_out);
+    j->waited = true;
+    return Q3ASR_OK;
+}
+
+int q3asr_job_logprobs(const q3asr_job* j, float* out) {
+    if (j == nullptr || out == nullptr || !j->has_lp || !j->waited) return Q3ASR_ERR_INVALID;
+    std::copy(j->lp.begin(), j->lp.end(), out);
     return Q3ASR_OK;
 }
 

@@ -125,6 +125,13 @@ struct TranscriptionSegment {  // StreamingASR.swift:7-21
     float startTime = 0.f, endTime = 0.f;
     bool isFinal = true;
     int segmentIndex = 0;
+    float avgLogprob = 0.f;  // transcribeLong(..., withConfidence = true) only: mean token log-probability of the window
+};
+
+// a transcript with its score: mean token log-probability (EOS included, include/q3asr.h); confidence = exp(avgLogprob)
+struct ScoredTranscript {
+    std::string text;
+    float avgLogprob = 0.f;
 };
 
 class Qwen3ASRModel;
@@ -236,8 +243,10 @@ class Qwen3ASRModel {
     std::vector<std::vector<int32_t>> transcribeIds(const std::vector<const std::vector<float>*>& audio, int maxTokens = 448,
                                                     bool stopOnEos = true, const std::vector<int32_t>& contextIds = {},
                                                     const std::vector<int32_t>& languageIds = {}, std::string* error = nullptr,
-                                                    const std::vector<int>& sampleRates = {}, const Qwen3DecodingOptions* options = nullptr) {
+                                                    const std::vector<int>& sampleRates = {}, const Qwen3DecodingOptions* options = nullptr,
+                                                    std::vector<std::vector<float>>* logprobs = nullptr) {
         const int n = (int)audio.size();
+        if (logprobs) logprobs->assign(n, {});
         if (!sampleRates.empty() && (int)sampleRates.size() != n) {
             if (error) *error = "sampleRates must have one entry per utterance";
             return std::vector<std::vector<int32_t>>(n);
@@ -255,37 +264,36 @@ class Qwen3ASRModel {
         std::vector<std::vector<int32_t>> out(n);
         q3asr_sampling samp{1.0f, 0, 0.0f, 0, 0};
         if (options) samp = q3asr_sampling{options->repetitionPenalty, options->noRepeatNgramSize, options->temperature, options->seed, 0};
-        int rc = q3asr_transcribe_ids_opts(h_, pcm.data(), len.data(), sampleRates.empty() ? nullptr : sampleRates.data(), n, prompts.data(),
-                                           options ? &samp : nullptr, maxTokens, stopOnEos ? 1 : 0, ids.data(), lens.data());
+        std::vector<float> lp(logprobs ? (size_t)n * maxTokens : 0);
+        int rc = q3asr_transcribe_ids_lp(h_, pcm.data(), len.data(), sampleRates.empty() ? nullptr : sampleRates.data(), n, prompts.data(),
+                                         options ? &samp : nullptr, maxTokens, stopOnEos ? 1 : 0, ids.data(), lens.data(),
+                                         logprobs ? lp.data() : nullptr);
         if (rc != Q3ASR_OK) {
             if (error) *error = q3asr_last_error(h_);
             return out;
         }
-        for (int i = 0; i < n; i++) out[i].assign(ids.begin() + (size_t)i * maxTokens, ids.begin() + (size_t)i * maxTokens + lens[i]);
+        for (int i = 0; i < n; i++) {
+            out[i].assign(ids.begin() + (size_t)i * maxTokens, ids.begin() + (size_t)i * maxTokens + lens[i]);
+            if (logprobs) (*logprobs)[i].assign(lp.begin() + (size_t)i * maxTokens, lp.begin() + (size_t)i * maxTokens + lens[i]);
+        }
         return out;
     }
 
     std::vector<std::string> transcribeBatch(const std::vector<const std::vector<float>*>& audio, const std::optional<std::string>& language = {},
                                              int maxTokens = 448, const std::optional<std::string>& context = {},
                                              const std::vector<int>& sampleRates = {}, const Qwen3DecodingOptions* options = nullptr) {
-        const size_t n = audio.size();
-        if (!isLoaded()) return std::vector<std::string>(n, "[Audio encoded] - Text decoder not loaded");  // Qwen3ASR.swift:116-119
-        std::vector<int32_t> ctx, lang;
-        if (tok_.encode) {
-            if (context) ctx = tok_.encode(*context);                  // Qwen3ASR.swift:203-206
-            if (language) lang = tok_.encode("language " + *language);  // Qwen3ASR.swift:228-232
-        }
-        std::string err;
-        auto ids = transcribeIds(audio, maxTokens, true, ctx, lang, &err, sampleRates, options);
-        std::vector<std::string> out(n);
-        for (size_t i = 0; i < n; i++) {
-            if (!err.empty()) {
-                out[i] = "[Qwen3-ASR B200 error: " + err + "]";
-                continue;
-            }
-            out[i] = textFromIds(tok_, ids[i]);
-        }
+        std::vector<std::string> out;
+        for (ScoredTranscript& t : run(audio, language, maxTokens, context, sampleRates, options, false)) out.push_back(std::move(t.text));
         return out;
+    }
+
+    // transcribeBatch plus each utterance's mean token log-probability (0 for an utterance without tokens or after an error)
+    std::vector<ScoredTranscript> transcribeBatchWithConfidence(const std::vector<const std::vector<float>*>& audio,
+                                                                const std::optional<std::string>& language = {}, int maxTokens = 448,
+                                                                const std::optional<std::string>& context = {},
+                                                                const std::vector<int>& sampleRates = {},
+                                                                const Qwen3DecodingOptions* options = nullptr) {
+        return run(audio, language, maxTokens, context, sampleRates, options, true);
     }
 
     // trimmingCharacters(in: .whitespaces): Unicode space separators (Zs) and TAB at either end, not line breaks
@@ -322,7 +330,8 @@ class Qwen3ASRModel {
 
     // Long-form audio (BASELINE config 5): fixed windows of windowSeconds, each an independent utterance, `batch` windows per pass.
     std::vector<TranscriptionSegment> transcribeLong(const std::vector<float>& audio, int sampleRate = 16000, float windowSeconds = 30.f,
-                                                     int maxTokens = 448, int batch = 64, const std::optional<std::string>& language = {}) {
+                                                     int maxTokens = 448, int batch = 64, const std::optional<std::string>& language = {},
+                                                     bool withConfidence = false) {
         std::vector<TranscriptionSegment> out;
         const size_t window = (size_t)((double)windowSeconds * sampleRate + 0.5);
         const size_t minTail = std::max<size_t>(160, ((size_t)160 * sampleRate + 15999) / 16000);
@@ -338,10 +347,11 @@ class Qwen3ASRModel {
                 clips[i].assign(audio.begin() + starts[b0 + i], audio.begin() + starts[b0 + i] + lens[b0 + i]);
                 ptrs[i] = &clips[i];
             }
-            auto texts = transcribeBatch(ptrs, language, maxTokens, {}, std::vector<int>((size_t)nb, sampleRate));
+            auto texts = run(ptrs, language, maxTokens, {}, std::vector<int>((size_t)nb, sampleRate), nullptr, withConfidence);
             for (int i = 0; i < nb; i++) {
                 TranscriptionSegment seg;
-                seg.text = texts[i];
+                seg.text = texts[i].text;
+                seg.avgLogprob = texts[i].avgLogprob;
                 seg.startTime = (float)((double)starts[b0 + i] / sampleRate);
                 seg.endTime = (float)((double)(starts[b0 + i] + lens[b0 + i]) / sampleRate);
                 seg.segmentIndex = b0 + i;
@@ -358,6 +368,35 @@ class Qwen3ASRModel {
     q3asr_handle* handle() const { return h_; }
 
   private:
+    std::vector<ScoredTranscript> run(const std::vector<const std::vector<float>*>& audio, const std::optional<std::string>& language,
+                                      int maxTokens, const std::optional<std::string>& context, const std::vector<int>& sampleRates,
+                                      const Qwen3DecodingOptions* options, bool scored) {
+        const size_t n = audio.size();
+        if (!isLoaded()) return std::vector<ScoredTranscript>(n, {"[Audio encoded] - Text decoder not loaded", 0.f});  // Qwen3ASR.swift:116-119
+        std::vector<int32_t> ctx, lang;
+        if (tok_.encode) {
+            if (context) ctx = tok_.encode(*context);                  // Qwen3ASR.swift:203-206
+            if (language) lang = tok_.encode("language " + *language);  // Qwen3ASR.swift:228-232
+        }
+        std::string err;
+        std::vector<std::vector<float>> lp;
+        auto ids = transcribeIds(audio, maxTokens, true, ctx, lang, &err, sampleRates, options, scored ? &lp : nullptr);
+        std::vector<ScoredTranscript> out(n);
+        for (size_t i = 0; i < n; i++) {
+            if (!err.empty()) {
+                out[i].text = "[Qwen3-ASR B200 error: " + err + "]";
+                continue;
+            }
+            out[i].text = textFromIds(tok_, ids[i]);
+            if (scored && !lp[i].empty()) {
+                double sum = 0;
+                for (float v : lp[i]) sum += v;
+                out[i].avgLogprob = (float)(sum / lp[i].size());
+            }
+        }
+        return out;
+    }
+
     Qwen3ASRModel(ASRModelSize size, int device) {
         q3asr_config cfg;
         q3asr_config_preset(size == ASRModelSize::large ? "1.7B" : "0.6B", &cfg);

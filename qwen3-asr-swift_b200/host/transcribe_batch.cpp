@@ -9,6 +9,9 @@
 //
 //   transcribe_batch <inputDir> [--output-dir D] [--model 0.6B|1.7B] [--model-dir DIR] [--language L] [--extensions wav]
 //                    [--jsonl] [--batch N] [--max-tokens N] [--window-seconds S] [--devices 0,1,...] [--workers-per-gpu W] [--list]
+//                    [--confidence]
+// --confidence adds each file's average token log-probability (over all its windows, EOS included: include/q3asr.h) to its JSONL
+// record ("avg_logprob") and progress line — the score a caller uses to flag hallucinated or low-quality output.
 // Two pool workers per GPU by default: the decode steps of two batches in flight on one GPU interleave (each is a chain of
 // latency-bound launches), which measured +24 % aggregate throughput over one batch at a time (tools/pool_concurrency.py).
 // Without --model-dir the weights are random-init (this repo has no checkpoint offline); --list only prints the files.
@@ -80,6 +83,8 @@ static std::vector<fs::path> find_audio_files(const std::string& dir, const std:
 struct Item {
     std::string name, error, text;
     double duration = 0, time = 0;
+    double lp_sum = 0;  // --confidence: sum and count of the token log-probabilities of the file's windows
+    long lp_n = 0;
 };
 struct Unit { size_t item; std::vector<float> samples; int rate; };
 
@@ -97,7 +102,7 @@ struct Group {
 int main(int argc, char** argv) {
     std::string inputDir, outputDir, model = "0.6B", modelDir, extensions = "wav,flac,mp3", devicesArg = "0";
     std::optional<std::string> language;
-    bool jsonl = false, listOnly = false;
+    bool jsonl = false, listOnly = false, confidence = false;
     int batch = 256, maxTokens = 448, workersPerGpu = 2;
     float windowSeconds = 30.f;
     for (int i = 1; i < argc; i++) {
@@ -110,6 +115,7 @@ int main(int argc, char** argv) {
         else if (a == "--extensions") extensions = val();
         else if (a == "--jsonl") jsonl = true;
         else if (a == "--list") listOnly = true;
+        else if (a == "--confidence") confidence = true;
         else if (a == "--batch") batch = std::max(1, atoi(val().c_str()));
         else if (a == "--max-tokens") maxTokens = std::max(1, atoi(val().c_str()));
         else if (a == "--window-seconds") windowSeconds = (float)atof(val().c_str());
@@ -189,17 +195,22 @@ int main(int argc, char** argv) {
     auto submit = [&](Group* g, int tokens) {
         g->t0 = now_s();
         if (g->units.empty()) return true;
-        return q3asr_pool_submit(pool, g->pcm.data(), g->n.data(), g->rates.data(), (int)g->units.size(), g->prompts.data(), nullptr, tokens, 1,
-                                 batch, &g->job) == Q3ASR_OK;
+        return (confidence ? q3asr_pool_submit_lp : q3asr_pool_submit)(pool, g->pcm.data(), g->n.data(), g->rates.data(), (int)g->units.size(),
+                                                                      g->prompts.data(), nullptr, tokens, 1, batch, &g->job) == Q3ASR_OK;
     };
     double totalInference = 0;
     std::vector<int32_t> ids;
     std::vector<int> lens;
+    std::vector<float> lps;
     auto finish = [&](Group* g, int tokens, bool record) {
         if (g->job != nullptr) {
             ids.assign(g->units.size() * (size_t)tokens, 0);
             lens.assign(g->units.size(), 0);
-            const int rc = q3asr_job_wait(g->job, ids.data(), lens.data());
+            int rc = q3asr_job_wait(g->job, ids.data(), lens.data());
+            if (rc == Q3ASR_OK && confidence) {
+                lps.assign(g->units.size() * (size_t)tokens, 0.f);
+                rc = q3asr_job_logprobs(g->job, lps.data());
+            }
             const double elapsed = now_s() - g->t0;
             if (record) {
                 totalInference += elapsed;
@@ -212,6 +223,8 @@ int main(int argc, char** argv) {
                         continue;
                     }
                     std::vector<int32_t> t(ids.begin() + k * (size_t)tokens, ids.begin() + k * (size_t)tokens + lens[k]);
+                    if (confidence)
+                        for (int s = 0; s < lens[k]; s++) { it.lp_sum += lps[k * (size_t)tokens + s]; it.lp_n++; }
                     if (!t.empty() && t.back() == Q3ASR_EOS_TOKEN) t.pop_back();
                     if (!it.text.empty()) it.text += " ";
                     it.text += Qwen3ASRModel::textFromIds(tok, t);
@@ -259,9 +272,16 @@ int main(int argc, char** argv) {
         }
         totalAudio += it.duration;
         const double rtf = it.time / std::max(it.duration, 0.001);
-        if (jsonl)
+        const double avg_lp = it.lp_n ? it.lp_sum / it.lp_n : 0.0;
+        if (jsonl && confidence)
+            printf("{\"file\":\"%s\",\"text\":\"%s\",\"time\":%.3f,\"rtf\":%.4f,\"duration\":%.2f,\"avg_logprob\":%.6f}\n",
+                   json_escape(it.name).c_str(), json_escape(it.text).c_str(), it.time, rtf, it.duration, avg_lp);
+        else if (jsonl)
             printf("{\"file\":\"%s\",\"text\":\"%s\",\"time\":%.3f,\"rtf\":%.4f,\"duration\":%.2f}\n", json_escape(it.name).c_str(),
                    json_escape(it.text).c_str(), it.time, rtf, it.duration);
+        else if (confidence)
+            printf("  [%zu/%zu] (%.0f%%) %s: %s  (%.2fs, RTF=%.3f, avg_logprob=%.3f)\n", i + 1, items.size(), 100.0 * (i + 1) / items.size(),
+                   it.name.c_str(), it.text.c_str(), it.time, rtf, avg_lp);
         else
             printf("  [%zu/%zu] (%.0f%%) %s: %s  (%.2fs, RTF=%.3f)\n", i + 1, items.size(), 100.0 * (i + 1) / items.size(), it.name.c_str(),
                    it.text.c_str(), it.time, rtf);

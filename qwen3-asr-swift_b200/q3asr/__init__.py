@@ -90,6 +90,8 @@ EXPORTS = [
     "q3asr_transcribe_ids_opts", "q3asr_batch_set_sampling", "q3asr_pick_next_token",
     "q3asr_align_indices", "q3asr_enforce_monotonicity", "q3asr_lis_positions", "q3asr_trailing_plateau_start",
     "q3asr_pool_transcribe_ids_opts", "q3asr_pool_submit", "q3asr_job_done", "q3asr_job_wait", "q3asr_job_last_error", "q3asr_job_free",
+    "q3asr_transcribe_ids_lp", "q3asr_batch_set_logprobs", "q3asr_batch_download_logprobs", "q3asr_pool_transcribe_ids_lp",
+    "q3asr_pool_submit_lp", "q3asr_job_logprobs",
 ]
 
 _lib = None
@@ -196,6 +198,12 @@ def lib():
         L.q3asr_lis_positions.argtypes = [vp, ci, vp, ctypes.POINTER(ci)]
         L.q3asr_trailing_plateau_start.argtypes = [vp, ci, ctypes.c_float, ci]
         L.q3asr_pick_next_token.argtypes = [vp, vp, ci, vp, ci, ctypes.POINTER(Sampling), ci, ctypes.POINTER(ctypes.c_int32)]
+        L.q3asr_transcribe_ids_lp.argtypes = [vp, vp, vp, vp, ci, vp, ctypes.POINTER(Sampling), ci, ci, vp, vp, vp]
+        L.q3asr_batch_set_logprobs.argtypes = [vp, ci]
+        L.q3asr_batch_download_logprobs.argtypes = [vp, vp, ci]
+        L.q3asr_pool_transcribe_ids_lp.argtypes = [vp, vp, vp, vp, ci, vp, ctypes.POINTER(Sampling), ci, ci, ci, vp, vp, vp]
+        L.q3asr_pool_submit_lp.argtypes = [vp, vp, vp, vp, ci, vp, ctypes.POINTER(Sampling), ci, ci, ci, ctypes.POINTER(vp)]
+        L.q3asr_job_logprobs.argtypes = [vp, vp]
         _lib = L
     return _lib
 
@@ -335,6 +343,13 @@ def longform_plan(n_samples, window, min_tail=160):
     if rc != OK:
         raise Q3Error(rc, lib().q3asr_io_last_error().decode())
     return [(int(starts[i]), int(lens[i])) for i in range(cnt.value)]
+
+
+def avg_logprob(logprobs):
+    """Utterance score of one utterance's per-token log-probabilities (include/q3asr.h): their mean, EOS included; exp() of it is
+    the confidence.  An empty utterance scores 0."""
+    lp = np.asarray(logprobs, dtype=np.float64)
+    return float(lp.mean()) if lp.size else 0.0
 
 
 def f32_to_bf16_bits(x):
@@ -582,15 +597,25 @@ class Qwen3ASRModel:
         return out[:ntok.value].copy()
 
     def transcribe_ids(self, clips, max_tokens=448, stop_on_eos=True, prompts=None, sample_rates=None, options=None,
-                       force_device_sampler=False):
+                       force_device_sampler=False, return_logprobs=False):
         """Batched transcription -> list of int32 id arrays (EOS included when it stops the loop).  sample_rates: per-clip
         rates; clips not at 16 kHz are converted on the device (AudioPreprocessing.swift:323-337).  options: a
-        Qwen3DecodingOptions whose decoder knobs (repetition penalty, no-repeat n-gram, temperature) run as a device kernel."""
+        Qwen3DecodingOptions whose decoder knobs (repetition penalty, no-repeat n-gram, temperature) run as a device kernel.
+        return_logprobs: (ids, logprobs) lists instead, logprobs[i] the float32 log-probability of every id (q3asr_transcribe_ids_lp)."""
         clips = [np.ascontiguousarray(c, dtype=np.float32) for c in clips]
         n = np.array([c.size for c in clips], dtype=np.uint64)
         ids = np.zeros((len(clips), max_tokens), dtype=np.int32)
         lens = np.zeros(len(clips), dtype=np.int32)
         pp = _PromptPack(prompts, len(clips))
+        if return_logprobs:
+            lp = np.zeros((len(clips), max_tokens), dtype=np.float32)
+            sr = None if sample_rates is None else np.ascontiguousarray(sample_rates, dtype=np.int32)
+            samp = None if options is None else options.c_struct(force_device_sampler)
+            self._ck(lib().q3asr_transcribe_ids_lp(self._h, ctypes.cast(_ptr_array(clips), ctypes.c_void_p), n.ctypes.data,
+                                                   sr.ctypes.data if sr is not None else None, len(clips), pp.ptr,
+                                                   ctypes.byref(samp) if samp is not None else None, int(max_tokens),
+                                                   int(bool(stop_on_eos)), ids.ctypes.data, lens.ctypes.data, lp.ctypes.data))
+            return ([ids[i, :lens[i]].copy() for i in range(len(clips))], [lp[i, :lens[i]].copy() for i in range(len(clips))])
         if options is not None:
             sr = None if sample_rates is None else np.ascontiguousarray(sample_rates, dtype=np.int32)
             samp = options.c_struct(force_device_sampler)
@@ -823,6 +848,15 @@ class Qwen3ASRModel:
     def batch_run(self, stages=STAGE_ALL, max_tokens=128, stop_on_eos=False):
         self._ck(lib().q3asr_batch_run(self._h, int(stages), int(max_tokens), int(bool(stop_on_eos))))
 
+    def batch_set_logprobs(self, enable=True):
+        self._ck(lib().q3asr_batch_set_logprobs(self._h, int(bool(enable))))
+
+    def batch_download_logprobs(self, batch, max_tokens):
+        """[batch, max_tokens] float32, zeros past each utterance's length"""
+        lp = np.zeros((batch, max(max_tokens, 1)), dtype=np.float32)
+        self._ck(lib().q3asr_batch_download_logprobs(self._h, lp.ctypes.data, int(max_tokens)))
+        return lp[:, :max_tokens]
+
     def batch_download(self, batch, max_tokens):
         ids = np.zeros((batch, max(max_tokens, 1)), dtype=np.int32)
         lens = np.zeros(batch, dtype=np.int32)
@@ -873,6 +907,8 @@ class Qwen3ASRModel:
             out = np.empty((M, N), dtype=np.float32)
         elif epi in (EPI_ARGMAX, 7):  # 7: the decode-step LM-head kernel (lmhead.cuh)
             out = np.empty(M, dtype=np.int32)
+        elif epi in (8, 9):  # 8 / 9: the LM-head kernel / EPI_ARGMAX with the log-sum-exp: ids [M], then float32 logprobs [M]
+            out = np.empty(2 * M, dtype=np.int32)
         elif epi == EPI_SWIGLU:
             out = np.empty((M, N // 2), dtype=np.uint16)
         else:
@@ -880,6 +916,8 @@ class Qwen3ASRModel:
         self._ck(lib().q3asr_debug_gemm(self._h, a.ctypes.data, w.ctypes.data, b.ctypes.data if b is not None else None,
                                         r.ctypes.data if r is not None else None, M, N, K, int(epi), int(bool(gelu)), int(bn),
                                         int(bool(simt)), out.ctypes.data))
+        if epi in (8, 9):
+            return out[:M].copy(), out[M:].view(np.float32).copy()
         return bf16_bits_to_f32(out) if out.dtype == np.uint16 else out
 
     def debug_attention(self, q, k, v, segs, heads, group, causal, scale, kernel=0):
@@ -985,24 +1023,31 @@ class Pool:
         if rc != OK:
             raise Q3Error(rc, "pool_create failed: " + lib().q3asr_pool_last_error(None).decode())
 
-    def transcribe_ids(self, clips, max_tokens=448, stop_on_eos=True, max_batch_per_gpu=64, sample_rates=None, options=None):
+    def transcribe_ids(self, clips, max_tokens=448, stop_on_eos=True, max_batch_per_gpu=64, sample_rates=None, options=None,
+                       return_logprobs=False):
         clips = [np.ascontiguousarray(c, dtype=np.float32) for c in clips]
         n = np.array([c.size for c in clips], dtype=np.uint64)
         ids = np.zeros((len(clips), max_tokens), dtype=np.int32)
         lens = np.zeros(len(clips), dtype=np.int32)
         sr = None if sample_rates is None else np.ascontiguousarray(sample_rates, dtype=np.int32)
         samp = None if options is None else options.c_struct()
-        rc = lib().q3asr_pool_transcribe_ids_opts(self._p, ctypes.cast(_ptr_array(clips), ctypes.c_void_p), n.ctypes.data,
-                                                  sr.ctypes.data if sr is not None else None, len(clips), None,
-                                                  ctypes.byref(samp) if samp is not None else None, int(max_tokens),
-                                                  int(bool(stop_on_eos)), int(max_batch_per_gpu), ids.ctypes.data, lens.ctypes.data)
+        args = (self._p, ctypes.cast(_ptr_array(clips), ctypes.c_void_p), n.ctypes.data, sr.ctypes.data if sr is not None else None, len(clips),
+                None, ctypes.byref(samp) if samp is not None else None, int(max_tokens), int(bool(stop_on_eos)), int(max_batch_per_gpu),
+                ids.ctypes.data, lens.ctypes.data)
+        if return_logprobs:
+            lp = np.zeros((len(clips), max_tokens), dtype=np.float32)
+            rc = lib().q3asr_pool_transcribe_ids_lp(*args, lp.ctypes.data)
+        else:
+            rc = lib().q3asr_pool_transcribe_ids_opts(*args)
         if rc != OK:
             raise Q3Error(rc, lib().q3asr_pool_last_error(self._p).decode())
-        return [ids[i, :lens[i]].copy() for i in range(len(clips))]
+        out = [ids[i, :lens[i]].copy() for i in range(len(clips))]
+        return (out, [lp[i, :lens[i]].copy() for i in range(len(clips))]) if return_logprobs else out
 
-    def submit(self, clips, max_tokens=448, stop_on_eos=True, max_batch_per_gpu=64, sample_rates=None, options=None):
-        """Asynchronous transcribe_ids: returns a PoolJob whose wait() gives the ids; the clips are kept alive by the job."""
-        return PoolJob(self, clips, max_tokens, stop_on_eos, max_batch_per_gpu, sample_rates, options)
+    def submit(self, clips, max_tokens=448, stop_on_eos=True, max_batch_per_gpu=64, sample_rates=None, options=None, return_logprobs=False):
+        """Asynchronous transcribe_ids: returns a PoolJob whose wait() gives the ids (and log-probabilities with return_logprobs);
+        the clips are kept alive by the job."""
+        return PoolJob(self, clips, max_tokens, stop_on_eos, max_batch_per_gpu, sample_rates, options, return_logprobs)
 
     def close(self):
         if self._p:
@@ -1019,14 +1064,16 @@ class Pool:
 class PoolJob:
     """q3asr_pool_submit / q3asr_job_wait: a batch running on the library's own thread."""
 
-    def __init__(self, pool, clips, max_tokens, stop_on_eos, max_batch_per_gpu, sample_rates, options):
+    def __init__(self, pool, clips, max_tokens, stop_on_eos, max_batch_per_gpu, sample_rates, options, return_logprobs=False):
         self._clips = [np.ascontiguousarray(c, dtype=np.float32) for c in clips]
         self._n = np.array([c.size for c in self._clips], dtype=np.uint64)
         self._sr = None if sample_rates is None else np.ascontiguousarray(sample_rates, dtype=np.int32)
         self._samp = None if options is None else options.c_struct()
         self._max_tokens = int(max_tokens)
+        self._lp = bool(return_logprobs)
         self._j = ctypes.c_void_p()
-        rc = lib().q3asr_pool_submit(pool._p, ctypes.cast(_ptr_array(self._clips), ctypes.c_void_p), self._n.ctypes.data,
+        submit = lib().q3asr_pool_submit_lp if self._lp else lib().q3asr_pool_submit
+        rc = submit(pool._p, ctypes.cast(_ptr_array(self._clips), ctypes.c_void_p), self._n.ctypes.data,
                                      self._sr.ctypes.data if self._sr is not None else None, len(self._clips), None,
                                      ctypes.byref(self._samp) if self._samp is not None else None, self._max_tokens, int(bool(stop_on_eos)),
                                      int(max_batch_per_gpu), ctypes.byref(self._j))
@@ -1045,8 +1092,15 @@ class PoolJob:
             msg = lib().q3asr_job_last_error(self._j).decode()
             self.free()
             raise Q3Error(rc, msg)
+        if self._lp:
+            lp = np.zeros((len(self._clips), self._max_tokens), dtype=np.float32)
+            rc = lib().q3asr_job_logprobs(self._j, lp.ctypes.data)
+            self.free()
+            if rc != OK:
+                raise Q3Error(rc, "job_logprobs failed")
         self.free()
-        return [ids[i, :lens[i]].copy() for i in range(len(self._clips))]
+        out = [ids[i, :lens[i]].copy() for i in range(len(self._clips))]
+        return (out, [lp[i, :lens[i]].copy() for i in range(len(self._clips))]) if self._lp else out
 
     def free(self):
         if self._j:

@@ -108,13 +108,29 @@ public final class Qwen3ASRB200Model {
     /// Batched greedy transcription: utterances are independent, the library batches them on the GPU.
     public func transcribeBatch(audio: [[Float]], language: String? = nil, maxTokens: Int = 448, context: String? = nil,
                                 sampleRates: [Int]? = nil, options: Qwen3DecodingOptions? = nil) -> [String] {
+        return run(audio: audio, language: language, maxTokens: maxTokens, context: context, sampleRates: sampleRates, options: options,
+                   scored: false).map { $0.text }
+    }
+
+    /// transcribeBatch plus each utterance's confidence = exp(mean token log-probability, EOS included) — the value the reference's
+    /// C bridge carries in sc_transcription_result_t.confidence (VoicePipeline.swift:374-411); 0 for an utterance without tokens.
+    public func transcribeBatchWithConfidence(audio: [[Float]], language: String? = nil, maxTokens: Int = 448, context: String? = nil,
+                                              sampleRates: [Int]? = nil, options: Qwen3DecodingOptions? = nil)
+        -> [(text: String, confidence: Float)] {
+        return run(audio: audio, language: language, maxTokens: maxTokens, context: context, sampleRates: sampleRates, options: options,
+                   scored: true)
+    }
+
+    private func run(audio: [[Float]], language: String?, maxTokens: Int, context: String?, sampleRates: [Int]?,
+                     options: Qwen3DecodingOptions?, scored: Bool) -> [(text: String, confidence: Float)] {
         guard q3asr_is_loaded(handle) != 0 else {
-            return audio.map { _ in "[Audio encoded] - Text decoder not loaded" }   // Qwen3ASR.swift:116-119
+            return audio.map { _ in ("[Audio encoded] - Text decoder not loaded", 0) }   // Qwen3ASR.swift:116-119
         }
         let n = audio.count
         let (ctx, lang) = promptIds(language: language, context: context)
         var ids = [Int32](repeating: 0, count: n * maxTokens)
         var lens = [Int32](repeating: 0, count: n)
+        var lp = [Float](repeating: 0, count: scored ? n * maxTokens : 0)
         var sizes = audio.map { $0.count }
         // borrow every clip's storage for the duration of the call
         var ptrs = [UnsafePointer<Float>?](repeating: nil, count: n)
@@ -134,22 +150,27 @@ public final class Qwen3ASRB200Model {
                                           no_repeat_ngram_size: Int32(options?.noRepeatNgramSize ?? 0),
                                           temperature: options?.temperature ?? 0.0,
                                           seed: UInt64.random(in: 0 ... UInt64.max), force_device_sampler: 0)
-                return withAll(0) {
-                    q3asr_transcribe_ids_opts(handle, &ptrs, &sizes, &rates, Int32(n), &prompts, &samp, Int32(maxTokens), 1, &ids, &lens)
+                return lp.withUnsafeMutableBufferPointer { lpb in
+                    withAll(0) {
+                        q3asr_transcribe_ids_lp(handle, &ptrs, &sizes, &rates, Int32(n), &prompts, &samp, Int32(maxTokens), 1, &ids, &lens,
+                                                scored ? lpb.baseAddress : nil)
+                    }
                 }
             }
         }
         if rc != Q3ASR_OK {
             let msg = String(cString: q3asr_last_error(handle))
-            return audio.map { _ in "[Qwen3-ASR B200 error: \(msg)]" }             // cf. CoreMLASRModel.swift:299-305
+            return audio.map { _ in ("[Qwen3-ASR B200 error: \(msg)]", 0) }             // cf. CoreMLASRModel.swift:299-305
         }
         return (0..<n).map { i in
-            var toks = Array(ids[(i * maxTokens)..<(i * maxTokens + Int(lens[i]))]).map(Int.init)
+            let len = Int(lens[i])
+            let conf: Float = scored && len > 0 ? exp(lp[(i * maxTokens)..<(i * maxTokens + len)].reduce(0, +) / Float(len)) : 0
+            var toks = Array(ids[(i * maxTokens)..<(i * maxTokens + len)]).map(Int.init)
             if toks.last == Int(Q3ASR_EOS_TOKEN) { toks.removeLast() }
-            guard let tokenizer = tokenizer else { return toks.map(String.init).joined(separator: " ") } // id-string fallback, Qwen3ASR.swift:283-289
+            guard let tokenizer = tokenizer else { return (toks.map(String.init).joined(separator: " "), conf) } // id-string fallback, Qwen3ASR.swift:283-289
             let raw = tokenizer.decode(tokens: toks)
-            if let r = raw.range(of: "<asr_text>") { return String(raw[r.upperBound...]).trimmingCharacters(in: .whitespaces) }
-            return raw.trimmingCharacters(in: .whitespaces)
+            if let r = raw.range(of: "<asr_text>") { return (String(raw[r.upperBound...]).trimmingCharacters(in: .whitespaces), conf) }
+            return (raw.trimmingCharacters(in: .whitespaces), conf)
         }
     }
 
