@@ -192,6 +192,19 @@ int q3asr_batch_set_sampling(q3asr_handle* h, const q3asr_sampling* sampling);
 int q3asr_transcribe_ids_lp(q3asr_handle* h, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
                             const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos,
                             int32_t* ids_out, int* lens_out, float* logprobs_out);
+/* Continuous batching: the whole request runs as ONE resident decode batch of at most max_rows rows (max_rows <= 0: 256).  The
+ * first max_rows utterances are prefilled together; whenever a poll of the decode loop (every 16 steps) finds at least
+ * max(4, max_rows / 4) rows finished (or none active), the finished rows leave the batch and the next waiting utterances, in request
+ * order, go through mel -> encoder -> prefill as a group whose KV cache is written into the freed page blocks; they join the
+ * decode rows at once.  The call returns when no utterance waits and no row is active.  Greedy only (there is no sampling
+ * argument).  ids_out [batch, max_tokens], lens_out [batch] and logprobs_out [batch, max_tokens] (may be NULL) are in request order
+ * and equal, bit for bit, what q3asr_transcribe_ids_lp returns for the same utterances: only the schedule changes.  The next
+ * group's samples are staged on the copy stream while the decode runs.  q3asr_stage_ms: mel / encoder / prefill summed over the
+ * first group and every admission, decode = the rest; q3asr_decode_stats covers the whole call (a partition of the decode rows
+ * counts as a compaction).  Q3ASR_ERR_INVALID: max_rows > 256, batch <= 0 or > 65536. */
+int q3asr_transcribe_ids_continuous(q3asr_handle* h, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
+                                    const q3asr_prompt* prompts, int max_tokens, int stop_on_eos, int max_rows, int32_t* ids_out,
+                                    int* lens_out, float* logprobs_out);
 /* resident-batch form: enable != 0 between q3asr_batch_upload and the prefill stage (every upload starts with them off), then
  * q3asr_batch_download_logprobs after the run: out [batch, max_tokens], the layout of q3asr_batch_download's ids.
  * Q3ASR_ERR_STATE when they were not enabled for the batch. */
@@ -261,6 +274,9 @@ uint64_t q3asr_launch_count(const q3asr_handle* h);
  * decode batch (the reference stops each utterance at EOS, Qwen3ASR.swift:378-379), so row-steps follow the tokens actually
  * generated instead of batch x longest utterance. */
 int q3asr_decode_stats(const q3asr_handle* h, uint64_t* out4);
+/* the last q3asr_transcribe_ids_continuous: out2 = {admissions (groups prefilled after the first), utterances admitted after the first
+ * group}; {0, 0} after any other run */
+int q3asr_decode_admissions(const q3asr_handle* h, uint64_t* out2);
 /* per-kernel-family device timing (CUDA events around tagged launches of the encoder / prefill / decode stages).
  * report: one line per tag "tag,launches,total_ms,algorithmic_flops,algorithmic_bytes"; reading it resets the log. */
 int q3asr_profile(q3asr_handle* h, int enable);
@@ -296,6 +312,10 @@ int q3asr_pool_transcribe_ids_lp(q3asr_pool* p, const float* const* pcm, const s
  * library while the caller prepares the next one.  The sample, prompt-id and sample-rate arrays are borrowed until q3asr_job_wait
  * returns (the pointer tables themselves are copied); jobs of one pool run one after the other.  q3asr_job_wait blocks, copies
  * ids [batch, max_tokens] / lens [batch] out and may be called once; q3asr_job_free joins if needed. */
+/* enable != 0: every q3asr_pool_transcribe_ids* / q3asr_pool_submit* call runs each worker's whole length-sorted share through
+ * q3asr_transcribe_ids_continuous with max_batch_per_gpu as max_rows, instead of sub-batches one after the other.  Same ids.  A call
+ * with non-greedy decoder knobs on a continuous pool returns Q3ASR_ERR_INVALID. */
+int q3asr_pool_set_continuous(q3asr_pool* p, int enable);
 typedef struct q3asr_job q3asr_job;
 int q3asr_pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, const int* sample_rates, int batch,
                       const q3asr_prompt* prompts, const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu,

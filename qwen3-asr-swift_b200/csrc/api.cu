@@ -373,6 +373,19 @@ int q3asr_transcribe_ids_lp(q3asr_handle* h, const float* const* pcm, const size
         transcribe_chunked(x, pcm, n, sample_rates, batch, prompts, sampling, true, max_tokens, stop_on_eos, ids_out, lens_out, logprobs_out);
     });
 }
+int q3asr_transcribe_ids_continuous(q3asr_handle* h, const float* const* pcm, const size_t* n, const int* sample_rates, int batch,
+                                    const q3asr_prompt* prompts, int max_tokens, int stop_on_eos, int max_rows, int32_t* ids_out, int* lens_out,
+                                    float* logprobs_out) {
+    return guarded(h, [&](Handle& x) {
+        Q3_CHECK(max_rows <= SKINNY_MAX_ROWS && batch > 0 && max_tokens >= 0, Q3ASR_ERR_INVALID,
+                 "transcribe_continuous: max_rows > 256, empty batch or max_tokens < 0");
+        if (max_tokens == 0) {  // nothing is decoded: the static path validates the clips and returns empty utterances
+            transcribe_chunked(x, pcm, n, sample_rates, batch, prompts, nullptr, false, 0, stop_on_eos, ids_out, lens_out, logprobs_out);
+            return;
+        }
+        transcribe_continuous(&x, pcm, n, sample_rates, batch, prompts, max_tokens, stop_on_eos, max_rows, ids_out, lens_out, logprobs_out);
+    });
+}
 int q3asr_batch_set_logprobs(q3asr_handle* h, int enable) {
     return guarded(h, [&](Handle& x) { batch_set_logprobs(&x, enable); });
 }
@@ -438,6 +451,13 @@ int q3asr_decode_stats(const q3asr_handle* h, uint64_t* out4) {
     out4[1] = bs ? bs->stat_row_steps : 0;
     out4[2] = bs ? bs->stat_compactions : 0;
     out4[3] = bs ? (uint64_t)bs->dec_rows : 0;
+    return Q3ASR_OK;
+}
+int q3asr_decode_admissions(const q3asr_handle* h, uint64_t* out2) {
+    if (h == nullptr || out2 == nullptr) return Q3ASR_ERR_INVALID;
+    const BatchState* bs = h->h.batch.get();
+    out2[0] = bs ? bs->stat_admissions : 0;
+    out2[1] = bs ? bs->stat_admitted : 0;
     return Q3ASR_OK;
 }
 int q3asr_profile(q3asr_handle* h, int enable) {

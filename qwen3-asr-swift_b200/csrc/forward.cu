@@ -52,14 +52,18 @@ size_t push_ints(std::vector<int>& buf, const std::vector<T>& v) {
     return off;
 }
 
-BatchState* fresh_batch(Handle* h) {
-    if (!h->batch) {
-        h->batch.reset(new BatchState());
-        h->batch->bind(&h->dev_bytes);
-        for (auto& e : h->batch->ev) Q3_CUDA(cudaEventCreate(&e));
+BatchState* fresh_state(Handle* h, std::unique_ptr<BatchState>& slot) {
+    if (!slot) {
+        slot.reset(new BatchState());
+        slot->bind(&h->dev_bytes);
+        for (auto& e : slot->ev) Q3_CUDA(cudaEventCreate(&e));
     }
-    return h->batch.get();
+    return slot.get();
 }
+BatchState* fresh_batch(Handle* h) { return fresh_state(h, h->batch); }
+
+// outputs (out_ids, out_lp, out_len, finished) are sized for this many sequences
+int seq_count(const BatchState* bs) { return std::max(bs->n_seqs, bs->B); }
 
 // Plans the encoder side for clips with the given frame counts (mel already known or to be computed).
 void plan_encoder(Handle* h, BatchState* bs, const std::vector<int>& frames, const std::vector<long long>& mel_off,
@@ -163,7 +167,7 @@ void plan_decoder(Handle* h, BatchState* bs, const q3asr_prompt* prompts, int ma
 // transcribe(maxTokens:) takes any value, Qwen3ASR.swift:131-136) as long as the prefill has not written any page yet.
 void plan_pages(Handle* h, BatchState* bs, int max_tokens) {
     bs->max_tokens = max_tokens;
-    bs->pages_per_seq = (bs->max_prompt + max_tokens + KV_PAGE - 1) / KV_PAGE;
+    bs->pages_per_seq = (std::max(bs->max_prompt, bs->page_prompt) + max_tokens + KV_PAGE - 1) / KV_PAGE;
     const size_t n = (size_t)bs->B * bs->pages_per_seq;
     bs->page_tab.reserve(n * sizeof(int));
     bs->page_tab2.reserve(n * sizeof(int));  // target of the next compaction of the decode rows
@@ -236,28 +240,28 @@ void reserve_decoder(Handle* h, BatchState* bs) {
         }
     }
     const size_t page_elems = (size_t)c.dec_layers * 2 * c.dec_kv_heads * KV_PAGE * hd;
-    bs->kv_pool.reserve((size_t)bs->B * bs->pages_per_seq * page_elems * 2);
+    if (!bs->kv_from) bs->kv_pool.reserve((size_t)bs->B * bs->pages_per_seq * page_elems * 2);  // an admission group writes the resident pool
     const size_t tiles = c.dec_vocab / 32;  // upper bound on LM-head n-tiles
     bs->amax_val.reserve((size_t)bs->B * tiles * 4);
     bs->amax_idx.reserve((size_t)bs->B * tiles * 4);
-    const size_t B = bs->B, mt = std::max(bs->max_tokens, 1);
+    const size_t B = bs->B, S = seq_count(bs), mt = std::max(bs->max_tokens, 1);
     bs->st_next_tok.reserve(B * 4);
     bs->st_next_val.reserve(B * 4);
     bs->st_cur_tok.reserve(B * 4);
     bs->st_pos.reserve(B * 4);
     bs->st_kv_len.reserve(B * 4);
-    bs->st_out_ids.reserve(B * mt * 4);
-    bs->st_out_val.reserve(B * mt * 4);
-    bs->st_out_len.reserve(B * 4);
-    bs->st_finished.reserve(B * 4);
+    bs->st_out_ids.reserve(S * mt * 4);
+    bs->st_out_val.reserve(S * mt * 4);
+    bs->st_out_len.reserve(S * 4);
+    bs->st_finished.reserve(S * 4);
     bs->st_slot_seq.reserve(B * 4);
     bs->st_scalars.reserve(64);
     if (bs->logprobs_on) {
         bs->amax_sum.reserve((size_t)bs->B * tiles * 4);
         bs->st_next_lp.reserve(B * 4);
-        bs->st_out_lp.reserve(B * mt * 4);
+        bs->st_out_lp.reserve(S * mt * 4);
     }
-    bs->h_out.reserve(B * mt * 8 + B * 8 + 64);
+    bs->h_out.reserve(S * mt * 8 + S * 8 + 64);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -445,9 +449,16 @@ void run_encoder(Handle* h, BatchState* bs, const float* d_mel) {
 
 KvCache kv_cache(Handle* h, BatchState* bs) {
     KvCache kc;
-    kc.pool = bs->kv_pool.as<bf16>();
-    kc.page_table = (bs->page_cur ? bs->page_tab2 : bs->page_tab).as<int>();
-    kc.max_pages = bs->pages_per_seq;
+    if (bs->kv_from) {  // admission group: the resident pool, through the resident page table's rows from kv_row0 on
+        const BatchState* r = bs->kv_from;
+        kc.pool = r->kv_pool.as<bf16>();
+        kc.page_table = (r->page_cur ? r->page_tab2 : r->page_tab).as<int>() + (size_t)bs->kv_row0 * r->pages_per_seq;
+        kc.max_pages = r->pages_per_seq;
+    } else {
+        kc.pool = bs->kv_pool.as<bf16>();
+        kc.page_table = (bs->page_cur ? bs->page_tab2 : bs->page_tab).as<int>();
+        kc.max_pages = bs->pages_per_seq;
+    }
     kc.layers = h->cfg.dec_layers;
     kc.kv_heads = h->cfg.dec_kv_heads;
     kc.head_dim = h->cfg.dec_head_dim;
@@ -714,14 +725,16 @@ void run_prefill(Handle* h, BatchState* bs, int stop_on_eos, bool forced) {
     // decode state: positions / cache lengths start at the prompt length
     Q3_CUDA(cudaMemcpyAsync(bs->st_pos.p, ints + bs->o_pos0, sizeof(int) * B, cudaMemcpyDeviceToDevice, st));
     Q3_CUDA(cudaMemcpyAsync(bs->st_kv_len.p, ints + bs->o_seq_len, sizeof(int) * B, cudaMemcpyDeviceToDevice, st));
-    Q3_CUDA(cudaMemsetAsync(bs->st_out_len.p, 0, sizeof(int) * B, st));
-    Q3_CUDA(cudaMemsetAsync(bs->st_finished.p, 0, sizeof(int) * B, st));
+    const size_t S = seq_count(bs);
+    Q3_CUDA(cudaMemsetAsync(bs->st_out_len.p, 0, sizeof(int) * S, st));
+    Q3_CUDA(cudaMemsetAsync(bs->st_finished.p, 0, sizeof(int) * S, st));
     Q3_CUDA(cudaMemcpyAsync(bs->st_slot_seq.p, ints + bs->o_ident, sizeof(int) * B, cudaMemcpyDeviceToDevice, st));
     bs->dec_rows = B;
-    bs->slot_map_on = false;
+    bs->slot_map_on = bs->per_seq_steps;  // per-sequence steps index the outputs through the map from the start (identity here)
     bs->stat_row_steps = bs->stat_steps = bs->stat_compactions = 0;
-    Q3_CUDA(cudaMemsetAsync(bs->st_out_ids.p, 0, sizeof(int32_t) * B * std::max(bs->max_tokens, 1), st));
-    if (bs->logprobs_on) Q3_CUDA(cudaMemsetAsync(bs->st_out_lp.p, 0, sizeof(float) * B * std::max(bs->max_tokens, 1), st));
+    bs->stat_admissions = bs->stat_admitted = 0;
+    Q3_CUDA(cudaMemsetAsync(bs->st_out_ids.p, 0, sizeof(int32_t) * S * std::max(bs->max_tokens, 1), st));
+    if (bs->logprobs_on) Q3_CUDA(cudaMemsetAsync(bs->st_out_lp.p, 0, sizeof(float) * S * std::max(bs->max_tokens, 1), st));
     const int scal[2] = {B, 0};
     memcpy(bs->h_out.p, scal, sizeof(scal));
     Q3_CUDA(cudaMemcpyAsync(bs->st_scalars.p, bs->h_out.p, sizeof(scal), cudaMemcpyHostToDevice, st));
@@ -730,7 +743,7 @@ void run_prefill(Handle* h, BatchState* bs, int stop_on_eos, bool forced) {
     // prompt_len - 1 / prompt_len and come out as prompt_len (position of the first generated token) and
     // prompt_len + 1 (keys visible to the first decode step).
     DecodeState s = decode_state(h, bs, stop_on_eos, forced);
-    decode_advance_launch(s, B, st);
+    decode_advance_launch(s, B, st, bs->per_seq_steps);
     h->launches++;
     bs->prefill_done = true;
     bs->steps_done = 1;
@@ -752,7 +765,7 @@ void decode_step_kernels(Handle* h, BatchState* bs, int stop_on_eos, bool forced
         decoder_layers(h, bs, rows, false);
         lm_head_argmax(h, bs, nullptr);
     }
-    decode_advance_launch(decode_state(h, bs, stop_on_eos, forced), rows, st);
+    decode_advance_launch(decode_state(h, bs, stop_on_eos, forced), rows, st, bs->per_seq_steps);
     h->launches++;
 }
 
@@ -906,9 +919,26 @@ int encoder_tokens_for(int frames) {
     return full * 13 + (rem > 0 ? std::max(conv_len3(rem), 1) : 0);
 }
 
-void batch_upload(Handle* h, const float* const* pcm, const size_t* n_in, int batch, const q3asr_prompt* prompts, const int* rates,
-                  bool defer_join) {
-    finish_upload(h->batch.get());  // (a previous upload whose caller never ran it to the end)
+namespace {
+
+// The clips at another rate, converted to 16 kHz on the compute stream once their copy has landed (their event).
+void resample_clips(Handle* h, BatchState* bs, const int* rates, const size_t* n_in, const size_t* raw_off) {
+    for (int b = 0; b < bs->B; b++)
+        if (rates[b] != 16000) {
+            wait_recorded(bs, b);
+            Q3_CUDA(cudaStreamWaitEvent(h->stream, h->copy_ev[(size_t)b], 0));
+            bs->copy_waited[(size_t)b] = 1;
+            resample_device(h, bs->raw_pcm.as<float>() + raw_off[b], n_in[b], rates[b], 16000, bs->pcm.as<float>() + bs->mel.clips[b].in_off,
+                            (size_t)bs->mel.clips[b].n, h->stream);
+        }
+}
+
+// Upload into a given state.  staged (continuous batching's next group): only the host side runs now — the staging threads copy
+// the samples on the copy stream while the decode goes on, and the plan is kept on the host; nothing is queued on the compute
+// stream and nothing waits for it.  upload_staged finishes the upload when the group is admitted.
+void batch_upload_into(Handle* h, BatchState* bs, const float* const* pcm, const size_t* n_in, int batch, const q3asr_prompt* prompts,
+                       const int* rates, bool defer_join, bool staged) {
+    finish_upload(bs);  // (a previous upload whose caller never ran it to the end)
     Q3_CHECK(pcm != nullptr && n_in != nullptr && batch > 0, Q3ASR_ERR_INVALID, "batch_upload: null argument / empty batch");
     Q3_CHECK(batch <= 1024, Q3ASR_ERR_INVALID, "batch_upload: at most 1024 utterances per call");
     // clips at another rate are converted to 16 kHz on the device (Qwen3ASRModel.transcribe resamples first,
@@ -928,8 +958,13 @@ void batch_upload(Handle* h, const float* const* pcm, const size_t* n_in, int ba
                  "batch_upload: every clip needs at least 160 samples at 16 kHz (one mel frame)");
     }
     const size_t* n = n16.data();
-    BatchState* bs = fresh_batch(h);
     bs->B = batch;
+    bs->n_seqs = batch;
+    bs->page_prompt = 0;
+    bs->per_seq_steps = false;
+    bs->kv_from = nullptr;
+    bs->kv_row0 = 0;
+    bs->stat_admissions = bs->stat_admitted = 0;
     bs->mel = mel_plan(n, batch);
     bs->mel_done = bs->enc_done = bs->prefill_done = false;
     bs->steps_done = 0;
@@ -1003,7 +1038,7 @@ void batch_upload(Handle* h, const float* const* pcm, const size_t* n_in, int ba
                 J->werr[(size_t)w] = e;
             });
     }
-    Q3_CUDA(cudaMemcpyAsync(bs->mel_clips.p, bs->mel.clips.data(), sizeof(MelClip) * batch, cudaMemcpyHostToDevice, h->stream));
+    if (!staged) Q3_CUDA(cudaMemcpyAsync(bs->mel_clips.p, bs->mel.clips.data(), sizeof(MelClip) * batch, cudaMemcpyHostToDevice, h->stream));
     // plan
     std::vector<int> frames(batch);
     std::vector<long long> mel_off(batch);
@@ -1018,20 +1053,34 @@ void batch_upload(Handle* h, const float* const* pcm, const size_t* n_in, int ba
     // re-plans them when a larger value is asked for
     const int reserve_tokens = std::max(1, env_int("Q3ASR_RESERVE_TOKENS", 448));
     plan_decoder(h, bs, prompts, reserve_tokens, &ints);
+    if (staged) {
+        bs->plan_ints = std::move(ints);
+        bs->up_rates.clear();
+        if (raw_floats) bs->up_rates.assign(rates, rates + batch);
+        bs->up_n.assign(n_in, n_in + batch);
+        bs->up_raw_off = raw_off;
+        return;
+    }
     if (!defer_join) finish_upload(bs);
-    if (raw_floats)  // the conversions follow their clip's copy (its event)
-        for (int b = 0; b < batch; b++)
-            if (rates[b] != 16000) {
-                wait_recorded(bs, b);
-                Q3_CUDA(cudaStreamWaitEvent(h->stream, h->copy_ev[(size_t)b], 0));
-                bs->copy_waited[(size_t)b] = 1;
-                resample_device(h, bs->raw_pcm.as<float>() + raw_off[(size_t)b], n_in[b], rates[b], 16000,
-                                bs->pcm.as<float>() + bs->mel.clips[b].in_off, n[b], h->stream);
-            }
+    if (raw_floats) resample_clips(h, bs, rates, n_in, raw_off.data());  // the conversions follow their clip's copy (its event)
     upload_ints(h, bs, ints);  // (synchronises the COMPUTE stream; the sample copies may still be in flight on the copy stream: the
                                // caller's buffers are free — they were copied to the staging area — and run_mel waits per clip)
     plan_pages(h, bs, reserve_tokens);
     bs->prompt_ids.clear();
+}
+
+// The compute-stream half of a staged upload: clip table, sample-rate conversions, plan.
+void upload_staged(Handle* h, BatchState* bs) {
+    Q3_CUDA(cudaMemcpyAsync(bs->mel_clips.p, bs->mel.clips.data(), sizeof(MelClip) * bs->B, cudaMemcpyHostToDevice, h->stream));
+    if (!bs->up_rates.empty()) resample_clips(h, bs, bs->up_rates.data(), bs->up_n.data(), bs->up_raw_off.data());
+    upload_ints(h, bs, bs->plan_ints);
+}
+
+}  // namespace
+
+void batch_upload(Handle* h, const float* const* pcm, const size_t* n_in, int batch, const q3asr_prompt* prompts, const int* rates,
+                  bool defer_join) {
+    batch_upload_into(h, fresh_batch(h), pcm, n_in, batch, prompts, rates, defer_join, false);
 }
 
 // Qwen3ForcedAligner.align (ForcedAligner.swift:226-331), batched: mel -> encoder -> one causal prefill over the aligner template ->
@@ -1213,7 +1262,7 @@ void batch_download(Handle* h, int32_t* ids, int max_tokens, int* lens) {
     BatchState* bs = h->batch.get();
     Q3_CHECK(bs != nullptr && bs->B > 0, Q3ASR_ERR_STATE, "batch_download: no batch");
     Q3_CHECK(ids != nullptr && lens != nullptr && max_tokens >= 0, Q3ASR_ERR_INVALID, "batch_download: bad argument");
-    const int B = bs->B, mt = bs->max_tokens;
+    const int B = seq_count(bs), mt = bs->max_tokens;
     cudaStream_t st = h->stream;
     if (!bs->prefill_done) {
         Q3_CUDA(cudaStreamSynchronize(st));
@@ -1241,7 +1290,7 @@ void batch_download_logprobs(Handle* h, float* out, int max_tokens) {
     Q3_CHECK(bs != nullptr && bs->B > 0, Q3ASR_ERR_STATE, "batch_download_logprobs: no batch");
     Q3_CHECK(out != nullptr && max_tokens >= 0, Q3ASR_ERR_INVALID, "batch_download_logprobs: bad argument");
     Q3_CHECK(bs->logprobs_on, Q3ASR_ERR_STATE, "batch_download_logprobs: log-probabilities were not requested for this batch");
-    const int B = bs->B, mt = bs->max_tokens;
+    const int B = seq_count(bs), mt = bs->max_tokens;
     cudaStream_t st = h->stream;
     std::fill(out, out + (size_t)B * max_tokens, 0.f);
     if (!bs->prefill_done) {
@@ -1350,6 +1399,226 @@ void prefill_logits(Handle* h, const float* pcm, size_t n, const q3asr_prompt* p
     gemm(bs->dlast.as<bf16>(), c.dec_hidden, 1, c.dec_hidden, h->model->embed, c.dec_vocab, e, st);
     Q3_CUDA(cudaStreamSynchronize(st));
     Q3_CUDA(cudaMemcpy(logits, bs->logits.p, (size_t)c.dec_vocab * 4, cudaMemcpyDeviceToHost));
+}
+
+// ---------------------------------------------------------------------------------------------
+// Continuous batching: one request decoded by one resident batch of at most max_rows rows.  The first max_rows utterances are
+// prefilled as usual; whenever a poll finds enough rows finished, the finished rows are partitioned out of the decode rows and the
+// next waiting utterances (request order) go through mel -> encoder -> prefill as a group whose KV lands directly in the freed page
+// blocks, then join the decode rows.  Every utterance runs the same kernels on the same rows as in a static batch, so its ids and
+// log-probabilities do not depend on the schedule.
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+struct ContinuousRun {
+    Handle* h;
+    BatchState* bs;  // the resident state
+    const float* const* pcm;
+    const size_t* n;
+    const int* rates;
+    const q3asr_prompt* prompts;
+    int batch, max_rows, stop_on_eos;
+    int next_stage = 0;              // first utterance not yet staged
+    int staged = -1, staged_k = 0, staged_seq0 = 0, next_adm = 0;  // the staged group (h->adm[staged])
+    std::vector<cudaEvent_t> ev;     // four per admission: start, encoder, prefill, end
+    float adm_ms[3] = {0.f, 0.f, 0.f};
+
+    ~ContinuousRun() {
+        for (std::unique_ptr<BatchState>* s : {&h->batch, &h->adm[0], &h->adm[1]}) {  // the staging threads borrow the caller's buffers
+            try {
+                finish_upload(s->get());
+            } catch (...) {
+            }
+        }
+        for (cudaEvent_t e : ev) cudaEventDestroy(e);
+    }
+
+    // the next group's samples go to the copy stream now; its size is the rows that will be free when it is admitted, at least
+    // the admission threshold
+    void stage(int threshold) {
+        if (staged >= 0 || next_stage >= batch) return;
+        const int k = std::min(batch - next_stage, std::max(threshold, max_rows - bs->dec_rows));
+        BatchState* a = fresh_state(h, h->adm[next_adm]);
+        batch_upload_into(h, a, pcm + next_stage, n + next_stage, k, prompts ? prompts + next_stage : nullptr, rates ? rates + next_stage : nullptr,
+                          true, true);
+        staged = next_adm;
+        staged_k = k;
+        staged_seq0 = next_stage;
+        next_stage += k;
+        next_adm ^= 1;
+    }
+
+    // Rows [n_live, B) of the resident page table become the finished rows' blocks (and those of rows already free).
+    void partition(int n_live) {
+        cudaStream_t st = h->stream;
+        int* cur = (bs->page_cur ? bs->page_tab2 : bs->page_tab).as<int>();
+        int* nxt = (bs->page_cur ? bs->page_tab : bs->page_tab2).as<int>();
+        decode_compact_launch(bs->dec_rows, bs->st_finished.as<int>(), bs->st_slot_seq.as<int>(), bs->st_cur_tok.as<int32_t>(), bs->st_pos.as<int>(),
+                              bs->st_kv_len.as<int>(), cur, nxt, bs->pages_per_seq, st, bs->B);
+        h->launches++;
+        bs->page_cur ^= 1;
+        bs->dec_rows = n_live;
+        bs->stat_compactions++;
+    }
+
+    // The staged group: mel -> encoder -> prefill with its KV written into the resident rows [dec_rows, dec_rows + k), then step 0
+    // straight into the resident decode state.
+    void admit() {
+        cudaStream_t st = h->stream;
+        BatchState* a = h->adm[staged].get();
+        const int k = staged_k, row0 = bs->dec_rows;
+        Q3_CHECK(row0 + k <= bs->B, Q3ASR_ERR_STATE, "continuous: admission beyond the resident rows");
+        a->kv_from = bs;
+        a->kv_row0 = row0;
+        a->pages_per_seq = bs->pages_per_seq;
+        a->max_tokens = bs->max_tokens;
+        a->logprobs_on = bs->logprobs_on;
+        a->sampler_on = false;
+        while (ev.size() < stat_events() + 4) {
+            cudaEvent_t e = nullptr;
+            Q3_CUDA(cudaEventCreate(&e));
+            ev.push_back(e);
+        }
+        cudaEvent_t* e = ev.data() + stat_events();
+        Q3_CUDA(cudaEventRecord(e[0], st));
+        upload_staged(h, a);
+        if (!(copies_pending(h, a) && a->n_tok > 0)) run_mel(h, a);  // else interleaved with the convolution stack, as in batch_run
+        Q3_CUDA(cudaEventRecord(e[1], st));
+        reserve_encoder(h, a);
+        run_encoder(h, a, a->mel_out.as<float>());
+        finish_upload(a);
+        Q3_CUDA(cudaEventRecord(e[2], st));
+        reserve_decoder(h, a);
+        const int* ints = a->ints.as<int>();
+        embed_splice_launch(ints + a->o_ids, ints + a->o_audio_src, h->model->embed, a->audio.as<bf16>(), a->dx.as<bf16>(), a->R, h->cfg.dec_hidden, st);
+        h->launches++;
+        decoder_layers(h, a, a->R, true);
+        lm_head_argmax(h, a, ints + a->o_last_row);
+        {
+            PdlScope pdl(env_int("Q3ASR_NO_PDL", 0) == 0 && !h->prof_on);  // a programmatic dependent of the LM head's reduction
+            decode_admit_launch(decode_state(h, bs, stop_on_eos, false), a->st_next_tok.as<int32_t>(), a->st_next_val.as<float>(),
+                                bs->logprobs_on ? a->st_next_lp.as<float>() : nullptr, ints + a->o_seq_len, row0, k, staged_seq0, st);
+            h->launches++;
+        }
+        Q3_CUDA(cudaEventRecord(e[3], st));
+        bs->dec_rows = row0 + k;
+        bs->stat_admissions++;
+        bs->stat_admitted += (unsigned long long)k;
+        staged = -1;
+    }
+    size_t stat_events() const { return (size_t)bs->stat_admissions * 4; }
+
+    void decode() {
+        cudaStream_t st = h->stream;
+        const bool use_graph = env_int("Q3ASR_NO_GRAPH", 0) == 0;
+        const int threshold = std::min(max_rows, std::max(4, max_rows / 4));  // today's compaction threshold at max_rows rows
+        int* h_active = reinterpret_cast<int*>(bs->h_out.p);
+        bool graph_ok = false;
+        unsigned long long per_step = 0;
+        auto rows_changed = [&]() {
+            graph_ok = false;
+            bs->mega_ready = false;
+            if (bs->dec_rows > 0 && mega_wanted(h, bs)) megastep_prepare(h, bs);
+        };
+        rows_changed();
+        stage(threshold);
+        // every utterance needs at most max_tokens steps; a poll window without an active row always ends in an admission or the end
+        const long long max_steps = (long long)batch * (bs->max_tokens + 32) + 64;
+        long long steps = 0;
+        for (;;) {
+            for (int i = 0; i < 16 && bs->dec_rows > 0; i++, steps++) {
+                if (!use_graph || h->prof_on || !h->decode_warm) {
+                    decode_step_kernels(h, bs, stop_on_eos, false);
+                    h->decode_warm = true;
+                } else {
+                    if (!graph_ok) {
+                        per_step = capture_step_graph(h, bs, stop_on_eos, false);
+                        graph_ok = true;
+                    }
+                    Q3_CUDA(cudaGraphLaunch(bs->step_graph, st));
+                    h->launches += per_step;
+                }
+                bs->stat_steps++;
+                bs->stat_row_steps += (unsigned long long)bs->dec_rows;
+            }
+            Q3_CHECK(steps <= max_steps, Q3ASR_ERR_STATE, "continuous: the decode loop did not finish");
+            Q3_CUDA(cudaMemcpyAsync(h_active, bs->st_scalars.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+            Q3_CUDA(cudaStreamSynchronize(st));
+            const int n_live = *h_active;
+            if (n_live <= 0 && staged < 0 && next_stage >= batch) break;
+            if (staged >= 0 && max_rows - n_live >= staged_k) {
+                if (bs->dec_rows > n_live) partition(n_live);
+                admit();
+                rows_changed();
+                stage(threshold);
+            } else if (staged < 0 && n_live < bs->dec_rows && bs->dec_rows - n_live >= std::max(4, bs->dec_rows / 4)) {
+                partition(n_live);  // nothing waits any more: shrink the batch as a static run does
+                rows_changed();
+            }
+        }
+        bs->steps_done = (int)std::min<long long>(steps, 1 << 30);
+    }
+};
+
+}  // namespace
+
+void transcribe_continuous(Handle* h, const float* const* pcm, const size_t* n, const int* rates, int batch, const q3asr_prompt* prompts,
+                           int max_tokens, int stop_on_eos, int max_rows, int32_t* ids_out, int* lens_out, float* lp_out) {
+    if (max_rows <= 0) max_rows = SKINNY_MAX_ROWS;
+    Q3_CHECK(max_rows <= SKINNY_MAX_ROWS, Q3ASR_ERR_INVALID, "transcribe_continuous: max_rows > 256");
+    Q3_CHECK(pcm != nullptr && n != nullptr && ids_out != nullptr && lens_out != nullptr && batch > 0 && batch <= (1 << 16), Q3ASR_ERR_INVALID,
+             "transcribe_continuous: null argument, empty batch or more than 65536 utterances");
+    Q3_CHECK(max_tokens >= 1 && max_tokens <= (1 << 20), Q3ASR_ERR_INVALID, "transcribe_continuous: max_tokens out of range");
+    Q3_CHECK(h->loaded && h->model, Q3ASR_ERR_STATE, "weights are not loaded (q3asr_init_random / q3asr_load_safetensors)");
+    // every utterance is checked up front (a later group must not fail mid-decode), and the KV pages are planned for the longest
+    // prompt of the whole request: an utterance with a long context admitted late still fits its block
+    int max_prompt = 0;
+    for (int b = 0; b < batch; b++) {
+        Q3_CHECK(pcm[b] != nullptr && n[b] < (size_t)1 << 30 && (rates == nullptr || rates[b] > 0), Q3ASR_ERR_INVALID,
+                 "transcribe_continuous: null clip, clip too long or bad sample rate");
+        const size_t n16 = rates != nullptr && rates[b] != 16000 ? resample_len(n[b], rates[b], 16000) : n[b];
+        Q3_CHECK(n16 >= (size_t)MEL_HOP && n16 < (size_t)1 << 30, Q3ASR_ERR_INVALID,
+                 "transcribe_continuous: every clip needs at least 160 samples at 16 kHz (one mel frame)");
+        std::vector<int32_t> ids;
+        int at = 0;
+        build_prompt(h->cfg, prompts ? &prompts[b] : nullptr, encoder_tokens_for(mel_frames_for(n16)), &ids, &at);
+        max_prompt = std::max(max_prompt, (int)ids.size());
+    }
+    const int rows = std::min(batch, max_rows);
+    BatchState* bs = fresh_batch(h);
+    ContinuousRun run{h, bs, pcm, n, rates, prompts, batch, max_rows, stop_on_eos};
+    run.next_stage = rows;
+    cudaStream_t st = h->stream;
+    batch_upload_into(h, bs, pcm, n, rows, prompts, rates, true, false);
+    bs->n_seqs = batch;
+    bs->page_prompt = max_prompt;
+    bs->per_seq_steps = true;
+    bs->logprobs_on = lp_out != nullptr;
+    plan_pages(h, bs, max_tokens);
+    Q3_CUDA(cudaEventRecord(bs->ev[0], st));
+    if (!(copies_pending(h, bs) && bs->n_tok > 0)) run_mel(h, bs);
+    Q3_CUDA(cudaEventRecord(bs->ev[1], st));
+    reserve_encoder(h, bs);
+    run_encoder(h, bs, bs->mel_out.as<float>());
+    finish_upload(bs);
+    Q3_CUDA(cudaEventRecord(bs->ev[2], st));
+    reserve_decoder(h, bs);
+    run_prefill(h, bs, stop_on_eos, false);
+    Q3_CUDA(cudaEventRecord(bs->ev[3], st));
+    run.decode();
+    Q3_CUDA(cudaEventRecord(bs->ev[4], st));
+    batch_download(h, ids_out, max_tokens, lens_out);  // (synchronises; stage times of the first group)
+    if (lp_out) batch_download_logprobs(h, lp_out, max_tokens);
+    float adm[3] = {0.f, 0.f, 0.f};
+    for (size_t i = 0; i + 3 < run.ev.size() && i < run.stat_events(); i += 4)
+        for (int s = 0; s < 3; s++) {
+            float ms = 0.f;
+            if (cudaEventElapsedTime(&ms, run.ev[i + s], run.ev[i + s + 1]) == cudaSuccess) adm[s] += ms;
+        }
+    for (int s = 0; s < 3; s++) {
+        h->stage_ms[s] += adm[s];
+        h->stage_ms[3] -= adm[s];  // the admissions ran inside the decode window
+    }
 }
 
 }  // namespace q3

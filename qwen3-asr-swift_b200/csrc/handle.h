@@ -111,6 +111,8 @@ struct Handle {
     bool loaded = false;
     std::unique_ptr<Model> model;
     std::unique_ptr<BatchState> batch;
+    // continuous batching: the admission groups, two so the next group's samples are staged while the current one is admitted
+    std::unique_ptr<BatchState> adm[2];
 
     // optional per-kernel-family profiling (q3asr_profile): CUDA events around tagged launches
     struct ProfRec {
@@ -211,6 +213,9 @@ void batch_run(Handle* h, int stages, int max_tokens, int stop_on_eos);
 void batch_download(Handle* h, int32_t* ids, int max_tokens, int* lens);
 void batch_set_logprobs(Handle* h, int enable);
 void batch_download_logprobs(Handle* h, float* out, int max_tokens);
+// continuous batching (q3asr_transcribe_ids_continuous): the whole request through one resident batch of at most max_rows rows
+void transcribe_continuous(Handle* h, const float* const* pcm, const size_t* n, const int* rates, int batch, const q3asr_prompt* prompts,
+                           int max_tokens, int stop_on_eos, int max_rows, int32_t* ids_out, int* lens_out, float* lp_out);
 void encode_one(Handle* h, const float* mel, int frames, float* out, int* tokens);
 void decode_forced(Handle* h, const float* pcm, size_t n, const q3asr_prompt* prompt, const int32_t* forced, int n_forced,
                    int32_t* argmax_out, float* top_out, const float* audio_embeds = nullptr, int n_audio_tokens = 0);

@@ -105,6 +105,18 @@ struct BatchState {
     int page_cur = 0;             // which of page_tab / page_tab2 the decode rows index through
     bool slot_map_on = false;     // st_slot_seq holds the row -> sequence map (identity until the first compaction)
     unsigned long long stat_row_steps = 0, stat_steps = 0, stat_compactions = 0;  // q3asr_decode_stats
+    // continuous batching (transcribe_continuous): the resident state decodes a whole request of n_seqs utterances through its B rows
+    int n_seqs = 0;               // sequences the outputs (out_ids / out_lp / out_len / finished) are sized and indexed for; B otherwise
+    int page_prompt = 0;          // prompt length the KV pages are planned for when it exceeds max_prompt (the request's longest prompt)
+    bool per_seq_steps = false;   // decode_advance counts steps per sequence (admitted sequences start mid-loop)
+    unsigned long long stat_admissions = 0, stat_admitted = 0;  // q3asr_decode_admissions
+    // an admission group's state borrows the resident state's KV pool: its prefill writes through the resident page table from row
+    // kv_row0 on (the freed rows' blocks)
+    BatchState* kv_from = nullptr;
+    int kv_row0 = 0;
+    std::vector<int> plan_ints;   // host plan of a staged group, uploaded when it is admitted
+    std::vector<int> up_rates;    // sample rates of a staged group (empty: all 16 kHz), converted when it is admitted
+    std::vector<size_t> up_n, up_raw_off;
 
     // device buffers
     DevBuf pcm, mel_out, mel_clips, mel_gmax, mel_tmin;

@@ -953,11 +953,38 @@ __global__ void __launch_bounds__(1024) reduce_resid_rmsnorm_kernel(const float*
 }
 
 // ------------------------------------------------------------------------------------------
+// PER_SEQ (continuous batching): every sequence counts its own steps (out_len), because an admitted utterance starts at step 0 in
+// the middle of the loop; it finishes on EOS or at max_tokens, and a finished row stays where it is (pos / kv_len frozen) until a
+// partition takes it out, so it never appends past the last page of its block.
+template <bool PER_SEQ>
 __global__ void decode_advance_kernel(DecodeState s, int n_seqs) {
     ptx::grid_dep_launch();
     ptx::grid_dep_wait();
     const int i = blockIdx.x * blockDim.x + threadIdx.x;  // decode row
     const int step = *s.step;
+    if (PER_SEQ) {
+        if (i < n_seqs) {
+            const int q = s.slot_seq[i];
+            if (!s.finished[q]) {
+                const int32_t tok = s.next_tok[i];
+                const int t = s.out_len[q];
+                s.out_ids[(size_t)q * s.max_tokens + t] = tok;
+                if (s.out_val && s.next_val) s.out_val[(size_t)q * s.max_tokens + t] = s.next_val[i];
+                if (s.out_lp && s.next_lp) s.out_lp[(size_t)q * s.max_tokens + t] = s.next_lp[i];
+                s.out_len[q] = t + 1;
+                if ((s.stop_on_eos && tok == s.eos) || t + 1 >= s.max_tokens) {
+                    s.finished[q] = 1;
+                    atomicSub(s.n_active, 1);
+                }
+                s.cur_tok[i] = tok;
+                s.pos[i] += 1;
+                s.kv_len[i] += 1;
+            }
+        }
+        __syncthreads();
+        if (i == 0) *s.step = step + 1;
+        return;
+    }
     if (i < n_seqs) {
         const int32_t tok = s.next_tok[i];
         const int q = s.slot_seq ? s.slot_seq[i] : i;  // the sequence this row decodes
@@ -980,10 +1007,12 @@ __global__ void decode_advance_kernel(DecodeState s, int n_seqs) {
 }
 
 // ------------------------------------------------------------------------------------------
-// Compaction of the decode rows: see decode_compact_launch (ops.cuh).
+// Compaction of the decode rows: see decode_compact_launch (ops.cuh).  PARTITION: the finished rows' page-table rows follow the live
+// ones (stable), and the rows [rows, cap) are carried over, so every page block stays named in the new table.
+template <bool PARTITION>
 __global__ void __launch_bounds__(1024) decode_compact_kernel(int rows, const int* __restrict__ finished, int* slot_seq, int32_t* cur_tok, int* pos,
                                                               int* kv_len, const int* __restrict__ page_in, int* __restrict__ page_out,
-                                                              int max_pages) {
+                                                              int max_pages, int cap) {
     __shared__ int s_warp[32];
     const int i = threadIdx.x, lane = i & 31, warp = i >> 5;
     int q = 0, tok = 0, p = 0, kl = 0, alive = 0;
@@ -1009,6 +1038,46 @@ __global__ void __launch_bounds__(1024) decode_compact_kernel(int rows, const in
         kv_len[j] = kl;
         for (int k = 0; k < max_pages; k++) page_out[(size_t)j * max_pages + k] = page_in[(size_t)i * max_pages + k];
     }
+    if (PARTITION) {
+        int live = base;
+        for (int w = warp; w < 32; w++) live += s_warp[w];
+        if (i < rows && !alive) {
+            const int j = live + (i - base - in_warp);  // live rows first, then the finished ones in row order
+            for (int k = 0; k < max_pages; k++) page_out[(size_t)j * max_pages + k] = page_in[(size_t)i * max_pages + k];
+        } else if (i >= rows && i < cap) {
+            for (int k = 0; k < max_pages; k++) page_out[(size_t)i * max_pages + k] = page_in[(size_t)i * max_pages + k];
+        }
+    }
+}
+
+// Step 0 of an admitted group (continuous batching), written straight into the resident decode state at rows [row0, row0 + k):
+// group member j is request sequence seq0 + j, its first token comes from the group's prefill LM head (tok / val / lp [k]).
+__global__ void decode_admit_kernel(DecodeState s, const int32_t* __restrict__ tok, const float* __restrict__ val, const float* __restrict__ lp,
+                                    const int* __restrict__ prompt_len, int row0, int k, int seq0) {
+    ptx::grid_dep_launch();
+    ptx::grid_dep_wait();
+    __shared__ int s_alive;
+    const int j = threadIdx.x;
+    if (j == 0) s_alive = 0;
+    __syncthreads();
+    if (j < k) {
+        const int q = seq0 + j, r = row0 + j;
+        const int32_t t = tok[j];
+        const size_t o = (size_t)q * s.max_tokens;
+        const_cast<int*>(s.slot_seq)[r] = q;  // (the step kernels only read the map; the admission extends it)
+        s.cur_tok[r] = t;
+        s.pos[r] = prompt_len[j];
+        s.kv_len[r] = prompt_len[j] + 1;
+        s.out_ids[o] = t;
+        if (s.out_val && val) s.out_val[o] = val[j];
+        if (s.out_lp && lp) s.out_lp[o] = lp[j];
+        s.out_len[q] = 1;
+        const int fin = (s.stop_on_eos && t == s.eos) || s.max_tokens <= 1;
+        s.finished[q] = fin;
+        if (!fin) atomicAdd(&s_alive, 1);
+    }
+    __syncthreads();
+    if (j == 0 && s_alive) atomicAdd(s.n_active, s_alive);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1310,16 +1379,28 @@ void reduce_resid_rmsnorm_launch(const float* part, int splits, long long split_
     launch_kernel(reduce_resid_rmsnorm_kernel, rows, ncg * sg, 0, st, part, splits, split_stride, x, w, y, d, eps);
 }
 
-void decode_advance_launch(const DecodeState& s, int n_seqs, cudaStream_t st) {
+void decode_advance_launch(const DecodeState& s, int n_seqs, cudaStream_t st, bool per_seq) {
     Q3_CHECK(n_seqs <= 1024, 1, "decode_advance: at most 1024 sequences per handle");
-    launch_kernel(decode_advance_kernel, 1, 1024, 0, st, s, n_seqs);
+    Q3_CHECK(!per_seq || s.slot_seq != nullptr, 1, "decode_advance: per-sequence steps need the row -> sequence map");
+    if (per_seq) launch_kernel(decode_advance_kernel<true>, 1, 1024, 0, st, s, n_seqs);
+    else launch_kernel(decode_advance_kernel<false>, 1, 1024, 0, st, s, n_seqs);
 }
 
 void decode_compact_launch(int rows, const int* finished, int* slot_seq, int32_t* cur_tok, int* pos, int* kv_len, const int* page_in,
-                           int* page_out, int max_pages, cudaStream_t st) {
-    Q3_CHECK(rows >= 1 && rows <= 1024, 1, "decode_compact: 1..1024 rows");
-    decode_compact_kernel<<<1, 1024, 0, st>>>(rows, finished, slot_seq, cur_tok, pos, kv_len, page_in, page_out, max_pages);
+                           int* page_out, int max_pages, cudaStream_t st, int partition_cap) {
+    Q3_CHECK(rows >= 1 && rows <= 1024 && partition_cap <= 1024, 1, "decode_compact: 1..1024 rows");
+    if (partition_cap > 0)
+        decode_compact_kernel<true><<<1, 1024, 0, st>>>(rows, finished, slot_seq, cur_tok, pos, kv_len, page_in, page_out, max_pages,
+                                                        partition_cap);
+    else
+        decode_compact_kernel<false><<<1, 1024, 0, st>>>(rows, finished, slot_seq, cur_tok, pos, kv_len, page_in, page_out, max_pages, 0);
     Q3_CUDA(cudaGetLastError());
+}
+
+void decode_admit_launch(const DecodeState& s, const int32_t* tok, const float* val, const float* lp, const int* prompt_len, int row0, int k,
+                         int seq0, cudaStream_t st) {
+    Q3_CHECK(k >= 1 && k <= 1024 && s.slot_seq != nullptr, 1, "decode_admit: 1..1024 rows and a row -> sequence map");
+    launch_kernel(decode_admit_kernel, 1, 1024, 0, st, s, tok, val, lp, prompt_len, row0, k, seq0);
 }
 
 int sample_parts(int vocab) { return vocab >= 32768 ? 4 : 1; }

@@ -99,13 +99,22 @@ struct DecodeState {
     int eos;
     int stop_on_eos;
 };
-void decode_advance_launch(const DecodeState& s, int n_seqs, cudaStream_t st);
+// per_seq (continuous batching): out_ids / out_lp are indexed by each sequence's own out_len instead of the batch step; a sequence also
+// finishes at max_tokens (stop_on_eos or not), and a finished row no longer advances pos / kv_len.  Needs slot_seq.
+void decode_advance_launch(const DecodeState& s, int n_seqs, cudaStream_t st, bool per_seq = false);
 // Drops the finished sequences from the decode rows (Qwen3ASR.swift:378-379 stops an utterance at EOS; a batched loop has to take it
 // out of the batch, or its KV pages and a column of every product keep being streamed): the rows whose sequence is still active
 // move to the front, in order, together with their token / position / cache length / page-table row.  One CTA; rows <= 1024.
 // page_in / page_out: [rows][max_pages] (distinct buffers).  slot_seq is updated in place (identity on entry if it was never set).
+// partition_cap > 0 (continuous batching): a stable partition of the page table instead — the finished rows' page-table rows follow
+// the live ones and rows [rows, partition_cap) are copied as they are, so rows [live, partition_cap) of page_out name free blocks.
 void decode_compact_launch(int rows, const int* finished, int* slot_seq, int32_t* cur_tok, int* pos, int* kv_len, const int* page_in,
-                           int* page_out, int max_pages, cudaStream_t st);
+                           int* page_out, int max_pages, cudaStream_t st, int partition_cap = 0);
+// Continuous batching: step 0 of a freshly prefilled group of k utterances (request sequences seq0 ..), appended to the resident decode
+// state at rows [row0, row0 + k): slot_seq, cur_tok = tok[j], pos = prompt_len[j], kv_len = prompt_len[j] + 1, out_ids / out_val /
+// out_lp [q][0], out_len[q] = 1, finished[q] on EOS (stop_on_eos) or max_tokens <= 1; n_active grows by the rows still alive.
+void decode_admit_launch(const DecodeState& s, const int32_t* tok, const float* val, const float* lp, const int* prompt_len, int row0, int k,
+                         int seq0, cudaStream_t st);
 
 // Decoder knobs of Qwen3DecodingOptions (Qwen3ASR.swift:13-51) applied on the device: the reference pulls the [vocab] logits to
 // the CPU every token (pickNextToken, Qwen3ASR.swift:449-520); here one CTA per sequence applies the same three edits while it

@@ -20,6 +20,7 @@ struct q3asr_pool {
     std::vector<q3asr_handle*> handles;
     std::string last_error;
     std::mutex run_mu;  // one batch at a time on the pool's handles (submitted jobs queue on it in submission order of their threads)
+    std::atomic<int> continuous{0};  // q3asr_pool_set_continuous: each worker's share runs as one continuous batch
 };
 
 // an asynchronous q3asr_pool_transcribe_ids_opts call: the worker thread owns the result buffers until q3asr_job_wait copies them out
@@ -43,6 +44,11 @@ struct q3asr_job {
 namespace {
 thread_local std::string g_create_error;  // q3asr_pool_last_error(NULL): why the last q3asr_pool_create on this thread failed
 
+// the continuous schedule is greedy only (the sampler indexes generated ids by row and keys its noise by slot)
+bool greedy_sampling(const q3asr_sampling* s) {
+    return s == nullptr || (s->repetition_penalty == 1.0f && s->no_repeat_ngram_size == 0 && s->temperature == 0.0f && s->force_device_sampler == 0);
+}
+
 // One batch over the pool's handles (arguments checked by the caller, p->run_mu held).  May throw from its own host allocations or
 // thread creation; workers already started are joined first.
 int pool_run(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const int* sample_rates, int batch, const q3asr_prompt* prompts,
@@ -59,6 +65,7 @@ int pool_run(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const i
     q3asr_schedule(n_samples, batch, G, gpu.data());
     std::vector<int> rc(G, Q3ASR_OK);
     std::vector<std::string> host_err(G);  // failures of the worker's own host code (the handle keeps the message of a failed call)
+    const bool continuous = p->continuous.load() != 0;
     auto work = [&](int g) {
         try {  // nothing may escape a std::thread
             std::vector<int> mine;
@@ -66,8 +73,10 @@ int pool_run(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const i
                 if (gpu[i] == g) mine.push_back(i);
             // similar lengths together: prefill rows and decode steps stay homogeneous
             std::stable_sort(mine.begin(), mine.end(), [&](int a, int b) { return n_samples[a] > n_samples[b]; });
-            for (size_t s = 0; s < mine.size(); s += max_batch_per_gpu) {
-                const int nb = (int)std::min<size_t>(max_batch_per_gpu, mine.size() - s);
+            // continuous: the whole share is one request, max_batch_per_gpu rows resident at a time
+            const size_t step = continuous ? std::max<size_t>(mine.size(), 1) : (size_t)max_batch_per_gpu;
+            for (size_t s = 0; s < mine.size(); s += step) {
+                const int nb = (int)std::min<size_t>(step, mine.size() - s);
                 std::vector<const float*> pp(nb);
                 std::vector<size_t> nn(nb);
                 std::vector<int> rr(nb, 16000);
@@ -81,9 +90,14 @@ int pool_run(q3asr_pool* p, const float* const* pcm, const size_t* n_in, const i
                 std::vector<int32_t> ids((size_t)nb * max_tokens);
                 std::vector<int> lens(nb);
                 std::vector<float> lp(lp_out ? (size_t)nb * max_tokens : 0);
-                rc[g] = q3asr_transcribe_ids_lp(p->handles[g], pp.data(), nn.data(), sample_rates ? rr.data() : nullptr, nb,
-                                                prompts ? pr.data() : nullptr, sampling, max_tokens, stop_on_eos, ids.data(), lens.data(),
-                                                lp_out ? lp.data() : nullptr);
+                if (continuous)
+                    rc[g] = q3asr_transcribe_ids_continuous(p->handles[g], pp.data(), nn.data(), sample_rates ? rr.data() : nullptr, nb,
+                                                            prompts ? pr.data() : nullptr, max_tokens, stop_on_eos, max_batch_per_gpu,
+                                                            ids.data(), lens.data(), lp_out ? lp.data() : nullptr);
+                else
+                    rc[g] = q3asr_transcribe_ids_lp(p->handles[g], pp.data(), nn.data(), sample_rates ? rr.data() : nullptr, nb,
+                                                    prompts ? pr.data() : nullptr, sampling, max_tokens, stop_on_eos, ids.data(), lens.data(),
+                                                    lp_out ? lp.data() : nullptr);
                 if (rc[g] != Q3ASR_OK) break;
                 for (int j = 0; j < nb; j++) {  // host-side result gather, original order
                     const int i = mine[s + j];
@@ -133,6 +147,10 @@ int pool_transcribe_locked(q3asr_pool* p, const float* const* pcm, const size_t*
                 p->last_error = "pool_transcribe: sample rate <= 0";
                 return Q3ASR_ERR_INVALID;
             }
+    if (p->continuous.load() && !greedy_sampling(sampling)) {
+        p->last_error = "pool_transcribe: a continuous pool decodes greedily only (no decoder knobs)";
+        return Q3ASR_ERR_INVALID;
+    }
     try {
         return pool_run(p, pcm, n_in, sample_rates, batch, prompts, sampling, max_tokens, stop_on_eos, max_batch_per_gpu, ids_out, lens_out,
                         lp_out);
@@ -209,6 +227,13 @@ void q3asr_pool_destroy(q3asr_pool* p) {
     delete p;
 }
 
+int q3asr_pool_set_continuous(q3asr_pool* p, int enable) {
+    if (p == nullptr) return Q3ASR_ERR_INVALID;
+    std::lock_guard<std::mutex> run_lock(p->run_mu);  // not in the middle of a batch
+    p->continuous.store(enable != 0 ? 1 : 0);
+    return Q3ASR_OK;
+}
+
 const char* q3asr_pool_last_error(const q3asr_pool* p) { return p ? p->last_error.c_str() : g_create_error.c_str(); }
 
 int q3asr_pool_transcribe_ids(q3asr_pool* p, const float* const* pcm, const size_t* n_samples, int batch, const q3asr_prompt* prompts,
@@ -237,6 +262,7 @@ int pool_submit(q3asr_pool* p, const float* const* pcm, const size_t* n_samples,
                 const q3asr_sampling* sampling, int max_tokens, int stop_on_eos, int max_batch_per_gpu, bool want_lp, q3asr_job** out) {
     if (out) *out = nullptr;
     if (p == nullptr || pcm == nullptr || n_samples == nullptr || batch <= 0 || max_tokens <= 0 || out == nullptr) return Q3ASR_ERR_INVALID;
+    if (p->continuous.load() && !greedy_sampling(sampling)) return Q3ASR_ERR_INVALID;  // (see pool_transcribe_locked)
     q3asr_job* j = nullptr;
     try {
         j = new q3asr_job();

@@ -401,6 +401,8 @@ void model_commit(Handle* h) {
 
 void model_unload(Handle* h) {
     h->batch.reset();
+    h->adm[0].reset();
+    h->adm[1].reset();
     free_model(h);
     for (Tensor& t : h->tensors) {
         if (t.d) {

@@ -9,9 +9,11 @@
 //
 //   transcribe_batch <inputDir> [--output-dir D] [--model 0.6B|1.7B] [--model-dir DIR] [--language L] [--extensions wav]
 //                    [--jsonl] [--batch N] [--max-tokens N] [--window-seconds S] [--devices 0,1,...] [--workers-per-gpu W] [--list]
-//                    [--confidence]
+//                    [--confidence] [--continuous]
 // --confidence adds each file's average token log-probability (over all its windows, EOS included: include/q3asr.h) to its JSONL
 // record ("avg_logprob") and progress line — the score a caller uses to flag hallucinated or low-quality output.
+// --continuous runs each worker's share of a group as one continuous batch of at most --batch rows (<= 256): rows freed by EOS are
+// refilled with the waiting utterances (q3asr_pool_set_continuous).  The output is the same as without it.
 // Two pool workers per GPU by default: the decode steps of two batches in flight on one GPU interleave (each is a chain of
 // latency-bound launches), which measured +24 % aggregate throughput over one batch at a time (tools/pool_concurrency.py).
 // Without --model-dir the weights are random-init (this repo has no checkpoint offline); --list only prints the files.
@@ -102,7 +104,7 @@ struct Group {
 int main(int argc, char** argv) {
     std::string inputDir, outputDir, model = "0.6B", modelDir, extensions = "wav,flac,mp3", devicesArg = "0";
     std::optional<std::string> language;
-    bool jsonl = false, listOnly = false, confidence = false;
+    bool jsonl = false, listOnly = false, confidence = false, continuous = false;
     int batch = 256, maxTokens = 448, workersPerGpu = 2;
     float windowSeconds = 30.f;
     for (int i = 1; i < argc; i++) {
@@ -116,6 +118,7 @@ int main(int argc, char** argv) {
         else if (a == "--jsonl") jsonl = true;
         else if (a == "--list") listOnly = true;
         else if (a == "--confidence") confidence = true;
+        else if (a == "--continuous") continuous = true;
         else if (a == "--batch") batch = std::max(1, atoi(val().c_str()));
         else if (a == "--max-tokens") maxTokens = std::max(1, atoi(val().c_str()));
         else if (a == "--window-seconds") windowSeconds = (float)atof(val().c_str());
@@ -146,6 +149,10 @@ int main(int argc, char** argv) {
     if (q3asr_pool_create(&cfg, devices.data(), (int)devices.size(), 20260418, modelDir.empty() ? nullptr : modelDir.c_str(), &pool) != Q3ASR_OK) {
         fprintf(stderr, "Error: modelLoadFailed: %s\n", q3asr_last_error(nullptr));
         return 1;
+    }
+    if (continuous) {
+        batch = std::min(batch, 256);  // the resident rows of a continuous batch
+        q3asr_pool_set_continuous(pool, 1);
     }
     Tokenizer tok;
     if (!modelDir.empty()) {

@@ -92,6 +92,7 @@ EXPORTS = [
     "q3asr_pool_transcribe_ids_opts", "q3asr_pool_submit", "q3asr_job_done", "q3asr_job_wait", "q3asr_job_last_error", "q3asr_job_free",
     "q3asr_transcribe_ids_lp", "q3asr_batch_set_logprobs", "q3asr_batch_download_logprobs", "q3asr_pool_transcribe_ids_lp",
     "q3asr_pool_submit_lp", "q3asr_job_logprobs",
+    "q3asr_transcribe_ids_continuous", "q3asr_decode_admissions", "q3asr_pool_set_continuous",
 ]
 
 _lib = None
@@ -204,6 +205,9 @@ def lib():
         L.q3asr_pool_transcribe_ids_lp.argtypes = [vp, vp, vp, vp, ci, vp, ctypes.POINTER(Sampling), ci, ci, ci, vp, vp, vp]
         L.q3asr_pool_submit_lp.argtypes = [vp, vp, vp, vp, ci, vp, ctypes.POINTER(Sampling), ci, ci, ci, ctypes.POINTER(vp)]
         L.q3asr_job_logprobs.argtypes = [vp, vp]
+        L.q3asr_transcribe_ids_continuous.argtypes = [vp, vp, vp, vp, ci, vp, ci, ci, ci, vp, vp, vp]
+        L.q3asr_decode_admissions.argtypes = [vp, vp]
+        L.q3asr_pool_set_continuous.argtypes = [vp, ci]
         _lib = L
     return _lib
 
@@ -546,6 +550,13 @@ class Qwen3ASRModel:
         self._ck(lib().q3asr_decode_stats(self._h, out.ctypes.data))
         return dict(steps=int(out[0]), row_steps=int(out[1]), compactions=int(out[2]), rows=int(out[3]))
 
+    def decode_admissions(self):
+        """{admissions, admitted} of the last continuous-batching call (q3asr_decode_admissions): groups prefilled after the first
+        one, and the utterances in them."""
+        out = np.zeros(2, dtype=np.uint64)
+        self._ck(lib().q3asr_decode_admissions(self._h, out.ctypes.data))
+        return dict(admissions=int(out[0]), admitted=int(out[1]))
+
     # -- weights -----------------------------------------------------------------------------
     def tensor_names(self):
         out = []
@@ -597,16 +608,29 @@ class Qwen3ASRModel:
         return out[:ntok.value].copy()
 
     def transcribe_ids(self, clips, max_tokens=448, stop_on_eos=True, prompts=None, sample_rates=None, options=None,
-                       force_device_sampler=False, return_logprobs=False):
+                       force_device_sampler=False, return_logprobs=False, continuous_rows=None):
         """Batched transcription -> list of int32 id arrays (EOS included when it stops the loop).  sample_rates: per-clip
         rates; clips not at 16 kHz are converted on the device (AudioPreprocessing.swift:323-337).  options: a
         Qwen3DecodingOptions whose decoder knobs (repetition penalty, no-repeat n-gram, temperature) run as a device kernel.
-        return_logprobs: (ids, logprobs) lists instead, logprobs[i] the float32 log-probability of every id (q3asr_transcribe_ids_lp)."""
+        return_logprobs: (ids, logprobs) lists instead, logprobs[i] the float32 log-probability of every id (q3asr_transcribe_ids_lp).
+        continuous_rows: continuous batching (q3asr_transcribe_ids_continuous) — the request runs as one resident decode batch of at
+        most that many rows (0: 256), refilled with the waiting clips as rows finish; the same ids, greedy only."""
         clips = [np.ascontiguousarray(c, dtype=np.float32) for c in clips]
         n = np.array([c.size for c in clips], dtype=np.uint64)
         ids = np.zeros((len(clips), max_tokens), dtype=np.int32)
         lens = np.zeros(len(clips), dtype=np.int32)
         pp = _PromptPack(prompts, len(clips))
+        if continuous_rows is not None:
+            if options is not None:
+                raise ValueError("continuous_rows: greedy decoding only (no decoder options)")
+            sr = None if sample_rates is None else np.ascontiguousarray(sample_rates, dtype=np.int32)
+            lp = np.zeros((len(clips), max_tokens), dtype=np.float32) if return_logprobs else None
+            self._ck(lib().q3asr_transcribe_ids_continuous(self._h, ctypes.cast(_ptr_array(clips), ctypes.c_void_p), n.ctypes.data,
+                                                           sr.ctypes.data if sr is not None else None, len(clips), pp.ptr, int(max_tokens),
+                                                           int(bool(stop_on_eos)), int(continuous_rows), ids.ctypes.data, lens.ctypes.data,
+                                                           lp.ctypes.data if lp is not None else None))
+            out = [ids[i, :lens[i]].copy() for i in range(len(clips))]
+            return (out, [lp[i, :lens[i]].copy() for i in range(len(clips))]) if return_logprobs else out
         if return_logprobs:
             lp = np.zeros((len(clips), max_tokens), dtype=np.float32)
             sr = None if sample_rates is None else np.ascontiguousarray(sample_rates, dtype=np.int32)
@@ -1014,7 +1038,9 @@ class Qwen3Tokenizer:
 class Pool:
     """Utterance-batching scheduler over several GPUs of one process (q3asr_pool_*)."""
 
-    def __init__(self, size="0.6B", devices=(0,), seed=20260418, weights_dir=None, config=None):
+    def __init__(self, size="0.6B", devices=(0,), seed=20260418, weights_dir=None, config=None, continuous=False):
+        """continuous: each worker runs its whole share as one continuous batch of max_batch_per_gpu rows
+        (q3asr_pool_set_continuous); greedy decoding only."""
         self.cfg = config if config is not None else preset(size)
         dev = np.ascontiguousarray(devices, dtype=np.int32)
         self._p = ctypes.c_void_p()
@@ -1022,6 +1048,11 @@ class Pool:
                                      os.fspath(weights_dir).encode() if weights_dir else None, ctypes.byref(self._p))
         if rc != OK:
             raise Q3Error(rc, "pool_create failed: " + lib().q3asr_pool_last_error(None).decode())
+        if continuous:
+            rc = lib().q3asr_pool_set_continuous(self._p, 1)
+            if rc != OK:
+                self.close()
+                raise Q3Error(rc, "pool_set_continuous failed")
 
     def transcribe_ids(self, clips, max_tokens=448, stop_on_eos=True, max_batch_per_gpu=64, sample_rates=None, options=None,
                        return_logprobs=False):
