@@ -410,6 +410,19 @@ int q3asr_debug_attention(q3asr_handle* h, const uint16_t* q, const uint16_t* k,
                           int head_dim, const int* seg_row0, const int* seg_len, int n_segs, int causal, float scale, int kernel,
                           uint16_t* out);
 
+/* Decode-step attention of one layer for n_seqs sequences, as the decode step runs it (head_dim 128; needs a loaded model, whose
+ * RoPE frequencies are used).  qkv_part: fp32 split-K partials of the QKV product [splits][n_seqs][(heads + 2*kv_heads)*128];
+ * q_norm / k_norm: bf16 [128]; kv_len[s] includes the new token, whose position is kv_len[s] - 1; page_table [n_seqs][max_pages],
+ * every entry in [0, n_pages); pool [n_pages][layers][2][kv_heads][32][128] bf16, in/out (the new k and v are appended at `layer`).
+ * variant: 0 = the decode step's own choice, 1 / 2 / 8 = the tensor-core kernel (1: two single-warp CTAs per item), 4 / 16 = the
+ * SIMT kernel's 4 / 16 warps (these need heads == 2*kv_heads); -1 = the general path (partials summed on the host in split order,
+ * rounded to bf16, then the separate norm + RoPE + append kernel and the paged attention kernel; heads / kv_heads 1 or 2).
+ * The same launch runs `launches` times back to back on the same buffers.  out: [launches][n_seqs][heads*128] bf16. */
+int q3asr_debug_decode_attention(q3asr_handle* h, const float* qkv_part, int splits, int n_seqs, int heads, int kv_heads,
+                                 const uint16_t* q_norm, const uint16_t* k_norm, float eps, float scale, const int* kv_len,
+                                 const int* page_table, int max_pages, uint16_t* pool, int n_pages, int layers, int layer, int variant,
+                                 int launches, uint16_t* out);
+
 #ifdef __cplusplus
 }
 #endif

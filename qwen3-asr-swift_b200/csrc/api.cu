@@ -53,6 +53,21 @@ void set_common_tokens(q3asr_config* c) {
     c->tok_timestamp = 151705;
 }
 
+// the device buffers of one debug-hook call, freed on every exit path
+struct DebugAllocs {
+    std::vector<void*> p;
+    template <typename T>
+    T* get(size_t n) {
+        void* q = nullptr;
+        Q3_CUDA(cudaMalloc(&q, n * sizeof(T)));
+        p.push_back(q);
+        return static_cast<T*>(q);
+    }
+    ~DebugAllocs() {
+        for (void* q : p) cudaFree(q);
+    }
+};
+
 }  // namespace
 
 extern "C" {
@@ -721,6 +736,77 @@ int q3asr_debug_attention(q3asr_handle* hh, const uint16_t* q, const uint16_t* k
         }
         cudaFree(dq); cudaFree(dk); cudaFree(dv); cudaFree(dout); cudaFree(dseg);
         Q3_CUDA(se);
+    });
+}
+
+int q3asr_debug_decode_attention(q3asr_handle* hh, const float* qkv_part, int splits, int n_seqs, int heads, int kv_heads,
+                                 const uint16_t* q_norm, const uint16_t* k_norm, float eps, float scale, const int* kv_len,
+                                 const int* page_table, int max_pages, uint16_t* pool, int n_pages, int layers, int layer, int variant,
+                                 int launches, uint16_t* out) {
+    return guarded(hh, [&](Handle& h) {
+        Q3_CHECK(h.loaded && h.model, Q3ASR_ERR_STATE, "debug_decode_attention: no model loaded (the RoPE frequencies come from it)");
+        Q3_CHECK(qkv_part && q_norm && k_norm && kv_len && page_table && pool && out && splits >= 1 && n_seqs >= 1 && kv_heads >= 1 &&
+                     heads >= 1 && max_pages >= 1 && n_pages >= 1 && layers >= 1 && layer >= 0 && layer < layers && launches >= 1,
+                 Q3ASR_ERR_INVALID, "debug_decode_attention: bad argument");
+        Q3_CHECK(variant == -1 || variant == 0 || variant == 1 || variant == 2 || variant == 4 || variant == 8 || variant == 16,
+                 Q3ASR_ERR_INVALID, "debug_decode_attention: variant must be -1, 0, 1, 2, 4, 8 or 16");
+        Q3_CHECK(variant == -1 ? (heads == kv_heads || heads == 2 * kv_heads) : heads == 2 * kv_heads, Q3ASR_ERR_INVALID,
+                 "debug_decode_attention: the fused kernels take 2 query heads per kv head, the general path 1 or 2");
+        for (size_t i = 0; i < (size_t)n_seqs * max_pages; i++)
+            Q3_CHECK(page_table[i] >= 0 && page_table[i] < n_pages, Q3ASR_ERR_INVALID, "debug_decode_attention: page-table entry out of range");
+        for (int s = 0; s < n_seqs; s++)
+            Q3_CHECK(kv_len[s] >= 1 && kv_len[s] <= max_pages * KV_PAGE, Q3ASR_ERR_INVALID, "debug_decode_attention: kv_len out of range");
+        const int nqkv = (heads + 2 * kv_heads) * 128, n_pos = max_pages * KV_PAGE;
+        const size_t part_n = (size_t)splits * n_seqs * nqkv, out_n = (size_t)n_seqs * heads * 128;
+        const size_t pool_n = (size_t)n_pages * layers * 2 * kv_heads * KV_PAGE * 128;
+        DebugAllocs a;
+        std::vector<int> pos(n_seqs), row_seq(n_seqs);
+        for (int s = 0; s < n_seqs; s++) { pos[s] = kv_len[s] - 1; row_seq[s] = s; }
+        float* dpart = a.get<float>(part_n);
+        bf16 *dqw = a.get<bf16>(128), *dkw = a.get<bf16>(128), *dpool = a.get<bf16>(pool_n), *dout = a.get<bf16>(out_n * launches);
+        int *dlen = a.get<int>(n_seqs), *dpos = a.get<int>(n_seqs), *dpt = a.get<int>((size_t)n_seqs * max_pages);
+        float2* drope = a.get<float2>((size_t)n_pos * 64);
+        Q3_H2D_SYNC(dpart, qkv_part, sizeof(float) * part_n);
+        Q3_H2D_SYNC(dqw, q_norm, 2 * 128);
+        Q3_H2D_SYNC(dkw, k_norm, 2 * 128);
+        Q3_H2D_SYNC(dpool, pool, 2 * pool_n);
+        Q3_H2D_SYNC(dlen, kv_len, sizeof(int) * n_seqs);
+        Q3_H2D_SYNC(dpos, pos.data(), sizeof(int) * n_seqs);
+        Q3_H2D_SYNC(dpt, page_table, sizeof(int) * (size_t)n_seqs * max_pages);
+        rope_table_launch(h.model->inv_freq, n_pos, drope, nullptr, h.stream);
+        const KvCache cache{dpool, dpt, max_pages, layers, kv_heads, 128};
+        if (variant == -1) {  // the general path: the product's bf16 rounding of q|k|v, then the separate norm + RoPE + append kernel
+            std::vector<bf16> qkv((size_t)n_seqs * nqkv);
+            for (size_t i = 0; i < qkv.size(); i++) {
+                float acc = 0.f;
+                for (int sp = 0; sp < splits; sp++) acc += qkv_part[(size_t)sp * n_seqs * nqkv + i];
+                qkv[i] = __float2bfloat16_rn(acc);
+            }
+            bf16 *dqkv = a.get<bf16>(qkv.size()), *dq = a.get<bf16>(out_n);
+            int* drow = a.get<int>(n_seqs);
+            Q3_H2D_SYNC(dqkv, qkv.data(), 2 * qkv.size());
+            Q3_H2D_SYNC(drow, row_seq.data(), sizeof(int) * n_seqs);
+            for (int i = 0; i < launches; i++) {
+                qknorm_rope_kv_launch(dqkv, nqkv, dqw, dkw, dpos, drow, n_seqs, heads, kv_heads, eps, drope, dq, nullptr, nullptr, cache, layer,
+                                      h.stream);
+                decode_attn_launch(dq, cache, layer, dlen, n_seqs, heads, scale, dout + i * out_n, h.stream);
+            }
+        } else {  // the fused kernels; the split variant's counters start at zero, as reserve_decoder leaves them
+            float* dsplit = a.get<float>(decode_attn_split_floats(n_seqs, kv_heads));
+            int* dcnt = a.get<int>((size_t)n_seqs * kv_heads);
+            Q3_CUDA(cudaMemsetAsync(dcnt, 0, sizeof(int) * n_seqs * kv_heads, h.stream));
+            struct PdlOn {  // back-to-back launches overlap as in the decode step: each one's prefetch runs ahead of the previous launch's end
+                bool prev = pdl_enabled();
+                PdlOn() { pdl_enabled() = true; }
+                ~PdlOn() { pdl_enabled() = prev; }
+            } pdl;
+            for (int i = 0; i < launches; i++)
+                decode_attn_fused_launch(dpart, splits, (long long)n_seqs * nqkv, nqkv, dqw, dkw, dpos, eps, drope, cache, layer, dlen, n_seqs,
+                                         heads, scale, dout + i * out_n, h.num_sms, h.stream, dsplit, dcnt, variant);
+        }
+        Q3_CUDA(cudaStreamSynchronize(h.stream));
+        Q3_CUDA(cudaMemcpy(out, dout, 2 * out_n * launches, cudaMemcpyDeviceToHost));
+        Q3_CUDA(cudaMemcpy(pool, dpool, 2 * pool_n, cudaMemcpyDeviceToHost));
     });
 }
 

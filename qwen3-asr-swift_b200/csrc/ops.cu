@@ -1324,10 +1324,13 @@ void decode_attn_launch(const bf16* q, const KvCache& cache, int layer, const in
 
 void decode_attn_fused_launch(const float* qkv_part, int splits, long long split_stride, int nqkv, const bf16* qw, const bf16* kw,
                               const int* pos, float eps, const float2* rope_tab, const KvCache& cache, int layer, const int* kv_len,
-                              int n_seqs, int heads, float scale, bf16* out, int num_sms, cudaStream_t st, float* split_part, int* split_cnt) {
+                              int n_seqs, int heads, float scale, bf16* out, int num_sms, cudaStream_t st, float* split_part, int* split_cnt,
+                              int force) {
     if (n_seqs <= 0) return;
     Q3_CHECK(cache.head_dim == 128, 1, "decoder head_dim must be 128");
     Q3_CHECK(heads == 2 * cache.kv_heads, 1, "fused decode attention is built for 2 query heads per kv head");
+    Q3_CHECK(force == 0 || force == 2 || force == 4 || force == 8 || force == 16 || (force == 1 && split_part != nullptr && split_cnt != nullptr), 1,
+             "fused decode attention: unknown variant");
     const float sl2 = scale * 1.4426950408889634f;
     dim3 grid(n_seqs, cache.kv_heads);
     // few (sequence, head) pairs: more warps per CTA so that short batches still spread the key loop
@@ -1349,7 +1352,12 @@ void decode_attn_fused_launch(const float* qkv_part, int splits, long long split
         const int w = atoi(f);
         if (w == 2 || w == 8 || (w == 1 && split_part != nullptr && split_cnt != nullptr)) warps = w;
     }
-    static const bool simt = getenv("Q3ASR_DECODE_ATTN_SIMT") != nullptr && atoi(getenv("Q3ASR_DECODE_ATTN_SIMT")) != 0;
+    static const bool simt_env = getenv("Q3ASR_DECODE_ATTN_SIMT") != nullptr && atoi(getenv("Q3ASR_DECODE_ATTN_SIMT")) != 0;
+    bool simt = simt_env;
+    if (force != 0) {  // the kernel test hook names the variant: 1, 2, 8 = the tensor-core kernel's warps, 4, 16 = the SIMT kernel's
+        simt = force == 4 || force == 16;
+        warps = force == 16 ? 8 : force == 4 ? 2 : force;
+    }
     if (!simt) {
         if (warps == 1)
             launch_kernel(decode_attn_mma_kernel<1, true>, dim3(n_seqs, cache.kv_heads, 2), 32, decode_attn_mma_smem(1), st, qkv_part, splits,

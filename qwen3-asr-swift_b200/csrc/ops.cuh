@@ -67,10 +67,12 @@ void decode_attn_launch(const bf16* q /*[n_seqs, heads*hd]*/, const KvCache& cac
 
 // Decode step, fused: sums the split-K partials of the QKV product (fp32 [splits][n_seqs][nqkv]), applies q/k-norm + RoPE,
 // appends k/v to the cache and attends (one launch instead of qknorm_rope_kv + decode_attn).
+// force (kernel tests): 0 = the choice for this batch and SM count (environment switches included); 1 = the split tensor-core variant
+// (needs split_part / split_cnt), 2 / 8 = the tensor-core kernel with 2 / 8 warps, 4 / 16 = the SIMT kernel with 4 / 16 warps.
 void decode_attn_fused_launch(const float* qkv_part, int splits, long long split_stride, int nqkv, const bf16* qw, const bf16* kw,
                               const int* pos, float eps, const float2* rope_tab, const KvCache& cache, int layer, const int* kv_len,
                               int n_seqs, int heads, float scale, bf16* out, int num_sms, cudaStream_t st, float* split_part = nullptr,
-                              int* split_cnt = nullptr);
+                              int* split_cnt = nullptr, int force = 0);
 // scratch of the split variant (two single-warp CTAs per (sequence, kv head)): floats for the partials, counters (zero before the first launch)
 constexpr size_t decode_attn_split_floats(size_t n_seqs, size_t kv_heads) { return n_seqs * kv_heads * 2 * 264; }
 // x += bf16(sum of split-K partials) (in place), y = RMSNorm(x) * w.  d % 128 == 0, d <= 2048.

@@ -82,7 +82,7 @@ EXPORTS = [
     "q3asr_timer_record", "q3asr_timer_elapsed_ms", "q3asr_stage_ms", "q3asr_launch_count", "q3asr_decode_stats", "q3asr_flush_l2",
     "q3asr_profile", "q3asr_profile_report",
     "q3asr_pool_create", "q3asr_pool_destroy", "q3asr_pool_last_error", "q3asr_pool_transcribe_ids", "q3asr_schedule",
-    "q3asr_debug_gemm", "q3asr_debug_conv", "q3asr_debug_attention",
+    "q3asr_debug_gemm", "q3asr_debug_conv", "q3asr_debug_attention", "q3asr_debug_decode_attention",
     "q3asr_tokenizer_load", "q3asr_tokenizer_from_pairs", "q3asr_tokenizer_add_merge", "q3asr_tokenizer_destroy",
     "q3asr_tokenizer_last_error", "q3asr_tokenizer_size", "q3asr_tokenizer_decode", "q3asr_tokenizer_encode", "q3asr_tokenizer_token_id",
     "q3asr_io_last_error", "q3asr_wav_parse", "q3asr_wav_load", "q3asr_wav_write", "q3asr_resample_len", "q3asr_resample", "q3asr_resample_design",
@@ -170,6 +170,8 @@ def lib():
         L.q3asr_debug_gemm.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, ci, vp]
         L.q3asr_debug_conv.argtypes = [vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, ci, ci, ci, vp]
         L.q3asr_debug_attention.argtypes = [vp, vp, vp, vp, ci, ci, ci, ci, vp, vp, ci, ci, ctypes.c_float, ci, vp]
+        L.q3asr_debug_decode_attention.argtypes = [vp, vp, ci, ci, ci, ci, vp, vp, ctypes.c_float, ctypes.c_float, vp, vp, ci, vp, ci, ci,
+                                                   ci, ci, ci, vp]
         L.q3asr_tokenizer_load.argtypes = [ctypes.c_char_p, ctypes.POINTER(vp)]
         L.q3asr_tokenizer_from_pairs.argtypes = [vp, vp, ci, ctypes.POINTER(vp)]
         L.q3asr_tokenizer_add_merge.argtypes = [vp, ctypes.c_char_p, ctypes.c_char_p]
@@ -956,6 +958,30 @@ class Qwen3ASRModel:
                                              r0.ctypes.data, ln.ctypes.data, len(segs), int(bool(causal)), ctypes.c_float(scale),
                                              int(kernel), out.ctypes.data))
         return bf16_bits_to_f32(out)
+
+    def debug_decode_attention(self, qkv_part, heads, kv_heads, q_norm, k_norm, kv_len, page_table, pool, layer, variant=0, launches=1,
+                               eps=1e-6, scale=None):
+        """One layer's decode-step attention (q3asr_debug_decode_attention).  qkv_part float32 [splits, n_seqs, (heads + 2*kv_heads)*128];
+        q_norm / k_norm float32 [128] holding bf16 values; kv_len [n_seqs] (new token included); page_table [n_seqs, max_pages];
+        pool uint16 (bf16 bits) [n_pages, layers, 2, kv_heads, 32, 128].  Returns (out float32 [launches, n_seqs, heads*128],
+        the pool after the calls, uint16)."""
+        part = np.ascontiguousarray(qkv_part, dtype=np.float32)
+        splits, n_seqs, nqkv = part.shape
+        assert nqkv == (heads + 2 * kv_heads) * 128
+        qw, kw = f32_to_bf16_bits(np.asarray(q_norm, np.float32)), f32_to_bf16_bits(np.asarray(k_norm, np.float32))
+        lens = np.ascontiguousarray(kv_len, dtype=np.int32)
+        pt = np.ascontiguousarray(page_table, dtype=np.int32)
+        pool = np.array(pool, dtype=np.uint16, order="C")  # a copy: the call writes the appended k / v into it
+        n_pages, layers = pool.shape[0], pool.shape[1]
+        assert pool.shape[2:] == (2, kv_heads, 32, 128) and pt.shape[0] == n_seqs and lens.shape == (n_seqs,)
+        if scale is None:
+            scale = 1.0 / np.sqrt(128.0)
+        out = np.empty((launches, n_seqs, heads * 128), dtype=np.uint16)
+        self._ck(lib().q3asr_debug_decode_attention(self._h, part.ctypes.data, splits, n_seqs, heads, kv_heads, qw.ctypes.data, kw.ctypes.data,
+                                                    ctypes.c_float(eps), ctypes.c_float(scale), lens.ctypes.data, pt.ctypes.data, pt.shape[1],
+                                                    pool.ctypes.data, n_pages, layers, int(layer), int(variant), int(launches),
+                                                    out.ctypes.data))
+        return bf16_bits_to_f32(out), pool
 
     def debug_conv(self, x, w, bias, box=(0, 0, 0), simt=False):
         """x [B,H,W,C], w [O,3,3,C] float32 (bf16-representable) -> gelu(conv3x3 s2 p1 + bias) [B,OH,OW,O]."""

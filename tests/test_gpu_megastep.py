@@ -47,6 +47,35 @@ def test_megastep_matches_multi_kernel_path(built_lib, monkeypatch, size, batche
         m.close()
 
 
+def test_megastep_matches_multi_kernel_path_at_long_context(built_lib, monkeypatch):
+    """Contexts of 500 to 1 200 keys: every one of the 8 key streams of an attention item holds several 16-key chunks, so the
+    persistent kernel's own copy of the attention body (megastep.cuh attention_item) runs its chunk walk, the online-softmax
+    rescale within a stream and the stream merge at depth; the short-clip tests above stay within one or two chunks per stream.
+    The multi-kernel side is pinned to a float64 reference by test_gpu_decode_attention.py."""
+    m = built_lib.Qwen3ASRModel.random_init("0.6B", seed=20260418)
+    try:
+        clips = [synth.clip(900 + i, 16000 * 30 - 1111 * i) for i in range(6)]
+        context = np.random.default_rng(11).integers(0, 150000, size=600).astype(np.int32)
+        prompts = [None] * 5 + [{"context": context}]
+        runs, launches = [], []
+        for mega in ("0", "1"):
+            monkeypatch.setenv("Q3ASR_MEGA", mega)
+            l0 = m.launch_count
+            runs.append([t.tolist() for t in m.transcribe_ids(clips, max_tokens=160, stop_on_eos=False, prompts=prompts)])
+            launches.append(m.launch_count - l0)
+        assert runs[1] == runs[0], [i for i, (a, b) in enumerate(zip(runs[0], runs[1])) if a != b]
+        assert all(len(t) == 160 for t in runs[0])
+        assert launches[1] < launches[0], launches  # the persistent kernel really ran
+        forced = np.random.default_rng(12).integers(0, 150000, size=300).astype(np.int32)
+        monkeypatch.setenv("Q3ASR_MEGA", "0")
+        ids0, top0 = m.decode_forced(clips[0], forced)
+        monkeypatch.setenv("Q3ASR_MEGA", "1")
+        ids1, top1 = m.decode_forced(clips[0], forced)
+        assert ids0.tolist() == ids1.tolist() and top0.tolist() == top1.tolist()
+    finally:
+        m.close()
+
+
 def test_megastep_stop_on_eos_and_long_decode(built_lib, monkeypatch):
     """A longer decode (KV pages cross several page boundaries, contexts of different lengths in one batch) and the EOS path."""
     m = built_lib.Qwen3ASRModel.random_init("0.6B", seed=20260418)
