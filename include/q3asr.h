@@ -423,6 +423,23 @@ int q3asr_debug_decode_attention(q3asr_handle* h, const float* qkv_part, int spl
                                  const int* page_table, int max_pages, uint16_t* pool, int n_pages, int layers, int layer, int variant,
                                  int launches, uint16_t* out);
 
+/* One decoder layer's prefill attention block for packed prompts, through the same host function as the prefill (head_dim 128;
+ * needs a loaded model, whose RoPE frequencies are tabulated for max_pages*32 positions).  x: the normed hidden states
+ * [rows][hidden] bf16; w: the fused weight [(heads + 2*kv_heads)*128][hidden] bf16 in q | k | v row order; q_norm / k_norm: bf16
+ * [128].  Segment s holds rows seg_row0[s] .. + seg_len[s] - 1 at positions 0 .. seg_len[s] - 1, and its KV pages are
+ * page_table row seg_table_row[s]; the segments are packed back to back from row 0 and cover the rows.  page_table
+ * [table_rows][max_pages], every entry in [0, n_pages); pool [n_pages][layers][2][kv_heads][32][128] bf16, in/out (k and v are
+ * written at `layer`).  qkv_variant: 0 = norm, RoPE and cache write in the product's epilogue (the prefill's path), -1 = the plain
+ * product + the separate norm / RoPE / cache kernel.  bn: the product's tile width, 0 = the prefill's choice, or 128 / 256.
+ * attn_variant: 0 = the tcgen05 kernel (the prefill's), 1 = the mma.sync kernel, -1 = none.  Outputs (bf16): q_out [rows][heads*128],
+ * k_out [rows][kv_heads*128], qkv_out [rows][(heads + 2*kv_heads)*128] (under qkv_variant 0 only its v columns are written),
+ * att_out [rows][heads*128]; whatever the call does not write reads back as NaN. */
+int q3asr_debug_prefill_attention(q3asr_handle* h, const uint16_t* x, const uint16_t* w, int rows, int hidden, int heads, int kv_heads,
+                                  const uint16_t* q_norm, const uint16_t* k_norm, float eps, float scale, const int* seg_row0,
+                                  const int* seg_len, const int* seg_table_row, int n_segs, const int* page_table, int table_rows,
+                                  int max_pages, uint16_t* pool, int n_pages, int layers, int layer, int qkv_variant, int bn,
+                                  int attn_variant, uint16_t* q_out, uint16_t* k_out, uint16_t* qkv_out, uint16_t* att_out);
+
 #ifdef __cplusplus
 }
 #endif

@@ -810,4 +810,73 @@ int q3asr_debug_decode_attention(q3asr_handle* hh, const float* qkv_part, int sp
     });
 }
 
+int q3asr_debug_prefill_attention(q3asr_handle* hh, const uint16_t* x, const uint16_t* w, int rows, int hidden, int heads, int kv_heads,
+                                  const uint16_t* q_norm, const uint16_t* k_norm, float eps, float scale, const int* seg_row0,
+                                  const int* seg_len, const int* seg_table_row, int n_segs, const int* page_table, int table_rows,
+                                  int max_pages, uint16_t* pool, int n_pages, int layers, int layer, int qkv_variant, int bn,
+                                  int attn_variant, uint16_t* q_out, uint16_t* k_out, uint16_t* qkv_out, uint16_t* att_out) {
+    return guarded(hh, [&](Handle& h) {
+        Q3_CHECK(h.loaded && h.model, Q3ASR_ERR_STATE, "debug_prefill_attention: no model loaded (the RoPE frequencies come from it)");
+        Q3_CHECK(x && w && q_norm && k_norm && seg_row0 && seg_len && seg_table_row && page_table && pool && q_out && k_out && qkv_out &&
+                     att_out && rows >= 1 && hidden >= 64 && hidden % 64 == 0 && heads >= 1 && kv_heads >= 1 && heads % kv_heads == 0 &&
+                     n_segs >= 1 && table_rows >= 1 && max_pages >= 1 && n_pages >= 1 && layers >= 1 && layer >= 0 && layer < layers,
+                 Q3ASR_ERR_INVALID, "debug_prefill_attention: bad argument");
+        const int nq = heads * 128, nkv = kv_heads * 128, nqkv = nq + 2 * nkv, n_pos = max_pages * KV_PAGE;
+        Q3_CHECK(qkv_variant == 0 || qkv_variant == -1, Q3ASR_ERR_INVALID, "debug_prefill_attention: qkv_variant must be 0 or -1");
+        Q3_CHECK(bn == 0 || ((bn == 128 || bn == 256) && nqkv % bn == 0), Q3ASR_ERR_INVALID,
+                 "debug_prefill_attention: bn must be 0, or 128 / 256 dividing (heads + 2 kv_heads) * 128");
+        Q3_CHECK(attn_variant >= -1 && attn_variant <= 1, Q3ASR_ERR_INVALID, "debug_prefill_attention: attn_variant must be -1, 0 or 1");
+        for (size_t i = 0; i < (size_t)table_rows * max_pages; i++)
+            Q3_CHECK(page_table[i] >= 0 && page_table[i] < n_pages, Q3ASR_ERR_INVALID, "debug_prefill_attention: page-table entry out of range");
+        // the segments tile the rows back to back, as the batch plan packs the prompts
+        std::vector<int> pos(rows), row_seq(rows);
+        int next = 0, max_len = 0;
+        for (int s = 0; s < n_segs; s++) {
+            Q3_CHECK(seg_row0[s] == next && seg_len[s] >= 1 && seg_len[s] <= n_pos && seg_len[s] <= rows - next, Q3ASR_ERR_INVALID,
+                     "debug_prefill_attention: segments must be packed back to back, each within the table's positions");
+            Q3_CHECK(seg_table_row[s] >= 0 && seg_table_row[s] < table_rows, Q3ASR_ERR_INVALID,
+                     "debug_prefill_attention: segment table row out of range");
+            for (int i = 0; i < seg_len[s]; i++) {
+                pos[next + i] = i;
+                row_seq[next + i] = seg_table_row[s];
+            }
+            next += seg_len[s];
+            max_len = std::max(max_len, seg_len[s]);
+        }
+        Q3_CHECK(next == rows, Q3ASR_ERR_INVALID, "debug_prefill_attention: the segments must cover the rows");
+        const size_t pool_n = (size_t)n_pages * layers * 2 * kv_heads * KV_PAGE * 128;
+        DebugAllocs a;
+        bf16 *dx = a.get<bf16>((size_t)rows * hidden), *dw = a.get<bf16>((size_t)nqkv * hidden), *dqw = a.get<bf16>(128),
+             *dkw = a.get<bf16>(128), *dpool = a.get<bf16>(pool_n), *dqkv = a.get<bf16>((size_t)rows * nqkv), *dq = a.get<bf16>((size_t)rows * nq),
+             *dk = a.get<bf16>((size_t)rows * nkv), *datt = a.get<bf16>((size_t)rows * nq);
+        int *dpt = a.get<int>((size_t)table_rows * max_pages), *dpos = a.get<int>(rows), *drow = a.get<int>(rows), *dseg = a.get<int>(2 * (size_t)n_segs);
+        float2 *drope = a.get<float2>((size_t)n_pos * 64), *drope_t = a.get<float2>((size_t)n_pos * 64);
+        Q3_H2D_SYNC(dx, x, 2 * (size_t)rows * hidden);
+        Q3_H2D_SYNC(dw, w, 2 * (size_t)nqkv * hidden);
+        Q3_H2D_SYNC(dqw, q_norm, 2 * 128);
+        Q3_H2D_SYNC(dkw, k_norm, 2 * 128);
+        Q3_H2D_SYNC(dpool, pool, 2 * pool_n);
+        Q3_H2D_SYNC(dpt, page_table, sizeof(int) * (size_t)table_rows * max_pages);
+        Q3_H2D_SYNC(dpos, pos.data(), sizeof(int) * rows);
+        Q3_H2D_SYNC(drow, row_seq.data(), sizeof(int) * rows);
+        Q3_H2D_SYNC(dseg, seg_row0, sizeof(int) * n_segs);
+        Q3_H2D_SYNC(dseg + n_segs, seg_len, sizeof(int) * n_segs);
+        // every output element the call does not write reads back as bf16 NaN (0xFFFF)
+        Q3_CUDA(cudaMemsetAsync(dqkv, 0xFF, 2 * (size_t)rows * nqkv, h.stream));
+        Q3_CUDA(cudaMemsetAsync(dq, 0xFF, 2 * (size_t)rows * nq, h.stream));
+        Q3_CUDA(cudaMemsetAsync(dk, 0xFF, 2 * (size_t)rows * nkv, h.stream));
+        Q3_CUDA(cudaMemsetAsync(datt, 0xFF, 2 * (size_t)rows * nq, h.stream));
+        rope_table_launch(h.model->inv_freq, n_pos, drope, drope_t, h.stream);
+        const PrefillAttn pa{dx, dw, dqw, dkw, rows, hidden, heads, kv_heads, eps, scale, dpos, drow, AttnSegs{dseg, dseg + n_segs, n_segs, max_len},
+                             drope, drope_t, n_pos, KvCache{dpool, dpt, max_pages, layers, kv_heads, 128}, layer, dqkv, dq, dk, datt};
+        prefill_attention(&h, pa, qkv_variant == 0, bn, attn_variant, 0.0);
+        Q3_CUDA(cudaStreamSynchronize(h.stream));
+        Q3_CUDA(cudaMemcpy(q_out, dq, 2 * (size_t)rows * nq, cudaMemcpyDeviceToHost));
+        Q3_CUDA(cudaMemcpy(k_out, dk, 2 * (size_t)rows * nkv, cudaMemcpyDeviceToHost));
+        Q3_CUDA(cudaMemcpy(qkv_out, dqkv, 2 * (size_t)rows * nqkv, cudaMemcpyDeviceToHost));
+        Q3_CUDA(cudaMemcpy(att_out, datt, 2 * (size_t)rows * nq, cudaMemcpyDeviceToHost));
+        Q3_CUDA(cudaMemcpy(pool, dpool, 2 * pool_n, cudaMemcpyDeviceToHost));
+    });
+}
+
 }  // extern "C"

@@ -480,6 +480,7 @@ void decoder_layers(Handle* h, BatchState* bs, int rows, bool prefill) {
     const int* row_seq = prefill ? ints + bs->o_row_seq : ints + bs->o_ident;
     AttnSegs segs{ints + bs->o_seq_row0, ints + bs->o_seq_len, bs->B, bs->max_prompt};
     const bool fuse_qkv = hd == 128 && env_int("Q3ASR_NO_QKV_FUSE", 0) == 0;  // "1": the separate norm + RoPE kernel (the checker)
+    const int attn = env_int("Q3ASR_ATTN_MMASYNC", 0) == 0 ? 0 : 1;  // tcgen05 attention unless the mma.sync checker kernel is asked for
     double causal_pairs = 0;  // sum over prompts of S(S+1)/2
     for (const ClipInfo& ci : bs->clips) causal_pairs += 0.5 * ci.prompt_len * (ci.prompt_len + 1.0);
     for (int l = 0; l < c.dec_layers; l++) {
@@ -492,33 +493,22 @@ void decoder_layers(Handle* h, BatchState* bs, int rows, bool prefill) {
         };
         tag("pre_norm", "dec_norm", 0, 4.0 * Rd * H);
         rmsnorm_launch(x, w.in_ln, xn, rows, H, c.dec_rms_eps, nullptr, st);
-        tag("pre_qkv", "dec_qkv", 2.0 * Rd * H * nqkv, 2.0 * H * nqkv);
-        if (prefill && fuse_qkv) {
-            // per-head RMSNorm + RoPE + the paged-KV write happen in the product's epilogue (gemm.cuh EPI_QKV): q, k and the cache
-            // are written once, the raw product never reaches memory (v does, as is: the attention reads it from there)
-            GemmEpiArgs e;
-            e.epi = EPI_QKV;
-            e.out = qkv;
-            e.ldo = nqkv;
-            e.rp = QkvRope{pos, row_seq, bs->rope_tab_t.as<float2>(), bs->rope_n, w.q_norm, w.k_norm, q, bs->dkc.as<bf16>(), kc.pool, kc.page_table,
-                           kc.max_pages, kc.layers, l, c.dec_heads, c.dec_kv_heads, c.dec_rms_eps};
-            gemm(xn, H, rows, H, w.qkv_w, nqkv, e, st);
+        if (prefill) {
+            delete ps;
+            ps = nullptr;
+            const PrefillAttn pa{xn, w.qkv_w, w.q_norm, w.k_norm, rows, H, c.dec_heads, c.dec_kv_heads, c.dec_rms_eps, scale, pos, row_seq,
+                                 segs, bs->rope_tab.as<float2>(), bs->rope_tab_t.as<float2>(), bs->rope_n, kc, l, qkv, q,
+                                 bs->dkc.as<bf16>(), att};
+            prefill_attention(h, pa, fuse_qkv, 0, attn, causal_pairs);
         } else {
+            tag("pre_qkv", "dec_qkv", 2.0 * Rd * H * nqkv, 2.0 * H * nqkv);
             gemm(xn, H, rows, H, w.qkv_w, nqkv, epi_store(qkv, nqkv, nullptr), st);
             tag("pre_rope", "dec_rope", 0, 4.0 * Rd * nqkv);
-            // v is not transformed: the prefill attention reads it straight from the QKV product, only k needs a contiguous copy
             qknorm_rope_kv_launch(qkv, nqkv, w.q_norm, w.k_norm, pos, row_seq, rows, c.dec_heads, c.dec_kv_heads, c.dec_rms_eps,
-                                  bs->rope_tab.as<float2>(), q, prefill ? bs->dkc.as<bf16>() : nullptr, nullptr, kc, l, st);
-        }
-        tag("pre_attn", "dec_attn", prefill ? 4.0 * causal_pairs * nq : 0, 0);
-        if (prefill && env_int("Q3ASR_ATTN_MMASYNC", 0) == 0)
-            flash_attn_tc_launch(q, nq, bs->dkc.as<bf16>(), nkv, qkv + nq + nkv, nqkv, att, nq, segs, rows, c.dec_heads,
-                                 c.dec_heads / c.dec_kv_heads, hd, true, scale, st);
-        else if (prefill)
-            flash_attn_launch(q, nq, bs->dkc.as<bf16>(), nkv, qkv + nq + nkv, nqkv, att, nq, segs, c.dec_heads,
-                              c.dec_heads / c.dec_kv_heads, hd, true, scale, st);
-        else
+                                  bs->rope_tab.as<float2>(), q, nullptr, nullptr, kc, l, st);
+            tag("pre_attn", "dec_attn", 0, 0);
             decode_attn_launch(q, kc, l, bs->st_kv_len.as<int>(), rows, c.dec_heads, scale, att, st);
+        }
         tag("pre_o", "dec_o", 2.0 * Rd * nq * H, 2.0 * nq * H);
         gemm(att, nq, rows, nq, w.o_w, H, epi_store(x, H, nullptr, 0, x, H), st);
         tag("pre_norm", "dec_norm", 0, 4.0 * Rd * H);
@@ -911,6 +901,40 @@ void run_decode(Handle* h, BatchState* bs, int max_tokens, int stop_on_eos, bool
 }
 
 }  // namespace
+
+void prefill_attention(Handle* h, const PrefillAttn& a, bool fuse_qkv, int bn, int attn, double causal_pairs) {
+    cudaStream_t st = h->stream;
+    const int hd = 128, nq = a.heads * hd, nkv = a.kv_heads * hd, nqkv = nq + 2 * nkv;
+    const double Rd = a.rows;
+    {
+        ProfScope ps(h, "pre_qkv", 2.0 * Rd * a.hidden * nqkv, 2.0 * a.hidden * nqkv);
+        if (fuse_qkv) {
+            // per-head RMSNorm + RoPE + the paged-KV write happen in the product's epilogue (gemm.cuh EPI_QKV): q, k and the cache
+            // are written once, the raw product never reaches memory (v does, as is: the attention reads it from there)
+            GemmEpiArgs e;
+            e.epi = EPI_QKV;
+            e.out = a.qkv;
+            e.ldo = nqkv;
+            e.rp = QkvRope{a.pos, a.row_seq, a.rope_t, a.rope_n, a.q_norm, a.k_norm, a.q, a.k, a.kc.pool, a.kc.page_table, a.kc.max_pages,
+                           a.kc.layers, a.layer, a.heads, a.kv_heads, a.eps};
+            gemm(a.xn, a.hidden, a.rows, a.hidden, a.w_qkv, nqkv, e, st, false, bn);
+        } else {
+            gemm(a.xn, a.hidden, a.rows, a.hidden, a.w_qkv, nqkv, epi_store(a.qkv, nqkv, nullptr), st, false, bn);
+        }
+    }
+    if (!fuse_qkv) {
+        ProfScope ps(h, "pre_rope", 0, 4.0 * Rd * nqkv);
+        // v is not transformed: the attention reads it straight from the QKV product, only k needs a contiguous copy
+        qknorm_rope_kv_launch(a.qkv, nqkv, a.q_norm, a.k_norm, a.pos, a.row_seq, a.rows, a.heads, a.kv_heads, a.eps, a.rope, a.q, a.k,
+                              nullptr, a.kc, a.layer, st);
+    }
+    ProfScope ps(h, "pre_attn", 4.0 * causal_pairs * nq, 0);
+    if (attn == 0)
+        flash_attn_tc_launch(a.q, nq, a.k, nkv, a.qkv + nq + nkv, nqkv, a.att, nq, a.segs, a.rows, a.heads, a.heads / a.kv_heads, hd, true,
+                             a.scale, st);
+    else if (attn == 1)
+        flash_attn_launch(a.q, nq, a.k, nkv, a.qkv + nq + nkv, nqkv, a.att, nq, a.segs, a.heads, a.heads / a.kv_heads, hd, true, a.scale, st);
+}
 
 int encoder_tokens_for(int frames) {
     // AudioEncoder.swift:287-303 with chunk = 100

@@ -169,6 +169,28 @@ struct BatchState {
     }
 };
 
+// One decoder layer's prefill attention block (forward.cu, FloatTextDecoder.swift:77-117): the q‖k‖v product of the normed rows,
+// per-head RMSNorm + split-half RoPE of q and k, k and v written into the paged cache, then the causal attention of every prompt.
+// decoder_layers runs it on the batch's buffers and q3asr_debug_prefill_attention on the caller's, so the kernel tests see the
+// product's own launches.
+struct PrefillAttn {
+    const bf16* xn;                       // [rows, hidden] normed hidden states
+    const bf16 *w_qkv, *q_norm, *k_norm;  // [(heads + 2 kv_heads) * 128, hidden] in q | k | v row order; [128]; [128]
+    int rows, hidden, heads, kv_heads;
+    float eps, scale;
+    const int *pos, *row_seq;             // [rows] position and page-table row of every packed row
+    AttnSegs segs;                        // the prompts
+    const float2 *rope, *rope_t;          // (cos, sin) tables [rope_n][64] and [64][rope_n]
+    int rope_n;
+    KvCache kc;
+    int layer;
+    bf16 *qkv, *q, *k, *att;              // [rows, nqkv] (the attention reads v from it), [rows, nq], [rows, nkv], [rows, nq]
+};
+// fuse_qkv: norm, RoPE and the cache write in the product's epilogue (EPI_QKV), else the plain product + qknorm_rope_kv_kernel;
+// bn: the product's tile width (0: gemm's choice); attn: 0 the tcgen05 kernel, 1 the mma.sync kernel, -1 none.
+// causal_pairs (sum over prompts of S(S+1)/2) only feeds the profile.
+void prefill_attention(Handle* h, const PrefillAttn& a, bool fuse_qkv, int bn, int attn, double causal_pairs);
+
 // persistent decode-step kernel (megastep.cu)
 bool megastep_supported(const Handle* h, const BatchState* bs);
 void megastep_prepare(Handle* h, BatchState* bs);

@@ -82,7 +82,7 @@ EXPORTS = [
     "q3asr_timer_record", "q3asr_timer_elapsed_ms", "q3asr_stage_ms", "q3asr_launch_count", "q3asr_decode_stats", "q3asr_flush_l2",
     "q3asr_profile", "q3asr_profile_report",
     "q3asr_pool_create", "q3asr_pool_destroy", "q3asr_pool_last_error", "q3asr_pool_transcribe_ids", "q3asr_schedule",
-    "q3asr_debug_gemm", "q3asr_debug_conv", "q3asr_debug_attention", "q3asr_debug_decode_attention",
+    "q3asr_debug_gemm", "q3asr_debug_conv", "q3asr_debug_attention", "q3asr_debug_decode_attention", "q3asr_debug_prefill_attention",
     "q3asr_tokenizer_load", "q3asr_tokenizer_from_pairs", "q3asr_tokenizer_add_merge", "q3asr_tokenizer_destroy",
     "q3asr_tokenizer_last_error", "q3asr_tokenizer_size", "q3asr_tokenizer_decode", "q3asr_tokenizer_encode", "q3asr_tokenizer_token_id",
     "q3asr_io_last_error", "q3asr_wav_parse", "q3asr_wav_load", "q3asr_wav_write", "q3asr_resample_len", "q3asr_resample", "q3asr_resample_design",
@@ -172,6 +172,8 @@ def lib():
         L.q3asr_debug_attention.argtypes = [vp, vp, vp, vp, ci, ci, ci, ci, vp, vp, ci, ci, ctypes.c_float, ci, vp]
         L.q3asr_debug_decode_attention.argtypes = [vp, vp, ci, ci, ci, ci, vp, vp, ctypes.c_float, ctypes.c_float, vp, vp, ci, vp, ci, ci,
                                                    ci, ci, ci, vp]
+        L.q3asr_debug_prefill_attention.argtypes = [vp, vp, vp, ci, ci, ci, ci, vp, vp, ctypes.c_float, ctypes.c_float, vp, vp, vp, ci, vp,
+                                                    ci, ci, vp, ci, ci, ci, ci, ci, ci, vp, vp, vp, vp]
         L.q3asr_tokenizer_load.argtypes = [ctypes.c_char_p, ctypes.POINTER(vp)]
         L.q3asr_tokenizer_from_pairs.argtypes = [vp, vp, ci, ctypes.POINTER(vp)]
         L.q3asr_tokenizer_add_merge.argtypes = [vp, ctypes.c_char_p, ctypes.c_char_p]
@@ -982,6 +984,37 @@ class Qwen3ASRModel:
                                                     pool.ctypes.data, n_pages, layers, int(layer), int(variant), int(launches),
                                                     out.ctypes.data))
         return bf16_bits_to_f32(out), pool
+
+    def debug_prefill_attention(self, x, w, heads, kv_heads, q_norm, k_norm, segs, seg_table_rows, page_table, pool, layer, qkv_variant=0,
+                                bn=0, attn_variant=0, eps=1e-6, scale=None):
+        """One decoder layer's prefill attention block (q3asr_debug_prefill_attention).  x [rows, hidden], w [(heads + 2*kv_heads)*128,
+        hidden], q_norm / k_norm [128]: float32 holding bf16 values; segs: (row0, len) packed back to back; seg_table_rows: the
+        page-table row of every segment; page_table [table_rows, max_pages]; pool uint16 (bf16 bits) [n_pages, layers, 2, kv_heads,
+        32, 128].  Returns (q, k, qkv, att) float32 (NaN where the call wrote nothing) and the pool after the call, uint16."""
+        xb, wb = f32_to_bf16_bits(np.asarray(x, np.float32)), f32_to_bf16_bits(np.asarray(w, np.float32))
+        rows, hidden = xb.shape
+        nq, nkv = heads * 128, kv_heads * 128
+        assert wb.shape == (nq + 2 * nkv, hidden)
+        qw, kw = f32_to_bf16_bits(np.asarray(q_norm, np.float32)), f32_to_bf16_bits(np.asarray(k_norm, np.float32))
+        r0 = np.ascontiguousarray([s[0] for s in segs], dtype=np.int32)
+        ln = np.ascontiguousarray([s[1] for s in segs], dtype=np.int32)
+        tr = np.ascontiguousarray(seg_table_rows, dtype=np.int32)
+        pt = np.ascontiguousarray(page_table, dtype=np.int32)
+        pool = np.array(pool, dtype=np.uint16, order="C")  # a copy: the call writes k and v into it
+        n_pages, layers = pool.shape[0], pool.shape[1]
+        assert pool.shape[2:] == (2, kv_heads, 32, 128) and pt.ndim == 2 and tr.shape == r0.shape
+        if scale is None:
+            scale = 1.0 / np.sqrt(128.0)
+        q = np.empty((rows, nq), dtype=np.uint16)
+        k = np.empty((rows, nkv), dtype=np.uint16)
+        qkv = np.empty((rows, nq + 2 * nkv), dtype=np.uint16)
+        att = np.empty((rows, nq), dtype=np.uint16)
+        self._ck(lib().q3asr_debug_prefill_attention(self._h, xb.ctypes.data, wb.ctypes.data, rows, hidden, heads, kv_heads, qw.ctypes.data,
+                                                     kw.ctypes.data, ctypes.c_float(eps), ctypes.c_float(scale), r0.ctypes.data, ln.ctypes.data,
+                                                     tr.ctypes.data, len(r0), pt.ctypes.data, pt.shape[0], pt.shape[1], pool.ctypes.data,
+                                                     n_pages, layers, int(layer), int(qkv_variant), int(bn), int(attn_variant), q.ctypes.data,
+                                                     k.ctypes.data, qkv.ctypes.data, att.ctypes.data))
+        return bf16_bits_to_f32(q), bf16_bits_to_f32(k), bf16_bits_to_f32(qkv), bf16_bits_to_f32(att), pool
 
     def debug_conv(self, x, w, bias, box=(0, 0, 0), simt=False):
         """x [B,H,W,C], w [O,3,3,C] float32 (bf16-representable) -> gelu(conv3x3 s2 p1 + bias) [B,OH,OW,O]."""
